@@ -8,6 +8,11 @@ clips.  Default workload = BASELINE.json configs[1]: train-time augmentation,
 the data path).  See DESIGN.md "Measurement".
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--mode custom|train|val] [--impl reference]
+                  [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (at most 64 MB; a larger output as a
+fixed, seeded sample of whole rows, see sample_outputs), so that two builds can be compared output for output: the
+inputs and the random decisions are seeded, identical from run to run.
 """
 import argparse
 import json
@@ -58,6 +63,38 @@ def ncu_traffic(workload, mode, out_dtype):
             return json.load(f).get(f"{workload}:{mode}:{out_dtype}")     # {"step": bytes, "kernels": {name: bytes}}
     except Exception:
         return None
+
+
+DUMP_BYTES = 64 << 20          # --dump-outputs: at most this many bytes written in all
+DUMP_SEED = 0
+
+
+def sample_outputs(arrays):
+    """{name: tensor} -> {file name: float32 / float64 ndarray} for --dump-outputs.  A tensor that fits its share of
+    DUMP_BYTES is kept whole as ``<name>``; a larger one becomes a fixed, seeded sample of whole last-axis rows,
+    ``<name>_rows`` [n, W] float32, with ``<name>_rows_index`` [n, ndim - 1] float64 holding each row's leading
+    indices.  The sample depends only on the shape, so two runs with the same arguments pick the same rows."""
+    share = DUMP_BYTES // len(arrays) - 4096        # room for the .npy headers
+    res = {}
+    for name, x in arrays.items():
+        if x.numel() * 4 <= share:
+            res[name] = x.float().cpu().numpy()
+            continue
+        lead, w = tuple(x.shape[:-1]), int(x.shape[-1])
+        n_rows = x.numel() // w
+        k = min(n_rows, share // (4 * w + 8 * len(lead)))
+        pick = torch.randperm(n_rows, generator=torch.Generator().manual_seed(DUMP_SEED))[:k].sort().values
+        idx = np.stack(np.unravel_index(pick.numpy(), lead), axis=1)
+        rows = x[tuple(torch.from_numpy(idx[:, d]).to(x.device) for d in range(len(lead)))]    # [k, w], no full copy
+        res[f"{name}_rows"] = rows.float().cpu().numpy()
+        res[f"{name}_rows_index"] = idx.astype(np.float64)
+    return res
+
+
+def write_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def measured_peaks():
@@ -302,7 +339,7 @@ def run_cfg4(args, rank, world, dev, out_dtype):
     from vision_collision_detection_b200.synth import make_clip_torch
     _, n, h, w, cs = WORKLOADS["cfg4"]
     video = torch.cat([make_clip_torch(100, h, w, seed=rank * 100 + i, kind="dashcam", device=dev) for i in range(n // 100)])
-    steps = min(args.steps, 50)
+    steps = args.steps
     warm = max(3, args.warmup)
 
     def timed(fn):
@@ -322,6 +359,7 @@ def run_cfg4(args, rank, world, dev, out_dtype):
 
     sw = SlidingWindowTransform(window=16, stride=8, out_dtype=out_dtype)
     ms, view = timed(lambda: sw.windows(video))
+    dump = sample_outputs({"windows": view}) if args.dump_outputs and rank == 0 else None
     launches = get_engine(dev).last_launches
     ms_m8, m8 = timed(lambda: sw.windows(video, materialize=True))
     sw1 = SlidingWindowTransform(window=16, stride=1, out_dtype=out_dtype)
@@ -354,6 +392,8 @@ def run_cfg4(args, rank, world, dev, out_dtype):
                "d2h_bytes_per_step": int(host_out.numel() * host_out.element_size()), "steps": e_steps,
                "note": "PCIe-bound: 3.3 GB of uint8 frames per video"}
         del pipe, host_video
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     if rank == 0:
         peaks, kind = measured_peaks()
         k = len(sliding_window_starts(n, 16, 8))
@@ -395,7 +435,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true", help="e2e legs: do not pin the rank to the GPU's NUMA-local CPUs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float32, at most 64 MB in all: "
+                         "a larger output is a fixed, seeded sample of whole rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup   # timing rules: W >= 3
 
     rank = int(os.environ.get("RANK", "0"))
@@ -485,6 +532,7 @@ def main():
     e1.record()
     barrier()
     t_wall1 = time.time()
+    last_out = out.clone() if args.dump_outputs and rank == 0 else None    # before the untimed steps below reuse out
     launches = eng.last_launches * args.steps
     ms_total = e0.elapsed_time(e1)
     if sampler is not None and sampler.proc is not None and sampler.count(t_wall0, t_wall1) < 3:
@@ -581,6 +629,8 @@ def main():
             e2e["note"] += ("; multi-GPU: h2d_GBs_per_gpu lists every rank's own rate - on a single-socket host the aggregate "
                             "saturates (about 190 GB/s on the 8 x B200 box of DESIGN.md section 6), which is what bounds this leg")
 
+    if last_out is not None:
+        write_outputs(args.dump_outputs, sample_outputs({"out": last_out}))
     if rank == 0:
         peaks, peak_kind = measured_peaks()
         per_clip = algorithmic_bytes_per_clip(t, h, w, cs, out.element_size())

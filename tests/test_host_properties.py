@@ -57,3 +57,21 @@ def test_algorithmic_bytes_match_the_survey():
     b, t, h, w, cs = bench.WORKLOADS["cfg3"]
     assert b == 256 and all(b % n == 0 for n in (1, 2, 4, 8))                          # one batch sharded over the GPUs
     assert bench.WORKLOADS["cfg2"] == (32, 16, 720, 1280, 224) and bench.WORKLOADS["cfg4"][1] == 1200
+
+
+def test_dumped_outputs_are_whole_or_a_fixed_row_sample_within_64_mb():
+    import torch
+
+    import bench
+    small = torch.arange(4 * 3 * 4 * 8 * 8, dtype=torch.float32).view(4, 3, 4, 8, 8).bfloat16()
+    d = bench.sample_outputs({"out": small})
+    assert list(d) == ["out"] and d["out"].dtype == np.float32 and np.array_equal(d["out"], small.float().numpy())
+    # cfg2's output shape (bf16): too large to keep whole, so a seeded sample of whole rows with their indices
+    big = torch.randn((32, 3, 16, 224, 224), generator=torch.Generator().manual_seed(3)).bfloat16()
+    d = bench.sample_outputs({"out": big})
+    rows, idx = d["out_rows"], d["out_rows_index"]
+    assert rows.dtype == np.float32 and idx.dtype == np.float64 and rows.shape == (len(idx), 224) and idx.shape[1] == 4
+    assert sum(a.nbytes + 128 for a in d.values()) <= 64 << 20 and len(idx) > 0.2 * 32 * 3 * 16 * 224
+    assert np.array_equal(rows, big.float().numpy()[tuple(idx.astype(np.int64).T)])
+    again = bench.sample_outputs({"out": big})
+    assert all(np.array_equal(d[k], again[k]) for k in d)

@@ -26,6 +26,7 @@ from __future__ import annotations
 from typing import Any, Dict, List, Optional, Sequence, Tuple
 
 import torch
+from torch.utils.data import default_collate
 
 _CANON_CLIP = ("C", "T", "H", "W")
 
@@ -220,7 +221,11 @@ def collate_deferred(batch: Sequence[Any], *, collate_fn_map=None) -> DeferredBa
         g["frames"].append(b.frames)
         g["index"].append(pos)
         g["params"].append(b.params)
-    groups = [{"frames": torch.stack(g["frames"]), "index": g["index"], "params": g["params"]} for g in by_shape.values()]
+    # default_collate stacks tensors the way it does for the reference's own items: inside a DataLoader worker straight
+    # into shared memory, so the batch crosses to the main process as a file descriptor and the result queue's feeder
+    # thread has no storage to move (an error there is only printed, and the batch is lost)
+    groups = [{"frames": default_collate(g["frames"]), "index": g["index"], "params": g["params"]}
+              for g in by_shape.values()]
     return DeferredBatch(groups, len(batch), first._canon_shape[1], first._canon_shape[2], first.spec, first._order)
 
 

@@ -26,7 +26,7 @@ from typing import Any, Callable, Dict, Iterable, List, Optional, Sequence
 
 import numpy as np
 import torch
-from torch.utils.data import Dataset
+from torch.utils.data import Dataset, default_collate
 
 from .sensors import find_sensor_path, load_and_sync_sensor, window_sensor
 from .video_aug import GpuVideoTransform
@@ -328,8 +328,8 @@ def deferred_collate(items: Sequence[Dict[str, Any]]) -> Dict[str, Any]:
         g["frames"].append(f)
         g["index"].append(pos)
         g["params"].append(it["params"])
-    batch = {
-        "groups": [{"frames_u8": torch.stack(g["frames"]), "index": g["index"], "params": g["params"]}
+    batch = {   # default_collate: inside a DataLoader worker the stacks go straight into shared memory (deferred.py)
+        "groups": [{"frames_u8": default_collate(g["frames"]), "index": g["index"], "params": g["params"]}
                    for g in by_shape.values()],
         "valid": [it["frames_u8"] is not None for it in items],
         "target": [it["target"] for it in items],
@@ -337,7 +337,7 @@ def deferred_collate(items: Sequence[Dict[str, Any]]) -> Dict[str, Any]:
         "need": items[0].get("need") if items else None,
     }
     if items and all("sensor" in it for it in items):
-        batch["sensor"] = torch.stack([it["sensor"] for it in items])
+        batch["sensor"] = default_collate([it["sensor"] for it in items])
     return batch
 
 
