@@ -50,7 +50,9 @@ enum {
  * interleaved chroma plane [H/2][src_row_stride] (U0 V0 U1 V1 ...), 1.5 bytes per pixel; converted on the device to
  * RGB bytes with the BT.601 limited-range integer formula (C = Y-16, D = U-128, E = V-128; R = clip((298C+409E+128)>>8),
  * G = clip((298C-100D-208E+128)>>8), B = clip((298C+516D+128)>>8); nearest-neighbour chroma), then identical to U8.
- * frame_offsets then point at the Y planes; the workspace grows by one RGB copy of the batch. */
+ * frame_offsets then point at the Y planes; the workspace grows by one RGB copy of the batch.
+ * nexar_plan_create(g, NEXAR_SRC_NV12, ...) is nexar_plan_create_yuv(g, {NV12, BT601, LIMITED, 0}, ...); the other
+ * 4:2:0 variants (I420, BT.709, full range, padded luma height) are described by NexarYuvFormat below. */
 enum { NEXAR_SRC_U8 = 0, NEXAR_SRC_F32 = 1, NEXAR_SRC_NV12 = 2 };
 enum { NEXAR_DST_F32 = 0, NEXAR_DST_BF16 = 1 };
 
@@ -135,6 +137,49 @@ int nexar_aa_taps(int32_t in_size, int32_t out_size, int32_t* start, int32_t* co
                   int32_t kmax_capacity, int32_t* kmax);
 
 int nexar_plan_create(const NexarGeometry* geom, int32_t src_dtype, NexarPlan** out);
+
+/* YUV 4:2:0 decoder surfaces (nearest-neighbour chroma, one chroma sample per 2 x 2 pixels).
+ *
+ * Addressing, with pitch = NexarTransformArgs.src_row_stride and L = luma_rows (0 means src_h; L >= src_h, even):
+ *   Y plane at frame_offsets[i]:                        L rows of pitch bytes; the visible src_h x src_w picture is its
+ *                                                       top-left corner (rows src_h..L-1 and bytes src_w..pitch-1 are
+ *                                                       never read)
+ *   NV12: UV plane at frame_offsets[i] + L*pitch:       L/2 rows of pitch bytes, U0 V0 U1 V1 ...
+ *   I420: U plane at frame_offsets[i] + L*pitch:        L/2 rows of pitch/2 bytes (pitch must be even),
+ *         V plane at frame_offsets[i] + L*pitch*5/4:    L/2 rows of pitch/2 bytes
+ * so every surface is an [L*3/2][pitch] byte block.  A 1080p NVDEC surface, for example, has L = 1088.
+ *
+ * Conversion, the classic 8-bit integer form with every coefficient round(256 * c) of the standard's float value:
+ *   C = Y - Yo, D = U - 128, E = V - 128
+ *   R = clip((Ys C + Rv E + 128) >> 8), G = clip((Ys C - Gu D - Gv E + 128) >> 8), B = clip((Ys C + Bu D + 128) >> 8)
+ *                    Yo  Ys   Rv   Gu  Gv   Bu
+ *   BT.601 limited   16  298  409  100 208  516     (NEXAR_SRC_NV12)
+ *   BT.601 full       0  256  359   88 183  454
+ *   BT.709 limited   16  298  459   55 136  541
+ *   BT.709 full       0  256  403   48 120  475
+ * into the packed RGB copy in the workspace; from there it is the NEXAR_SRC_U8 path bit for bit.
+ *
+ * The conversion reads 16 luma pixels per thread with 16-byte loads when src, pitch and src_w are multiples of 16;
+ * that path also needs every frame_offsets[i] to be a multiple of 16 (not checked: the offsets live on the device).
+ * Any other even size, pitch or alignment takes a byte-wise kernel. */
+enum { NEXAR_YUV_NV12 = 0, NEXAR_YUV_I420 = 1 };
+enum { NEXAR_YUV_BT601 = 0, NEXAR_YUV_BT709 = 1 };
+enum { NEXAR_YUV_LIMITED = 0, NEXAR_YUV_FULL = 1 };
+
+typedef struct NexarYuvFormat {
+  uint32_t struct_size;         /* sizeof(NexarYuvFormat), for ABI checking */
+  int32_t layout;               /* NEXAR_YUV_NV12 / NEXAR_YUV_I420 */
+  int32_t matrix;               /* NEXAR_YUV_BT601 / NEXAR_YUV_BT709 */
+  int32_t range;                /* NEXAR_YUV_LIMITED / NEXAR_YUV_FULL */
+  int32_t luma_rows;            /* luma rows of the surface (0: src_h) */
+} NexarYuvFormat;
+
+/* A plan for YUV 4:2:0 surfaces.  geom->src_h / src_w are the visible picture (both even). */
+int nexar_plan_create_yuv(const NexarGeometry* geom, const NexarYuvFormat* fmt, NexarPlan** out);
+/* The integer coefficients {Yo, Ys, Rv, Gu, Gv, Bu} the conversion uses for (matrix, range), for binding checks. */
+int nexar_yuv_coefficients(int32_t matrix, int32_t range, int32_t out[6]);
+size_t nexar_sizeof_yuv_format(void);
+
 void nexar_plan_destroy(NexarPlan* plan);
 int nexar_plan_geometry(const NexarPlan* plan, NexarGeometry* out);
 

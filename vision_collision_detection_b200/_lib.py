@@ -23,6 +23,9 @@ NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a",
 NEXAR_ABI_VERSION = 1
 OK, ERR_INVALID, ERR_CUDA, ERR_WORKSPACE, ERR_UNSUPPORTED = 0, -1, -2, -3, -4
 SRC_U8, SRC_F32, SRC_NV12 = 0, 1, 2
+YUV_NV12, YUV_I420 = 0, 1
+YUV_BT601, YUV_BT709 = 0, 1
+YUV_LIMITED, YUV_FULL = 0, 1
 DST_F32, DST_BF16 = 0, 1
 FLIP, AUG, AFFINE, GRAYSCALE, NOISE, BLUR, POSTERIZE, SOLARIZE, INVERT, CUTOUT = (1 << i for i in range(10))
 MAX_CUTOUT = 8
@@ -53,6 +56,11 @@ class TransformArgs(C.Structure):
                 ("dst_dtype", C.c_int32), ("normalize", C.c_int32), ("dst_stride", C.c_int64 * 5),
                 ("mean", C.c_float * 3), ("std", C.c_float * 3),
                 ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t), ("stream", C.c_void_p)]
+
+
+class YuvFormat(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("layout", C.c_int32), ("matrix", C.c_int32), ("range", C.c_int32),
+                ("luma_rows", C.c_int32)]
 
 
 class NexarError(RuntimeError):
@@ -132,6 +140,31 @@ def lib():
         raise RuntimeError("NexarTransformArgs layout mismatch between the header and the Python binding")
     _lib = L
     return L
+
+
+_yuv_bound = False
+
+
+def yuv_lib():
+    """``lib()`` with the YUV 4:2:0 entry points bound.  They are bound on first use only, so that a library built
+    before they existed (selected with NEXAR_LIB) still loads and serves every other call."""
+    global _yuv_bound
+    L = lib()
+    if not _yuv_bound:
+        L.nexar_plan_create_yuv.argtypes = [C.POINTER(Geometry), C.POINTER(YuvFormat), C.POINTER(C.c_void_p)]
+        L.nexar_yuv_coefficients.argtypes = [C.c_int32, C.c_int32, C.c_void_p]
+        L.nexar_sizeof_yuv_format.restype = C.c_size_t
+        if L.nexar_sizeof_yuv_format() != C.sizeof(YuvFormat):
+            raise RuntimeError("NexarYuvFormat layout mismatch between the header and the Python binding")
+        _yuv_bound = True
+    return L
+
+
+def yuv_coefficients(matrix: int, range_: int):
+    """-> (Yo, Ys, Rv, Gu, Gv, Bu), the integer conversion coefficients the library uses."""
+    out = (C.c_int32 * 6)()
+    check(yuv_lib().nexar_yuv_coefficients(matrix, range_, out))
+    return tuple(int(v) for v in out)
 
 
 def check(code: int):

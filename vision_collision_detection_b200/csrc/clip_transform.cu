@@ -9,7 +9,7 @@
 //   K3 geometry : affine gather with the fill=0 mask quirk, effects, normalise, store (a kernel specialised for the
 //                 production letterboxes, a general one for everything else).
 //   K4 blur     : only when blur_sigma > 0 (reflect-padded gaussian, then the rest of the chain).
-//   NV12 -> RGB : decoder surfaces converted in front of K1 (NEXAR_SRC_NV12); window gather for inference.
+//   YUV 4:2:0 -> RGB : decoder surfaces (NV12 / I420, BT.601 / BT.709, limited / full range) converted in front of K1; window gather for inference.
 // The /255 decision of VideoTransform.forward is clip-global and data dependent
 // (nexar_video_aug.py:814): K1 runs assuming "max > 1", records the clip maximum, and
 // a second, normally empty, launch (fixup_frame_kernel) redoes the clips whose maximum was <= 1.
@@ -72,9 +72,18 @@ struct DevPlan {
   int x_align4;            // the horizontal windows start at multiples of four pixels (8-byte aligned: LDS.64, no bank conflicts at 4:1)
 };
 
+// Integer YUV -> RGB coefficients (include/nexar_clip_transform.h): round(256 * c) of the standard's float values.
+struct YuvCoef { int yo, ys, rv, gu, gv, bu; };
+static const YuvCoef kYuvCoef[2][2] = {        // [matrix][range]
+    {{16, 298, 409, 100, 208, 516}, {0, 256, 359, 88, 183, 454}},    // BT.601 limited, full
+    {{16, 298, 459, 55, 136, 541}, {0, 256, 403, 48, 120, 475}}};    // BT.709 limited, full
+
 struct NexarPlan {
   NexarGeometry g;
-  int src_dtype;
+  int src_dtype;               // NEXAR_SRC_NV12 stands for every YUV 4:2:0 source; yuv_* below say which
+  int yuv_layout = NEXAR_YUV_NV12;
+  int yuv_luma_rows = 0;
+  YuvCoef yuv_coef = kYuvCoef[NEXAR_YUV_BT601][NEXAR_YUV_LIMITED];
   DevPlan d;
   void* dev_tables;
   std::vector<int> ystart, ycount, xstart, xcount;
@@ -341,7 +350,34 @@ extern "C" int nexar_aa_taps(int32_t in_size, int32_t out_size, int32_t* start, 
   return NEXAR_OK;
 }
 
+static int plan_create(const NexarGeometry* g, int32_t src_dtype, const NexarYuvFormat* yuv, NexarPlan** out);
+
 extern "C" int nexar_plan_create(const NexarGeometry* g, int32_t src_dtype, NexarPlan** out) {
+  return plan_create(g, src_dtype, nullptr, out);
+}
+
+extern "C" size_t nexar_sizeof_yuv_format(void) { return sizeof(NexarYuvFormat); }
+
+extern "C" int nexar_yuv_coefficients(int32_t matrix, int32_t range, int32_t out[6]) {
+  if (!out) return fail(NEXAR_ERR_INVALID, "yuv_coefficients: null argument");
+  if ((matrix != NEXAR_YUV_BT601 && matrix != NEXAR_YUV_BT709) || (range != NEXAR_YUV_LIMITED && range != NEXAR_YUV_FULL))
+    return fail(NEXAR_ERR_INVALID, "yuv_coefficients: unknown matrix or range");
+  const YuvCoef& k = kYuvCoef[matrix][range];
+  const int32_t v[6] = {k.yo, k.ys, k.rv, k.gu, k.gv, k.bu};
+  memcpy(out, v, sizeof(v));
+  return NEXAR_OK;
+}
+
+extern "C" int nexar_plan_create_yuv(const NexarGeometry* g, const NexarYuvFormat* f, NexarPlan** out) {
+  if (!f) return fail(NEXAR_ERR_INVALID, "plan_create_yuv: null argument");
+  if (f->struct_size != sizeof(NexarYuvFormat)) return fail(NEXAR_ERR_INVALID, "plan_create_yuv: NexarYuvFormat size mismatch (ABI)");
+  if (f->layout != NEXAR_YUV_NV12 && f->layout != NEXAR_YUV_I420) return fail(NEXAR_ERR_INVALID, "plan_create_yuv: unknown layout");
+  if (f->matrix != NEXAR_YUV_BT601 && f->matrix != NEXAR_YUV_BT709) return fail(NEXAR_ERR_INVALID, "plan_create_yuv: unknown matrix");
+  if (f->range != NEXAR_YUV_LIMITED && f->range != NEXAR_YUV_FULL) return fail(NEXAR_ERR_INVALID, "plan_create_yuv: unknown range");
+  return plan_create(g, NEXAR_SRC_NV12, f, out);
+}
+
+static int plan_create(const NexarGeometry* g, int32_t src_dtype, const NexarYuvFormat* yuv, NexarPlan** out) {
   if (!g || !out) return fail(NEXAR_ERR_INVALID, "plan_create: null argument");
   if (src_dtype != NEXAR_SRC_U8 && src_dtype != NEXAR_SRC_F32 && src_dtype != NEXAR_SRC_NV12)
     return fail(NEXAR_ERR_INVALID, "plan_create: bad src_dtype");
@@ -349,9 +385,17 @@ extern "C" int nexar_plan_create(const NexarGeometry* g, int32_t src_dtype, Nexa
     return fail(NEXAR_ERR_INVALID, "plan_create: NV12 frames need an even height and width");
   if (g->src_h <= 0 || g->src_w <= 0 || g->canvas <= 0 || g->resize_h <= 0 || g->resize_w <= 0)
     return fail(NEXAR_ERR_INVALID, "plan_create: bad geometry");
+  const int luma_rows = yuv && yuv->luma_rows ? yuv->luma_rows : g->src_h;
+  if (src_dtype == NEXAR_SRC_NV12 && (luma_rows < g->src_h || (luma_rows & 1)))
+    return fail(NEXAR_ERR_INVALID, "plan_create_yuv: luma_rows must be even and >= src_h");
   NexarPlan* p = new NexarPlan();
   p->g = *g;
   p->src_dtype = src_dtype;
+  p->yuv_luma_rows = luma_rows;
+  if (yuv) {
+    p->yuv_layout = yuv->layout;
+    p->yuv_coef = kYuvCoef[yuv->matrix][yuv->range];
+  }
   int ky = 0, kx = 0;
   aa_taps_host(g->src_h, g->resize_h, p->ystart, p->ycount, p->ywt, ky);
   aa_taps_host(g->src_w, g->resize_w, p->xstart, p->xcount, p->xwt, kx);
@@ -458,8 +502,8 @@ struct Workspace {
   FrameInfo* finfo;     // [n_frames] per-frame constants for K2/K3, written by K1.5
   uint2* inter;         // [n_frames][bh][bw]   q15 RGBX pixels (8 bytes), brightness-adjusted, then colour-adjusted in place
   float* canvas;        // [n_frames][3][cs][cs] pre-blur canvas (blur path only)
-  int64_t* rgb_offsets; // [n_frames] NV12 sources: byte offsets of the converted frames in `rgb`
-  unsigned char* rgb;   // [n_frames][src_h][src_w][3] NV12 sources: packed RGB produced by nv12_to_rgb_kernel
+  int64_t* rgb_offsets; // [n_frames] YUV sources: byte offsets of the converted frames in `rgb`
+  unsigned char* rgb;   // [n_frames][src_h][src_w][3] YUV sources: packed RGB produced by yuv420_to_rgb_*_kernel
   size_t total;
 };
 
@@ -2286,27 +2330,31 @@ __global__ void __launch_bounds__(256) blur_kernel(DevPlan P, KArgs A) {
 }
 
 // ---------------------------------------------------------------------------------
-// NV12 sources (what a hardware decoder produces: 1.5 bytes per pixel instead of 3).  Y plane [H][pitch], then the
-// interleaved chroma plane [H/2][pitch] (U0 V0 U1 V1 ...), one chroma pair per 2 x 2 pixels (nearest neighbour).
-// Conversion = ITU-R BT.601 limited range in its classic 8-bit integer form,
-//   C = Y - 16, D = U - 128, E = V - 128
-//   R = clip((298 C + 409 E + 128) >> 8)   G = clip((298 C - 100 D - 208 E + 128) >> 8)   B = clip((298 C + 516 D + 128) >> 8)
-// to packed RGB bytes — exactly the uint8 frames the resize kernels take, so everything downstream (the /255 rule on the
-// clip maximum included) is the RGB path bit for bit (oracle/nv12_oracle.py states the same formula in numpy).
+// YUV 4:2:0 sources (what decoders produce: 1.5 bytes per pixel instead of 3).  Y plane [L][pitch], then either the
+// interleaved chroma plane [L/2][pitch] (NV12: U0 V0 U1 V1 ...) or the U and V planes [L/2][pitch/2] each (I420), where
+// L >= H is the surface's luma height (uoff = L * pitch, voff = uoff + L/2 * pitch/2); one chroma pair per 2 x 2 pixels
+// (nearest neighbour).  Conversion = the classic 8-bit integer form with the coefficients of YuvCoef,
+//   C = Y - Yo, D = U - 128, E = V - 128
+//   R = clip((Ys C + Rv E + 128) >> 8)   G = clip((Ys C - Gu D - Gv E + 128) >> 8)   B = clip((Ys C + Bu D + 128) >> 8)
+// (BT.601 limited range: 16, 298, 409, 100, 208, 516) to packed RGB bytes — exactly the uint8 frames the resize kernels
+// take, so everything downstream (the /255 rule on the clip maximum included) is the RGB path bit for bit
+// (oracle/yuv420_oracle.py states the same formula in numpy).
 // clip(x >> 8) is evaluated as clamp(x, 0, 65535) >> 8, so the shift merges with the byte packing.
 // ---------------------------------------------------------------------------------
 __device__ __forceinline__ int clamp_u16(int x) { return min(max(x, 0), 65535); }
 struct ChromaTerms { int r, g, b; };
-__device__ __forceinline__ ChromaTerms chroma_terms(int u, int v) {
+__device__ __forceinline__ ChromaTerms chroma_terms(int u, int v, const YuvCoef& k) {
   const int d = u - 128, e = v - 128;
-  constexpr int base = -298 * 16 + 128;
-  return {409 * e + base, -100 * d - 208 * e + base, 516 * d + base};
+  const int base = 128 - k.ys * k.yo;
+  return {k.rv * e + base, -k.gu * d - k.gv * e + base, k.bu * d + base};
 }
 
-// 16 pixels of two rows per thread: three 16-byte loads, six 16-byte stores
-__global__ void __launch_bounds__(256) nv12_to_rgb_vec_kernel(const unsigned char* __restrict__ src, const int64_t* __restrict__ frame_offsets,
-                                                              int64_t pitch, int H, int W, unsigned char* __restrict__ rgb,
-                                                              int64_t* __restrict__ out_offsets) {
+// 16 pixels of two rows per thread: two 16-byte luma loads, one 16-byte (NV12) or two 8-byte (I420) chroma loads,
+// six 16-byte stores
+template <int Layout>
+__global__ void __launch_bounds__(256) yuv420_to_rgb_vec_kernel(const unsigned char* __restrict__ src, const int64_t* __restrict__ frame_offsets,
+                                                                int64_t pitch, int64_t uoff, int64_t voff, YuvCoef kc, int H, int W,
+                                                                unsigned char* __restrict__ rgb, int64_t* __restrict__ out_offsets) {
   const int frame = blockIdx.y;
   const int cols = W >> 4;
   const int unit = blockIdx.x * blockDim.x + threadIdx.x;
@@ -2317,19 +2365,29 @@ __global__ void __launch_bounds__(256) nv12_to_rgb_vec_kernel(const unsigned cha
   const unsigned char* f = src + frame_offsets[frame];
   const uint4 ya = __ldcs((const uint4*)(f + (int64_t)(2 * r2) * pitch + 16 * c));
   const uint4 yb = __ldcs((const uint4*)(f + (int64_t)(2 * r2 + 1) * pitch + 16 * c));
-  const uint4 uv = __ldcs((const uint4*)(f + (int64_t)(H + r2) * pitch + 16 * c));
-  const unsigned yaw[4] = {ya.x, ya.y, ya.z, ya.w}, ybw[4] = {yb.x, yb.y, yb.z, yb.w}, uvw[4] = {uv.x, uv.y, uv.z, uv.w};
+  unsigned uvw[4];   // U V U V bytes of pixels 4q .. 4q+3
+  if (Layout == NEXAR_YUV_NV12) {
+    const uint4 uv = __ldcs((const uint4*)(f + uoff + (int64_t)r2 * pitch + 16 * c));
+    uvw[0] = uv.x, uvw[1] = uv.y, uvw[2] = uv.z, uvw[3] = uv.w;
+  } else {
+    const int64_t cp = pitch >> 1;
+    const uint2 u = __ldcs((const uint2*)(f + uoff + (int64_t)r2 * cp + 8 * c));
+    const uint2 v = __ldcs((const uint2*)(f + voff + (int64_t)r2 * cp + 8 * c));
+    uvw[0] = __byte_perm(u.x, v.x, 0x5140), uvw[1] = __byte_perm(u.x, v.x, 0x7362);
+    uvw[2] = __byte_perm(u.y, v.y, 0x5140), uvw[3] = __byte_perm(u.y, v.y, 0x7362);
+  }
+  const unsigned yaw[4] = {ya.x, ya.y, ya.z, ya.w}, ybw[4] = {yb.x, yb.y, yb.z, yb.w};
   unsigned oa[12], ob[12];   // 48 output bytes per row
 #pragma unroll
   for (int q = 0; q < 4; ++q) {  // four pixels (two chroma pairs) per 32-bit word of luma
-    const ChromaTerms t0 = chroma_terms(uvw[q] & 255u, (uvw[q] >> 8) & 255u);
-    const ChromaTerms t1 = chroma_terms((uvw[q] >> 16) & 255u, uvw[q] >> 24);
+    const ChromaTerms t0 = chroma_terms(uvw[q] & 255u, (uvw[q] >> 8) & 255u, kc);
+    const ChromaTerms t1 = chroma_terms((uvw[q] >> 16) & 255u, uvw[q] >> 24, kc);
     unsigned char* pa = (unsigned char*)oa + 12 * q;
     unsigned char* pb = (unsigned char*)ob + 12 * q;
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
       const ChromaTerms& t = k < 2 ? t0 : t1;
-      const int la = 298 * (int)((yaw[q] >> (8 * k)) & 255u), lb = 298 * (int)((ybw[q] >> (8 * k)) & 255u);
+      const int la = kc.ys * (int)((yaw[q] >> (8 * k)) & 255u), lb = kc.ys * (int)((ybw[q] >> (8 * k)) & 255u);
       pa[3 * k + 0] = (unsigned char)(clamp_u16(la + t.r) >> 8);
       pa[3 * k + 1] = (unsigned char)(clamp_u16(la + t.g) >> 8);
       pa[3 * k + 2] = (unsigned char)(clamp_u16(la + t.b) >> 8);
@@ -2349,9 +2407,10 @@ __global__ void __launch_bounds__(256) nv12_to_rgb_vec_kernel(const unsigned cha
 }
 
 // any even size / pitch / alignment: one 2 x 2 block per thread
-__global__ void __launch_bounds__(256) nv12_to_rgb_any_kernel(const unsigned char* __restrict__ src, const int64_t* __restrict__ frame_offsets,
-                                                              int64_t pitch, int H, int W, unsigned char* __restrict__ rgb,
-                                                              int64_t* __restrict__ out_offsets) {
+template <int Layout>
+__global__ void __launch_bounds__(256) yuv420_to_rgb_any_kernel(const unsigned char* __restrict__ src, const int64_t* __restrict__ frame_offsets,
+                                                                int64_t pitch, int64_t uoff, int64_t voff, YuvCoef kc, int H, int W,
+                                                                unsigned char* __restrict__ rgb, int64_t* __restrict__ out_offsets) {
   const int frame = blockIdx.y;
   const int cols = W >> 1;
   const int unit = blockIdx.x * blockDim.x + threadIdx.x;
@@ -2360,15 +2419,22 @@ __global__ void __launch_bounds__(256) nv12_to_rgb_any_kernel(const unsigned cha
   if (unit >= cols * (H >> 1)) return;
   const int r2 = unit / cols, c = unit - r2 * cols;
   const unsigned char* f = src + frame_offsets[frame];
-  const unsigned char* uvp = f + (int64_t)(H + r2) * pitch + 2 * c;
-  const ChromaTerms t = chroma_terms(uvp[0], uvp[1]);
+  int u, v;
+  if (Layout == NEXAR_YUV_NV12) {
+    const unsigned char* uvp = f + uoff + (int64_t)r2 * pitch + 2 * c;
+    u = uvp[0], v = uvp[1];
+  } else {
+    const int64_t at = (int64_t)r2 * (pitch >> 1) + c;
+    u = f[uoff + at], v = f[voff + at];
+  }
+  const ChromaTerms t = chroma_terms(u, v, kc);
 #pragma unroll
   for (int dy = 0; dy < 2; ++dy) {
     const unsigned char* yp = f + (int64_t)(2 * r2 + dy) * pitch + 2 * c;
     unsigned char* o = rgb + (int64_t)frame * fbytes + ((int64_t)(2 * r2 + dy) * W + 2 * c) * 3;
 #pragma unroll
     for (int dx = 0; dx < 2; ++dx) {
-      const int l = 298 * (int)yp[dx];
+      const int l = kc.ys * (int)yp[dx];
       o[3 * dx + 0] = (unsigned char)(clamp_u16(l + t.r) >> 8);
       o[3 * dx + 1] = (unsigned char)(clamp_u16(l + t.g) >> 8);
       o[3 * dx + 2] = (unsigned char)(clamp_u16(l + t.b) >> 8);
@@ -2696,6 +2762,8 @@ extern "C" int nexar_clip_transform(const NexarPlan* p, const NexarTransformArgs
   const size_t esz = p->src_dtype == NEXAR_SRC_F32 ? 4 : 1;
   if (a->src_row_stride < (int64_t)(nv12 ? p->g.src_w : p->g.src_w * 3 * esz))
     return fail(NEXAR_ERR_INVALID, "clip_transform: src_row_stride smaller than a row");
+  if (nv12 && p->yuv_layout == NEXAR_YUV_I420 && (a->src_row_stride & 1))
+    return fail(NEXAR_ERR_INVALID, "clip_transform: I420 surfaces need an even src_row_stride");
 
   Workspace w = carve(p, a->n_clips, a->frames_per_clip, a->workspace, a->any_flags);
   KArgs K;
@@ -2706,13 +2774,23 @@ extern "C" int nexar_clip_transform(const NexarPlan* p, const NexarTransformArgs
     // decoder surfaces -> packed RGB bytes in the workspace (one launch), then the uint8 path on those
     const int H = p->g.src_h, W = p->g.src_w, nf = a->n_clips * a->frames_per_clip;
     cudaStream_t st = (cudaStream_t)a->stream;
-    const bool vec = (W % 16) == 0 && (a->src_row_stride % 16) == 0 && (((uintptr_t)a->src) & 15) == 0;
-    if (vec)
-      nv12_to_rgb_vec_kernel<<<dim3(((W / 16) * (H / 2) + 255) / 256, nf), 256, 0, st>>>(
-          (const unsigned char*)a->src, a->frame_offsets, a->src_row_stride, H, W, w.rgb, w.rgb_offsets);
-    else
-      nv12_to_rgb_any_kernel<<<dim3(((W / 2) * (H / 2) + 255) / 256, nf), 256, 0, st>>>(
-          (const unsigned char*)a->src, a->frame_offsets, a->src_row_stride, H, W, w.rgb, w.rgb_offsets);
+    const int64_t pitch = a->src_row_stride, uoff = (int64_t)p->yuv_luma_rows * pitch;
+    const int64_t voff = uoff + (int64_t)(p->yuv_luma_rows / 2) * (pitch / 2);
+    const unsigned char* s = (const unsigned char*)a->src;
+    // pitch % 16 == 0 with an even luma height also keeps the 8-byte I420 chroma loads aligned
+    const bool vec = (W % 16) == 0 && (pitch % 16) == 0 && (((uintptr_t)a->src) & 15) == 0;
+    const dim3 gv(((W / 16) * (H / 2) + 255) / 256, nf), ga(((W / 2) * (H / 2) + 255) / 256, nf);
+    if (p->yuv_layout == NEXAR_YUV_I420) {
+      if (vec)
+        yuv420_to_rgb_vec_kernel<NEXAR_YUV_I420><<<gv, 256, 0, st>>>(s, a->frame_offsets, pitch, uoff, voff, p->yuv_coef, H, W, w.rgb, w.rgb_offsets);
+      else
+        yuv420_to_rgb_any_kernel<NEXAR_YUV_I420><<<ga, 256, 0, st>>>(s, a->frame_offsets, pitch, uoff, voff, p->yuv_coef, H, W, w.rgb, w.rgb_offsets);
+    } else {
+      if (vec)
+        yuv420_to_rgb_vec_kernel<NEXAR_YUV_NV12><<<gv, 256, 0, st>>>(s, a->frame_offsets, pitch, uoff, voff, p->yuv_coef, H, W, w.rgb, w.rgb_offsets);
+      else
+        yuv420_to_rgb_any_kernel<NEXAR_YUV_NV12><<<ga, 256, 0, st>>>(s, a->frame_offsets, pitch, uoff, voff, p->yuv_coef, H, W, w.rgb, w.rgb_offsets);
+    }
     CUDA_TRY(cudaGetLastError());
     ++g_launches;
     K.src = w.rgb;

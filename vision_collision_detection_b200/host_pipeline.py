@@ -12,7 +12,7 @@ from typing import Any, Dict, List, Optional
 import torch
 
 from .engine import ClipTransformEngine
-from .video_aug import GpuVideoTransform
+from .video_aug import GpuVideoTransform, check_pixel_format
 
 
 def bind_to_gpu_numa_node(device_index: int) -> Optional[List[int]]:
@@ -47,15 +47,16 @@ def bind_to_gpu_numa_node(device_index: int) -> Optional[List[int]]:
 class HostClipPipeline:
     def __init__(self, transform: GpuVideoTransform, n_clips: int, frames: int, height: int, width: int,
                  device=None, clips_per_chunk: int = 4, n_streams: int = 3, out_dtype: Optional[torch.dtype] = None,
-                 pixel_format: str = "rgb"):
-        """``pixel_format="nv12"``: the host clips are decoder surfaces, uint8 ``[B,T,H*3/2,W]`` — half the bytes of
-        RGB over PCIe (the link is what bounds this path), converted to RGB on the device."""
+                 pixel_format: str = "rgb", color_matrix: str = "bt601", color_range: str = "limited"):
+        """``pixel_format="nv12"`` / ``"i420"``: the host clips are YUV 4:2:0 decoder surfaces, uint8 ``[B,T,H*3/2,W]``
+        — half the bytes of RGB over PCIe (the link is what bounds this path), converted to RGB on the device with
+        ``color_matrix`` / ``color_range`` (see ``GpuVideoTransform.forward_batch``)."""
         self.tf = transform
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-        if pixel_format not in ("rgb", "nv12"):
-            raise ValueError(f"unknown pixel_format {pixel_format!r}")
+        yuv = check_pixel_format(pixel_format, color_matrix, color_range)
         self.pixel_format = pixel_format
-        self.shape = (n_clips, frames, height * 3 // 2, width) if pixel_format == "nv12" else (n_clips, frames, height, width, 3)
+        self.yuv_kw = dict(pixel_format=pixel_format, color_matrix=color_matrix, color_range=color_range)
+        self.shape = (n_clips, frames, height * 3 // 2, width) if yuv else (n_clips, frames, height, width, 3)
         self.chunk = max(1, min(clips_per_chunk, n_clips))
         self.out_dtype = out_dtype or transform.out_dtype
         cs = transform.crop_size
@@ -82,7 +83,7 @@ class HostClipPipeline:
             raise ValueError(f"expected uint8 {self.shape}")
         n = self.shape[0]
         if params is None:
-            h = self.shape[2] * 2 // 3 if self.pixel_format == "nv12" else self.shape[2]
+            h = self.shape[2] * 2 // 3 if self.pixel_format != "rgb" else self.shape[2]
             params = self.tf.sample_params(n, h, self.shape[3])
         slot = self._slot
         self._slot ^= 1
@@ -96,8 +97,7 @@ class HostClipPipeline:
                 din = self.dev_in[i][: hi - lo]
                 din.copy_(host_clips[lo:hi], non_blocking=True)
                 dout = self.dev_out[i][: hi - lo]
-                self.tf.forward_batch(din, params=params[lo:hi], out=dout, engine=self.engines[i],
-                                      pixel_format=self.pixel_format)
+                self.tf.forward_batch(din, params=params[lo:hi], out=dout, engine=self.engines[i], **self.yuv_kw)
                 host_out[lo:hi].copy_(dout, non_blocking=True)
         for i, s in enumerate(self.streams):
             self._done[slot][i].record(s)
@@ -111,5 +111,5 @@ class HostClipPipeline:
 
     @torch.no_grad()
     def run(self, host_clips: torch.Tensor, params: Optional[List[Dict[str, Any]]] = None) -> torch.Tensor:
-        """host_clips: pinned uint8 [B,T,H,W,3] (or [B,T,H*3/2,W] for nv12).  Returns the pinned [B,3,T,cs,cs] result (valid on return)."""
+        """host_clips: pinned uint8 [B,T,H,W,3] (or [B,T,H*3/2,W] for nv12 / i420).  Returns the pinned [B,3,T,cs,cs] result (valid on return)."""
         return self.wait(self.submit(host_clips, params))

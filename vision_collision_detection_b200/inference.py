@@ -9,6 +9,9 @@ frame of the video is transformed exactly once and the windows are strided views
 (or one gather when a materialised ``[K,3,T,cs,cs]`` batch is wanted).
 Window rule: starts ``k*stride`` for ``k = 0..floor((N-window)/stride)``; a video
 shorter than the window is padded by repeating its last frame (nexar_videos.py:429-433).
+Every entry point also takes a video of YUV 4:2:0 decoder surfaces ``[N,R,P]`` with the
+``pixel_format`` / ``color_matrix`` / ``color_range`` / ``frame_size`` keywords of
+``GpuVideoTransform.forward_batch``.
 """
 from __future__ import annotations
 
@@ -18,7 +21,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .video_aug import GpuVideoTransform, create_video_transforms
+from .video_aug import GpuVideoTransform, check_pixel_format, create_video_transforms
 from .videos import select_start_frame, window_indices
 
 
@@ -30,13 +33,14 @@ def sliding_window_starts(num_frames: int, window: int, stride: int) -> List[int
 
 @torch.no_grad()
 def center_window(video_u8: torch.Tensor, transform: Optional[GpuVideoTransform] = None, fps: int = 10,
-                  duration: int = 5) -> torch.Tensor:
-    """[N,H,W,3] uint8 (device) -> [1,3,fps*duration,cs,cs]: sample_strategy='center' + val transform."""
+                  duration: int = 5, **source_format) -> torch.Tensor:
+    """[N,H,W,3] uint8 (device) -> [1,3,fps*duration,cs,cs]: sample_strategy='center' + val transform.  A video of YUV
+    surfaces [N,R,P] takes the source-format keywords of forward_batch (``pixel_format="i420"``, ...)."""
     tf = transform or create_video_transforms(mode="val")
     n = video_u8.shape[0]
     need = fps * duration
     idx = window_indices(n, need, select_start_frame(n, need, "center"))
-    return tf.forward_batch(video_u8.unsqueeze(0), frame_index=torch.tensor([idx], dtype=torch.int64))
+    return tf.forward_batch(video_u8.unsqueeze(0), frame_index=torch.tensor([idx], dtype=torch.int64), **source_format)
 
 
 class SlidingWindowTransform:
@@ -47,19 +51,25 @@ class SlidingWindowTransform:
         self.out_dtype = out_dtype
 
     @torch.no_grad()
-    def frames(self, video_u8: torch.Tensor) -> torch.Tensor:
-        """[N,H,W,3] uint8 on the device -> [N,3,cs,cs]: every frame transformed once."""
-        if video_u8.dim() != 4 or video_u8.shape[-1] != 3:
+    def frames(self, video_u8: torch.Tensor, pixel_format: str = "rgb", color_matrix: str = "bt601",
+               color_range: str = "limited", frame_size=None) -> torch.Tensor:
+        """[N,H,W,3] uint8 on the device -> [N,3,cs,cs]: every frame transformed once.  YUV surfaces [N,R,P] with
+        ``pixel_format="nv12"`` / ``"i420"`` and the other source-format keywords of forward_batch."""
+        if check_pixel_format(pixel_format, color_matrix, color_range):
+            if video_u8.dim() != 3:
+                raise ValueError(f"expected [N,R,P] {pixel_format} surfaces, got {tuple(video_u8.shape)}")
+        elif video_u8.dim() != 4 or video_u8.shape[-1] != 3:
             raise ValueError(f"expected [N,H,W,3], got {tuple(video_u8.shape)}")
         n = video_u8.shape[0]
-        out = self.tf.forward_batch(video_u8.unsqueeze(0), layout="BTCHW", out_dtype=self.out_dtype)  # [1,N,3,cs,cs]
+        out = self.tf.forward_batch(video_u8.unsqueeze(0), layout="BTCHW", out_dtype=self.out_dtype, pixel_format=pixel_format,
+                                    color_matrix=color_matrix, color_range=color_range, frame_size=frame_size)  # [1,N,3,cs,cs]
         if n < self.window:       # pad by repeating the last frame
             out = torch.cat([out, out[:, -1:].expand(1, self.window - n, *out.shape[2:])], dim=1)
         return out[0]
 
-    def windows(self, video_u8: torch.Tensor, materialize: bool = False) -> torch.Tensor:
+    def windows(self, video_u8: torch.Tensor, materialize: bool = False, **source_format) -> torch.Tensor:
         """-> [K,3,window,cs,cs].  A zero-copy strided view of the per-frame result unless ``materialize``."""
-        fr = self.frames(video_u8)                                   # [N',3,cs,cs]
+        fr = self.frames(video_u8, **source_format)                  # [N',3,cs,cs]
         starts = sliding_window_starts(fr.shape[0], self.window, self.stride)
         k = len(starts)
         s = fr.stride()
@@ -112,8 +122,10 @@ class WindowPredictor:
         self.swt = SlidingWindowTransform(window=window, stride=stride, transform=transform, out_dtype=out_dtype)
 
     @torch.no_grad()
-    def predict(self, video_u8: torch.Tensor, video_path: str = "", fps: float = 30.0) -> List[Dict[str, Any]]:
-        view = self.swt.windows(video_u8)                              # [K,3,T,cs,cs] strided view
+    def predict(self, video_u8: torch.Tensor, video_path: str = "", fps: float = 30.0,
+                **source_format) -> List[Dict[str, Any]]:
+        """``source_format``: the forward_batch keywords of a video of YUV surfaces (``pixel_format="i420"``, ...)."""
+        view = self.swt.windows(video_u8, **source_format)             # [K,3,T,cs,cs] strided view
         starts = sliding_window_starts(max(video_u8.shape[0], self.swt.window), self.swt.window, self.swt.stride)
         results: List[Dict[str, Any]] = []
         for lo in range(0, view.shape[0], self.batch_size):

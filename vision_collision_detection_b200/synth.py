@@ -85,3 +85,42 @@ def rgb_to_nv12(clip):
     import torch
     uv = torch.stack([u, v], dim=-1).reshape(u.shape[:-1] + (w,))
     return torch.cat([y, uv], dim=-2).clamp(0, 255).to(torch.uint8)
+
+
+def rgb_to_yuv420(clip: np.ndarray, layout: str = "nv12", matrix: str = "bt601", range_: str = "limited",
+                  luma_rows: int = None, pitch: int = None) -> np.ndarray:
+    """Synthetic decoder surfaces of any supported 4:2:0 variant: uint8 ``[...,H,W,3]`` -> uint8 ``[...,L*3/2,P]``
+    (``L = luma_rows`` >= H, ``P = pitch`` >= W, both default to the picture size; NV12: Y plane then the interleaved
+    UV plane, I420: Y, U and V planes; include/nexar_clip_transform.h).  The encode is the float64 one of the
+    standard with 2 x 2 chroma means, rounded to bytes; every padding byte is 255, so a reader that strays into the
+    padding shows."""
+    kr, kb = {"bt601": (0.299, 0.114), "bt709": (0.2126, 0.0722)}[matrix]
+    if range_ not in ("limited", "full") or layout not in ("nv12", "i420"):
+        raise ValueError(f"unknown range or layout: {range_!r}, {layout!r}")
+    x = clip.astype(np.float64)
+    h, w = x.shape[-3], x.shape[-2]
+    lr = h if luma_rows is None else luma_rows
+    p = w if pitch is None else pitch
+    if h % 2 or w % 2 or lr % 2 or lr < h or p < w or (layout == "i420" and p % 2):
+        raise ValueError(f"bad surface: picture {h}x{w}, luma rows {lr}, pitch {p}")
+    yv = kr * x[..., 0] + (1 - kr - kb) * x[..., 1] + kb * x[..., 2]
+    blk = x.reshape(x.shape[:-3] + (h // 2, 2, w // 2, 2, 3)).mean(axis=(-4, -2))
+    ym = kr * blk[..., 0] + (1 - kr - kb) * blk[..., 1] + kb * blk[..., 2]
+    pb = (blk[..., 2] - ym) / (2 * (1 - kb))
+    pr = (blk[..., 0] - ym) / (2 * (1 - kr))
+    if range_ == "limited":
+        y, u, v = 16 + yv * 219 / 255, 128 + pb * 224 / 255, 128 + pr * 224 / 255
+    else:
+        y, u, v = yv, 128 + pb, 128 + pr
+    q = lambda a: np.clip(np.floor(a + 0.5), 0, 255).astype(np.uint8)
+    lead = x.shape[:-3]
+    out = np.full(lead + (lr * 3 // 2, p), 255, np.uint8)
+    out[..., :h, :w] = q(y)
+    if layout == "nv12":
+        out[..., lr: lr + h // 2, :w] = np.stack([q(u), q(v)], axis=-1).reshape(lead + (h // 2, w))
+    else:
+        planes = np.full(lead + (lr, p // 2), 255, np.uint8)    # U plane rows, then V plane rows, P/2 bytes each
+        planes[..., : h // 2, : w // 2] = q(u)
+        planes[..., lr // 2: lr // 2 + h // 2, : w // 2] = q(v)
+        out[..., lr:, :] = planes.reshape(lead + (lr // 2, p))
+    return out

@@ -18,8 +18,8 @@ accepted and have no effect (they are never forwarded, :762-788).
 crop north_star names.
 
 Extra, GPU-only entry points: ``forward_batch`` (device-resident
-``[B,T,H,W,3]`` clips in, ``[B,3,T,cs,cs]`` out, fp32 or bf16, optional frame
-gather) — the call the loaders and bench use.
+``[B,T,H,W,3]`` clips or YUV 4:2:0 decoder surfaces in, ``[B,3,T,cs,cs]`` out,
+fp32 or bf16, optional frame gather) — the call the loaders and bench use.
 """
 from __future__ import annotations
 
@@ -33,6 +33,23 @@ import torch.nn as nn
 from . import _lib
 from .engine import _SRC, _alloc_out, get_engine
 from .params import VideoAugmentation, draw_noise_seed, pack_clip_params
+
+
+PIXEL_FORMATS = ("rgb", "nv12", "i420")
+_YUV_LAYOUT = {"nv12": _lib.YUV_NV12, "i420": _lib.YUV_I420}
+_YUV_MATRIX = {"bt601": _lib.YUV_BT601, "bt709": _lib.YUV_BT709}
+_YUV_RANGE = {"limited": _lib.YUV_LIMITED, "full": _lib.YUV_FULL}
+
+
+def check_pixel_format(pixel_format: str, color_matrix: str = "bt601", color_range: str = "limited") -> bool:
+    """Validates the source-format keywords of ``forward_batch``; returns True for the YUV 4:2:0 formats."""
+    if pixel_format not in PIXEL_FORMATS:
+        raise ValueError(f"unknown pixel_format {pixel_format!r}; expected one of {PIXEL_FORMATS}")
+    if color_matrix not in _YUV_MATRIX:
+        raise ValueError(f"unknown color_matrix {color_matrix!r}; expected one of {tuple(_YUV_MATRIX)}")
+    if color_range not in _YUV_RANGE:
+        raise ValueError(f"unknown color_range {color_range!r}; expected one of {tuple(_YUV_RANGE)}")
+    return pixel_format != "rgb"
 
 
 class _Stage:
@@ -182,7 +199,8 @@ class GpuVideoTransform(nn.Module):
     def forward_batch(self, frames: torch.Tensor, params: Optional[List[Dict[str, Any]]] = None,
                       frame_index: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None,
                       layout: str = "BCTHW", out_dtype: Optional[torch.dtype] = None, rng=random,
-                      engine=None, pixel_format: str = "rgb") -> torch.Tensor:
+                      engine=None, pixel_format: str = "rgb", color_matrix: str = "bt601",
+                      color_range: str = "limited", frame_size: Optional[Tuple[int, int]] = None) -> torch.Tensor:
         """frames: CUDA ``[B,T,H,W,3]`` (uint8 or float32, contiguous) — or, with ``frame_index``
         (int64 ``[B,T']`` indices into the flattened ``B*T`` frame axis), a frame pool from which each
         output clip gathers its frames (temporal sampling without a copy).  Returns ``[B,3,T',cs,cs]``.
@@ -190,15 +208,35 @@ class GpuVideoTransform(nn.Module):
         ``pixel_format="nv12"``: frames are decoder surfaces, uint8 ``[B,T,H*3/2,W]`` (Y plane, then the
         interleaved UV plane), 1.5 bytes per pixel; they are converted on the device (BT.601 limited range,
         include/nexar_clip_transform.h) to the RGB bytes the reference's decoder would have delivered
-        (nexar_videos.py:360,422) and take the uint8 path from there."""
-        nv12 = pixel_format == "nv12"
-        if pixel_format not in ("rgb", "nv12"):
-            raise ValueError(f"unknown pixel_format {pixel_format!r}")
-        if nv12:
+        (nexar_videos.py:360,422) and take the uint8 path from there.
+
+        ``pixel_format="i420"``: planar surfaces, the Y plane then the U and V planes of half the pitch each (what
+        libavcodec's ``yuv420p`` delivers).  ``color_matrix`` ("bt601" | "bt709") and ``color_range`` ("limited" |
+        "full") select the conversion of either YUV layout.  YUV frames are ``[B,T,R,P]`` surfaces with
+        ``L = R*2/3`` luma rows and pitch ``P``; ``frame_size=(h, w)`` is the visible picture in their top-left corner
+        (default ``(L, P)``), e.g. ``(1080, 1920)`` in the 1088-row surfaces of a hardware decoder.  The random
+        decisions are drawn for the visible ``h x w``, as for an RGB clip of that size."""
+        yuv = check_pixel_format(pixel_format, color_matrix, color_range)
+        if yuv:
             if frames.dim() != 4 or frames.dtype != torch.uint8 or frames.shape[2] % 3 or frames.shape[3] % 2:
-                raise ValueError(f"nv12 frames are uint8 [B,T,H*3/2,W] with even H and W, got {frames.dtype} {tuple(frames.shape)}")
+                raise ValueError(f"{pixel_format} frames are uint8 [B,T,H*3/2,W] with even H and W, got {frames.dtype} {tuple(frames.shape)}")
         elif frames.dim() != 5 or frames.shape[-1] != 3:
             raise ValueError(f"expected [B,T,H,W,3], got {tuple(frames.shape)}")
+        if frame_size is not None and not yuv:
+            raise ValueError("frame_size describes the visible picture of YUV surfaces; RGB frames have no padding")
+        if yuv:
+            b, t, rows, pitch = frames.shape
+            luma_rows = rows * 2 // 3
+            h, w = (luma_rows, pitch) if frame_size is None else (int(frame_size[0]), int(frame_size[1]))
+            if h <= 0 or w <= 0 or h % 2 or w % 2 or h > luma_rows or w > pitch:
+                raise ValueError(f"frame_size {(h, w)} must be even and fit the {luma_rows} luma rows x {pitch} pitch surface")
+            frame_bytes = rows * pitch
+            fmt = (_YUV_LAYOUT[pixel_format], _YUV_MATRIX[color_matrix], _YUV_RANGE[color_range], luma_rows)
+            # the format of the original NEXAR_SRC_NV12 plans keeps going through nexar_plan_create
+            src = "nv12" if fmt == (_lib.YUV_NV12, _lib.YUV_BT601, _lib.YUV_LIMITED, h) else fmt
+        else:
+            b, t, h, w, _ = frames.shape
+            frame_bytes = h * w * 3 * frames.element_size()
         if not frames.is_cuda:
             raise ValueError("forward_batch needs device-resident frames (use forward() for host tensors)")
         if frames.dtype not in _SRC:
@@ -206,12 +244,6 @@ class GpuVideoTransform(nn.Module):
         if not frames.is_contiguous():
             frames = frames.contiguous()
         eng = engine if engine is not None else get_engine(frames.device)
-        if nv12:
-            b, t, h, w = frames.shape[0], frames.shape[1], frames.shape[2] * 2 // 3, frames.shape[3]
-            frame_bytes = h * w * 3 // 2
-        else:
-            b, t, h, w, _ = frames.shape
-            frame_bytes = h * w * 3 * frames.element_size()
         if frame_index is not None:
             if frame_index.dim() != 2:
                 raise ValueError("frame_index must be [n_clips, frames_per_clip]")
@@ -235,9 +267,9 @@ class GpuVideoTransform(nn.Module):
         self.last_params = params
         packed, any_flags = pack_clip_params(params, self.crop_size, self.video_aug)
         two_pass = self.resize_short_side is not None and self.use_letterbox
-        if nv12 and two_pass:
-            raise ValueError("nv12 frames are not supported by the two-pass (short-side resize + letterbox) variant")
-        plan = None if two_pass else self._plan(eng, h, w, "nv12" if nv12 else frames.dtype)
+        if yuv and two_pass:
+            raise ValueError(f"{pixel_format} frames are not supported by the two-pass (short-side resize + letterbox) variant")
+        plan = None if two_pass else self._plan(eng, h, w, src if yuv else frames.dtype)
         dt = out_dtype or self.out_dtype
         if out is None:
             out, strides = _alloc_out(layout, n_clips, t_out, self.crop_size, dt, frames.device)
@@ -249,7 +281,7 @@ class GpuVideoTransform(nn.Module):
             return self._forward_two_pass(eng, frames, offsets, n_clips, t_out, packed, any_flags, out, strides)
         pdev = eng.upload_params(packed)
         eng.run(plan, frames, offsets, n_clips, t_out, pdev, any_flags, out, strides,
-                self.normalize, self.video_mean, self.video_std)
+                self.normalize, self.video_mean, self.video_std, src_row_stride=pitch if yuv else None)
         return out
 
     @torch.no_grad()

@@ -29,7 +29,7 @@ import torch
 from torch.utils.data import Dataset, default_collate
 
 from .sensors import find_sensor_path, load_and_sync_sensor, window_sensor
-from .video_aug import GpuVideoTransform
+from .video_aug import GpuVideoTransform, check_pixel_format
 
 
 # ---------------------------------------------------------------------------------
@@ -119,20 +119,51 @@ def _to_uint8_array(frames) -> np.ndarray:
     return np.asarray(frames)
 
 
+def _source_format(defer: bool, pixel_format: str, color_matrix: str, color_range: str) -> Optional[Dict[str, str]]:
+    """The forward_batch keywords of a dataset whose decoder delivers YUV 4:2:0 surfaces (None for RGB frames)."""
+    if not check_pixel_format(pixel_format, color_matrix, color_range):
+        return None
+    if not defer:
+        raise ValueError(f"pixel_format={pixel_format!r} needs defer=True: the surfaces are converted on the device by "
+                         "GpuAugLoader")
+    return {"pixel_format": pixel_format, "color_matrix": color_matrix, "color_range": color_range}
+
+
+def _blank_frame(shape, fmt: Optional[Dict[str, str]]) -> np.ndarray:
+    """A frame that converts to RGB zeros: zero bytes for RGB; for a YUV surface ``[H*3/2,W]`` Y = 16 (limited range)
+    or 0 (full range) and U = V = 128 (zero bytes there would be a strongly coloured picture)."""
+    if fmt is None:
+        return np.zeros(shape, np.uint8)
+    f = np.full(shape, 128, np.uint8)
+    f[: shape[0] * 2 // 3] = 16 if fmt["color_range"] == "limited" else 0
+    return f
+
+
+def _picture_hw(frames, fmt: Optional[Dict[str, str]]):
+    """(H, W) of a decoded window: [T,H,W,3] frames or [T,H*3/2,W] surfaces."""
+    return (frames.shape[1] * 2 // 3, frames.shape[2]) if fmt is not None else (frames.shape[1], frames.shape[2])
+
+
 class GpuDashcamDataset(Dataset):
     """``NvidiaDashcamDataset(metadata_df, base_dirs, fps, duration, is_train, skip_missing, transform,
     sample_strategy, sensor_subdir, time_column)`` work-alike for the frames path.  ``metadata_df`` may be a
     pandas DataFrame or a list of dicts with 'id', 'video_type' and, optionally, 'path' / the time column.
     'sensor' is the accelerometer CSV interpolated at the frame times and cut to the clip's window
     (``sensors.py``; nexar_videos.py:301-346, 453-477), zeros when there is no CSV beside the video - pass
-    ``sensor_resolver`` to find it somewhere else."""
+    ``sensor_resolver`` to find it somewhere else.
+
+    ``pixel_format="nv12"`` / ``"i420"`` (``defer=True`` only): the decoder's ``get_batch`` returns packed YUV 4:2:0
+    surfaces ``[n,H*3/2,W]``; they are what crosses to the main process (half the bytes of RGB) and ``GpuAugLoader``
+    converts them on the device with ``color_matrix`` / ``color_range``."""
 
     def __init__(self, metadata_df, base_dirs=None, fps=10, duration=5, is_train=True, skip_missing=True,
                  transform: Optional[GpuVideoTransform] = None, sample_strategy="random", sensor_subdir="signals",
                  time_column=None, *, decoder: Optional[Callable[[str], Any]] = None,
                  path_resolver: Optional[Callable[[str], Optional[str]]] = None, defer: bool = False,
                  video_fps_lookup: Optional[Callable[[str], float]] = None,
-                 sensor_resolver: Optional[Callable[[str], Optional[str]]] = None):
+                 sensor_resolver: Optional[Callable[[str], Optional[str]]] = None, pixel_format: str = "rgb",
+                 color_matrix: str = "bt601", color_range: str = "limited"):
+        self.source_format = _source_format(defer, pixel_format, color_matrix, color_range)
         rows = metadata_df.to_dict("records") if hasattr(metadata_df, "to_dict") else list(metadata_df)
         self.fps, self.duration, self.is_train = fps, duration, is_train
         self.transform = transform
@@ -209,7 +240,8 @@ class GpuDashcamDataset(Dataset):
             indices, start, end = self._window(reader, row, idx)
             frames = _to_uint8_array(reader.get_batch(indices))
             if len(frames) < need:          # nexar_videos.py:429-433
-                last = frames[-1] if len(frames) else np.zeros(frames.shape[1:] or (720, 1280, 3), np.uint8)
+                default = (1080, 1280) if self.source_format else (720, 1280, 3)
+                last = frames[-1] if len(frames) else _blank_frame(frames.shape[1:] or default, self.source_format)
                 frames = np.concatenate([frames, np.repeat(last[None], need - len(frames), axis=0)], axis=0)
             frames = torch.from_numpy(np.ascontiguousarray(frames[:need]))
             sensor = self._sensor(reader, idx, start, end)
@@ -222,8 +254,11 @@ class GpuDashcamDataset(Dataset):
                     "id": vid}
         if self.defer:
             t = self.transform
-            params = t.sample_params(1, frames.shape[1], frames.shape[2])[0] if t is not None else None
-            return {"frames_u8": frames, "params": params, "sensor": sensor, "target": target, "id": vid, "need": need}
+            params = t.sample_params(1, *_picture_hw(frames, self.source_format))[0] if t is not None else None
+            item = {"frames_u8": frames, "params": params, "sensor": sensor, "target": target, "id": vid, "need": need}
+            if self.source_format:
+                item["format"] = self.source_format
+            return item
         video = frames.permute(3, 0, 1, 2)                      # nexar_videos.py:441
         video = self.transform(video) if self.transform else video.float() / 255.0
         return {"frames": video.permute(1, 2, 3, 0), "sensor": sensor, "target": target, "id": vid}   # :451
@@ -234,12 +269,15 @@ class GpuVideoDataset(Dataset):
     center_time_column, metadata_df)`` work-alike (nexar_complete_with_validation.py:57-234): explicit path / label
     lists, strategies 'random', 'center' and 'metadata_center' (window centred on ``metadata_df[center_time_column]``
     seconds, random window when the value is missing), items ``{'frames', 'target', 'id'}`` - no sensor stream.
-    ``defer=True`` returns the uint8 window plus the clip's parameter record for ``GpuAugLoader``."""
+    ``defer=True`` returns the uint8 window plus the clip's parameter record for ``GpuAugLoader``; ``pixel_format``,
+    ``color_matrix`` and ``color_range`` as for ``GpuDashcamDataset``."""
 
     def __init__(self, video_paths, labels, video_ids=None, fps=10, duration=5, is_train=True,
                  transform: Optional[GpuVideoTransform] = None, sample_strategy="metadata_center",
                  center_time_column=None, metadata_df=None, *, decoder: Optional[Callable[[str], Any]] = None,
-                 defer: bool = False, video_fps_lookup: Optional[Callable[[str], float]] = None):
+                 defer: bool = False, video_fps_lookup: Optional[Callable[[str], float]] = None,
+                 pixel_format: str = "rgb", color_matrix: str = "bt601", color_range: str = "limited"):
+        self.source_format = _source_format(defer, pixel_format, color_matrix, color_range)
         assert len(video_paths) == len(labels), "video_paths and labels must have same length"      # ncwv:94
         assert sample_strategy in ("random", "center", "metadata_center"), \
             "sample_strategy must be 'random', 'center', or 'metadata_center'"                       # ncwv:95-96
@@ -297,7 +335,8 @@ class GpuVideoDataset(Dataset):
                 if len(frames) > 0:
                     frames = np.concatenate([frames, np.repeat(frames[-1][None], need - len(frames), axis=0)], axis=0)
                 else:
-                    frames = np.zeros((need, 720, 1280, 3), np.uint8)
+                    blank = _blank_frame((1080, 1280) if self.source_format else (720, 1280, 3), self.source_format)
+                    frames = np.repeat(blank[None], need, axis=0)
             frames = torch.from_numpy(np.ascontiguousarray(frames[:need]))
         except Exception:
             if self.defer:
@@ -306,8 +345,11 @@ class GpuVideoDataset(Dataset):
             return {"frames": torch.zeros(need, size[0], size[1], 3), "target": label, "id": vid}
         if self.defer:
             t = self.transform
-            params = t.sample_params(1, frames.shape[1], frames.shape[2])[0] if t is not None else None
-            return {"frames_u8": frames, "params": params, "target": label, "id": vid, "need": need}
+            params = t.sample_params(1, *_picture_hw(frames, self.source_format))[0] if t is not None else None
+            item = {"frames_u8": frames, "params": params, "target": label, "id": vid, "need": need}
+            if self.source_format:
+                item["format"] = self.source_format
+            return item
         video = frames.permute(3, 0, 1, 2)                      # ncwv:172
         video = self.transform(video) if self.transform else video.float() / 255.0
         return {"frames": video.permute(1, 2, 3, 0), "target": label, "id": vid}   # ncwv:181
@@ -317,19 +359,23 @@ def deferred_collate(items: Sequence[Dict[str, Any]]) -> Dict[str, Any]:
     """collate_fn for ``defer=True`` datasets.  The uint8 windows are stacked PER SOURCE RESOLUTION (a batch may mix
     720p, 1080p and portrait videos: the reference transforms every clip to cs x cs before collation, so it never
     sees the difference): ``groups`` is a list of ``{'frames_u8': [n,T,H,W,3], 'index': positions in the batch,
-    'params': [...]}``.  Failed items (``frames_u8 is None``) are in no group and become the zero clip.  'sensor' is
-    present for the NvidiaDashcamDataset protocol only."""
+    'params': [...]}``, plus the source ``'format'`` (forward_batch keywords) for YUV surfaces.  Failed items
+    (``frames_u8 is None``) are in no group and become the zero clip.  'sensor' is present for the NvidiaDashcamDataset
+    protocol only."""
     by_shape: Dict[Any, Dict[str, Any]] = {}
     for pos, it in enumerate(items):
         f = it["frames_u8"]
         if f is None:
             continue
-        g = by_shape.setdefault(tuple(f.shape), {"frames": [], "index": [], "params": []})
+        fmt = it.get("format")
+        g = by_shape.setdefault((tuple(f.shape), tuple(sorted(fmt.items())) if fmt else None),
+                                {"frames": [], "index": [], "params": [], "format": fmt})
         g["frames"].append(f)
         g["index"].append(pos)
         g["params"].append(it["params"])
     batch = {   # default_collate: inside a DataLoader worker the stacks go straight into shared memory (deferred.py)
-        "groups": [{"frames_u8": default_collate(g["frames"]), "index": g["index"], "params": g["params"]}
+        "groups": [dict({"frames_u8": default_collate(g["frames"]), "index": g["index"], "params": g["params"]},
+                        **({"format": g["format"]} if g["format"] else {}))
                    for g in by_shape.values()],
         "valid": [it["frames_u8"] is not None for it in items],
         "target": [it["target"] for it in items],
@@ -364,12 +410,12 @@ class GpuAugLoader:
                 g = groups[0]
                 params = g["params"] if all(p is not None for p in g["params"]) else None
                 out = tf.forward_batch(g["frames_u8"].to(self.device, non_blocking=True), params=params,
-                                       out_dtype=self.out_dtype)         # [n,3,T,cs,cs]
+                                       out_dtype=self.out_dtype, **g.get("format", {}))         # [n,3,T,cs,cs]
             else:
                 for g in groups:
                     params = g["params"] if all(p is not None for p in g["params"]) else None
                     res = tf.forward_batch(g["frames_u8"].to(self.device, non_blocking=True), params=params,
-                                           out_dtype=self.out_dtype)
+                                           out_dtype=self.out_dtype, **g.get("format", {}))
                     if out is None:   # failed items stay the reference's all-zeros clip (nexar_videos.py:479-489)
                         out = torch.zeros((n,) + tuple(res.shape[1:]), dtype=res.dtype, device=self.device)
                     out[torch.tensor(g["index"], device=self.device)] = res
