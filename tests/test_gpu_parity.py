@@ -210,26 +210,27 @@ def test_full_size_properties():
                                   "custom_small_s0", "allfx_small_s1"])
 @pytest.mark.parametrize("bands", [0, 1, 3, 7])
 def test_fast_and_general_resize_kernels_agree(name, bands):
-    """The fixed-point input-stationary kernel and the general fp32 kernel both meet the gate, for any banding."""
+    """The fixed-point input-stationary kernel and the general fp32 kernel both meet the gate, for any banding; the
+    serialised launch sequence (variant 2: no programmatic overlap) gives the default's result bit for bit."""
     from vision_collision_detection_b200 import _lib
     c = load_case(name)
     tol = TOL_AFTER if c["cfg"].normalize else TOL_BEFORE
     L = _lib.lib()
     try:
-        L.nexar_set_resize_kernel(1)
+        _lib.check(L.nexar_set_resize_kernel(1))
         general = _run(_tf(c["kwargs"]), c["clip"], c["params"])
-        L.nexar_set_resize_kernel(0)
+        _lib.check(L.nexar_set_resize_kernel(0))
         L.nexar_set_fast_bands(bands)
         fast = _run(_tf(c["kwargs"]), c["clip"], c["params"])
-        L.nexar_set_resize_kernel(3)            # TMA-ring variant: same arithmetic, bulk-copy staging
-        tma = _run(_tf(c["kwargs"]), c["clip"], c["params"])
+        _lib.check(L.nexar_set_resize_kernel(2))
+        serial = _run(_tf(c["kwargs"]), c["clip"], c["params"])
     finally:
         L.nexar_set_resize_kernel(0)
         L.nexar_set_fast_bands(0)
     assert np.abs(general - c["out"]).max() <= tol
     assert np.abs(fast - c["out"]).max() <= tol
     assert np.abs(fast - general).max() <= 2.5e-4      # fixed-point budget: < 3e-5 of full scale, /0.225
-    assert np.array_equal(tma, fast)
+    assert np.array_equal(serial, fast)
 
 
 @pytest.mark.parametrize("h,w,cs", [(720, 1280, 448), (480, 640, 224), (360, 640, 224), (1080, 1920, 320),

@@ -34,6 +34,21 @@ def test_library_loads_and_exports_every_declared_symbol():
     assert L.nexar_sizeof_transform_args() == ctypes.sizeof(_lib.TransformArgs)
 
 
+def test_resize_kernel_knob_refuses_unknown_variants():
+    """0 auto, 1 general, 2 serialised; 4 (fused cluster) only in a build that has it.  Anything else, such as the
+    removed variant 3, used to be accepted and silently run the default path."""
+    L = _lib.lib()
+    try:
+        for v in (0, 1, 2):
+            assert L.nexar_set_resize_kernel(v) == _lib.OK, v
+        assert L.nexar_set_resize_kernel(4) in (_lib.OK, _lib.ERR_UNSUPPORTED)
+        for v in (3, 5, -1, 1 << 20):
+            assert L.nexar_set_resize_kernel(v) == _lib.ERR_INVALID, v
+            assert b"variant" in L.nexar_last_error()
+    finally:
+        assert L.nexar_set_resize_kernel(0) == _lib.OK
+
+
 def test_geometry_matches_reference_table():
     for key, (nh, nw, ph, pw) in META["geometry"].items():
         hw, cs = key.split("->")

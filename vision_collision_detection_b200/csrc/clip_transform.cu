@@ -31,7 +31,11 @@
 static thread_local std::string g_err;
 static thread_local int g_launches = 0;
 // experiment knobs and the optional kernel timing are per calling thread (the library keeps no process-global mutable state)
-static thread_local int g_resize_variant = 0;  // 0 auto, 1 force the general fp32 kernels, 2 no programmatic overlap, 4 fused cluster kernel (optional build)
+// 0 auto, 1 force the general fp32 kernels, 2 no programmatic overlap (K1 -> K2 and K3 -> fix-up serialised by the stream),
+// 4 fused cluster kernel (optional build); nexar_set_resize_kernel refuses anything else.  tests/test_launch_paths.py pins
+// every launch sequence these select (fast / general letterbox, resize-crop, fix-up, blur) against the oracle, and variant
+// 2 against the overlapped default bit for bit.
+static thread_local int g_resize_variant = 0;
 static thread_local int g_fast_bands = 0;      // 0 auto
 static thread_local int g_chunk_clips = 0;     // clips per chunk of an augmented batch (0: the whole batch at once)
 static thread_local int g_geo_variant = 0;     // 0 auto (specialised geometry kernel when the shape allows it), 1 force the general one
@@ -247,6 +251,8 @@ extern "C" size_t nexar_sizeof_transform_args(void) { return sizeof(NexarTransfo
 extern "C" const char* nexar_last_error(void) { return g_err.c_str(); }
 extern "C" int nexar_last_launch_count(void) { return g_launches; }
 extern "C" int nexar_set_resize_kernel(int32_t v) {
+  if (v != 0 && v != 1 && v != 2 && v != 4)
+    return fail(NEXAR_ERR_INVALID, "set_resize_kernel: variant must be 0 (auto), 1 (general), 2 (no overlap) or 4 (fused cluster)");
 #ifndef NEXAR_WITH_FUSED_CLUSTER
   if (v == 4) return fail(NEXAR_ERR_UNSUPPORTED, "set_resize_kernel: variant 4 needs a build with -DNEXAR_WITH_FUSED_CLUSTER");
 #endif
