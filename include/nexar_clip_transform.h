@@ -213,10 +213,10 @@ int nexar_profile_end(float* ms_out, int32_t cap);
 /* Tuning knobs for experiments, per calling thread (the library keeps no process-global mutable state; the profile
  * events above are per thread too).  Resize kernel: 0 = auto (the fixed-point fast kernel when the geometry allows it,
  * followed by the colour and geometry kernels for augmented clips, the colour kernel being a programmatic dependent launch
- * that overlaps the resize kernel's last wave), 1 = force the general fp32 kernels, 2 = as 0 without that overlap, 4 = augmented
- * batches take the fused thread-block-cluster kernel (resize + colour + geometry in one launch; measured slower, compiled
- * only with -DNEXAR_WITH_FUSED_CLUSTER, NEXAR_ERR_UNSUPPORTED otherwise).  Any other value is NEXAR_ERR_INVALID and leaves
- * the setting unchanged.  Bands: the number of
+ * that overlaps the resize kernel's last wave), 1 = force the general fp32 kernels, 2 = as 0 without that overlap.
+ * 4 selected a fused thread-block-cluster kernel (resize + colour + geometry in one launch); it was measured slower and
+ * removed, and 4 now returns NEXAR_ERR_UNSUPPORTED.  Any other value is NEXAR_ERR_INVALID.  A refused value leaves the
+ * setting unchanged.  Bands: the number of
  * row bands each frame is split into by the fast kernel (0 = auto). */
 int nexar_set_resize_kernel(int32_t variant);
 int nexar_set_fast_bands(int32_t bands);

@@ -35,13 +35,13 @@ def test_library_loads_and_exports_every_declared_symbol():
 
 
 def test_resize_kernel_knob_refuses_unknown_variants():
-    """0 auto, 1 general, 2 serialised; 4 (fused cluster) only in a build that has it.  Anything else, such as the
-    removed variant 3, used to be accepted and silently run the default path."""
+    """0 auto, 1 general, 2 serialised.  4, the removed fused cluster kernel, is refused as unsupported.  Anything else,
+    such as the removed variant 3, used to be accepted and silently run the default path."""
     L = _lib.lib()
     try:
         for v in (0, 1, 2):
             assert L.nexar_set_resize_kernel(v) == _lib.OK, v
-        assert L.nexar_set_resize_kernel(4) in (_lib.OK, _lib.ERR_UNSUPPORTED)
+        assert L.nexar_set_resize_kernel(4) == _lib.ERR_UNSUPPORTED
         for v in (3, 5, -1, 1 << 20):
             assert L.nexar_set_resize_kernel(v) == _lib.ERR_INVALID, v
             assert b"variant" in L.nexar_last_error()

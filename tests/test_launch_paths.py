@@ -2,7 +2,7 @@
 
 test_gpu_parity.py pins the path bench.py times (720p -> 224 / 320, fast resize kernel, colour and geometry kernels).
 The other launch sequences have their own instruction streams and store code: the fix-up of clips whose maximum is
-<= 1 (fixup_frame_kernel, which finishes augmented clips with fused_colour_geometry), the general fp32 resize with its
+<= 1 (fixup_frame_kernel, which finishes augmented clips with fixup_colour_geometry), the general fp32 resize with its
 gray slot for those clips, the blur kernel behind the specialised geometry kernel, the resize-crop variant, float
 sources and the two-pass singular factory.  Each case asserts the launch count of the path it claims, writes every
 output layout in fp32 and bf16 into tensors pre-filled with NaN, and compares the fp32 result with the oracle.
@@ -170,7 +170,7 @@ def _fixup_oracle(cs):
 @pytest.mark.parametrize("cs", [224, 320])
 def test_fixup_clips_with_augmentation_on_every_path(cs, variant, path):
     """Clips whose maximum is <= 1 (a failed decode, the neutral surface of an undecodable YUV window) are not divided
-    by 255.  On the fast path fixup_frame_kernel redoes them (fp32 resample + fused_colour_geometry, gray slot 1); on
+    by 255.  On the fast path fixup_frame_kernel redoes them (fp32 resample + fixup_colour_geometry, gray slot 1); on
     the general path pass 1 of resize_general_kernel does, and frame_stats_kernel must read slot 1 for them.  BCTHW
     takes the specialised geometry kernel (125x224 / 180x320 content), the other layouts the general one."""
     from vision_collision_detection_b200 import create_video_transforms

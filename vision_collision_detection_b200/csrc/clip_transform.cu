@@ -31,8 +31,8 @@
 static thread_local std::string g_err;
 static thread_local int g_launches = 0;
 // experiment knobs and the optional kernel timing are per calling thread (the library keeps no process-global mutable state)
-// 0 auto, 1 force the general fp32 kernels, 2 no programmatic overlap (K1 -> K2 and K3 -> fix-up serialised by the stream),
-// 4 fused cluster kernel (optional build); nexar_set_resize_kernel refuses anything else.  tests/test_launch_paths.py pins
+// 0 auto, 1 force the general fp32 kernels, 2 no programmatic overlap (K1 -> K2 and K3 -> fix-up serialised by the stream);
+// nexar_set_resize_kernel refuses anything else.  tests/test_launch_paths.py pins
 // every launch sequence these select (fast / general letterbox, resize-crop, fix-up, blur) against the oracle, and variant
 // 2 against the overlapped default bit for bit.
 static thread_local int g_resize_variant = 0;
@@ -251,11 +251,9 @@ extern "C" size_t nexar_sizeof_transform_args(void) { return sizeof(NexarTransfo
 extern "C" const char* nexar_last_error(void) { return g_err.c_str(); }
 extern "C" int nexar_last_launch_count(void) { return g_launches; }
 extern "C" int nexar_set_resize_kernel(int32_t v) {
-  if (v != 0 && v != 1 && v != 2 && v != 4)
-    return fail(NEXAR_ERR_INVALID, "set_resize_kernel: variant must be 0 (auto), 1 (general), 2 (no overlap) or 4 (fused cluster)");
-#ifndef NEXAR_WITH_FUSED_CLUSTER
-  if (v == 4) return fail(NEXAR_ERR_UNSUPPORTED, "set_resize_kernel: variant 4 needs a build with -DNEXAR_WITH_FUSED_CLUSTER");
-#endif
+  if (v == 4) return fail(NEXAR_ERR_UNSUPPORTED, "set_resize_kernel: variant 4 (the fused cluster kernel) was removed");
+  if (v != 0 && v != 1 && v != 2)
+    return fail(NEXAR_ERR_INVALID, "set_resize_kernel: variant must be 0 (auto), 1 (general) or 2 (no overlap)");
   g_resize_variant = v;
   return NEXAR_OK;
 }
@@ -867,12 +865,8 @@ __device__ __forceinline__ void l2_prefetch_bulk(const void* p, unsigned bytes) 
 // streaming 128-bit load of source bytes (evict-first: every byte is used once)
 __device__ __forceinline__ uint4 ld_stream(const char* base, unsigned off) { return __ldcs((const uint4*)(base + off)); }
 
-#ifndef NEXAR_MINB
-#define NEXAR_MINB 3
-#endif
-#ifndef NEXAR_LOOKAHEAD
-#define NEXAR_LOOKAHEAD 4
-#endif
+constexpr int kFastMinB = 3;    // CTAs per SM of the 256-thread instances (the wider ones take 2)
+constexpr int kLookahead = 4;   // row pairs ahead pushed into L2 by the bulk-prefetch engine (multiple of 4)
 
 // table entry .w bits
 #define NEXAR_E_EMIT 1u
@@ -900,6 +894,8 @@ __device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
 // top bit set, ONE byte permute turns a stored value into the float 1 + q / 32768 (bits 0x3F800000 | q << 8), so the
 // affine gather pays one PRMT per sample instead of an integer-to-float conversion, and the constant 1 is taken out
 // once per pixel (see geometry_kernel).  Quantisation step 3.05e-5 of full scale (gate: 2.25e-4 after the division by std).
+// (Measured: plain uint16 unpacked by I2F.U16 makes the geometry kernel 20 % slower; the conversion pipe runs at a
+// quarter of the ALU rate.)
 constexpr float kQ21 = 2097151.0f;                  // 2^21 - 1
 constexpr float kQ21Inv = 1.0f / 2097151.0f;
 __device__ __forceinline__ uint2 pack_q21(float r, float g, float b) {
@@ -909,21 +905,6 @@ __device__ __forceinline__ uint2 pack_q21(float r, float g, float b) {
   const unsigned qb = __float_as_uint(fmaf(b, kQ21, 8388608.0f)) & 0x1FFFFFu;
   return make_uint2(qr | (qg << 21), (qg >> 11) | (qb << 10));
 }
-#ifndef NEXAR_STAGE2_Q16
-#define NEXAR_STAGE2_Q16 0   // measured: I2F.U16 runs on the quarter-rate conversion pipe, the geometry kernel gets 20 % slower
-#endif
-#if NEXAR_STAGE2_Q16
-// Stage 2 as plain uint16 = round(v * 65535).  A sample is unpacked by ONE conversion instruction that reads a 16-bit half
-// of the register directly (I2F.U16 Rd, Rs.H0 / .H1): no byte permute, and it runs on the conversion pipe instead of the
-// ALU pipe that bounds the geometry kernel.  value = U / 65535.
-constexpr float kQ15 = 65535.0f;
-constexpr float kQ15Magic = 8388608.0f;             // low 16 bits of float_bits(v * 65535 + 2^23) = round(v * 65535)
-constexpr float kS2Inv = 1.0f / 65535.0f;           // sum_content(w * v) = kS2Inv * sum(w * U) + kS2Off * sum(w)
-constexpr float kS2Off = 0.0f;
-__device__ __forceinline__ float q15_r(uint2 v) { return (float)(unsigned short)(v.x & 0xFFFFu); }
-__device__ __forceinline__ float q15_g(uint2 v) { return (float)(unsigned short)(v.x >> 16); }
-__device__ __forceinline__ float q15_b(uint2 v) { return (float)(unsigned short)(v.y & 0xFFFFu); }
-#else
 constexpr float kQ15 = 32767.0f;
 constexpr float kQ15Magic = 8388608.0f + 32768.0f;  // low 16 bits of float_bits(v * 32767 + magic) = 0x8000 | round(v * 32767)
 constexpr float kS2Inv = 32768.0f / 32767.0f;       // v = (F - 1) * kS2Inv: sum_content(w * v) = kS2Inv * sum(w * F) + kS2Off * sum(w)
@@ -931,7 +912,6 @@ constexpr float kS2Off = -kS2Inv;
 __device__ __forceinline__ float q15_r(uint2 v) { return __uint_as_float(__byte_perm(v.x, 0x3F000000u, 0x7104)); }
 __device__ __forceinline__ float q15_g(uint2 v) { return __uint_as_float(__byte_perm(v.x, 0x3F000000u, 0x7324)); }
 __device__ __forceinline__ float q15_b(uint2 v) { return __uint_as_float(__byte_perm(v.y, 0x3F000000u, 0x7104)); }
-#endif
 __device__ __forceinline__ uint2 pack_q15(float r, float g, float b) {
   const unsigned qr = __float_as_uint(fmaf(r, kQ15, kQ15Magic));
   const unsigned qg = __float_as_uint(fmaf(g, kQ15, kQ15Magic));
@@ -939,32 +919,15 @@ __device__ __forceinline__ uint2 pack_q15(float r, float g, float b) {
   return make_uint2(__byte_perm(qr, qg, 0x5410), qb & 0xFFFFu);
 }
 
-// thread-block cluster barrier (all threads of all CTAs of the cluster); release/acquire at cluster scope orders the
-// global-memory writes before the arrive with the reads after the wait
-#ifndef NEXAR_EXP
-#define NEXAR_EXP 0   // timing experiments only: 1 skip phase B, 2 skip phase C, 4 CTA barriers instead of cluster barriers
-#endif
-__device__ __forceinline__ void cluster_sync_all() {
-  if (NEXAR_EXP & 4) { __syncthreads(); return; }
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-
-template <typename DstT, int NT, bool CLUSTER>
-__device__ __forceinline__ void fused_colour_geometry(const DevPlan& P, const KArgs& A, const NexarClipParams* cp,
-                                                      unsigned flags, int frame, int clip, int t, int band, int nb,
-                                                      const Box& B, int i0, int i1, int slot);
 __device__ __forceinline__ void write_frame_info(const DevPlan& P, const KArgs& A, int frame, int slot, int nbands);
 
-// FUSED: the nb bands of a frame form one thread-block cluster; after the resize the cluster goes on, in the same
-// launch, with the colour chain (in place on the band's own rows) and the affine gather + store (see
-// fused_colour_geometry), so the augmented path is ONE kernel and the intermediate is consumed while it is L2-hot.
-template <int KX, int NT, int MINB, int RS, typename DstT, bool FUSED, bool AL4>
+template <int KX, int NT, int MINB, int RS, typename DstT, bool AL4>
 __global__ void __launch_bounds__(NT, MINB)
 resize_fast_kernel(const __grid_constant__ DevPlan P, const __grid_constant__ KArgs A) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ unsigned long long red[32];
   __shared__ __align__(8) unsigned long long rowbar;  // "row staged" barrier: one arrival per warp, waited on one pair later
-  constexpr int LA = NEXAR_LOOKAHEAD;  // row pairs ahead pushed into L2 by the bulk-prefetch engine (multiple of 4)
+  constexpr int LA = kLookahead;
   const int tid = threadIdx.x;
   // Programmatic dependent launch: the colour kernel's CTAs may be scheduled as soon as every CTA of this grid has
   // started, i.e. into the SM slots this grid's last wave leaves empty; they synchronise per frame through frame_done.
@@ -1225,20 +1188,15 @@ resize_fast_kernel(const __grid_constant__ DevPlan P, const __grid_constant__ KA
     const unsigned long long s = block_sum((unsigned long long)gsum, red);
     if (tid == 0) A.gray_partial[((size_t)(scale == 1.0f) * A.n_frames + frame) * kMaxBands + band] = s;
   }
-  if constexpr (FUSED) {
-    // aug is a property of the clip, hence uniform over the cluster: either every CTA of it takes the barriers or none
-    if (aug) fused_colour_geometry<DstT, NT, true>(P, A, cp, flags, frame, clip, t, band, nb, B, i0, i1, 0);
-  } else {
-    // K1.5 folded in: the last band of the frame to get here publishes the frame's constants for K2 / K3 (gray mean of
-    // the "divided by 255" pass; clips whose maximum turns out to be <= 1 are redone by fixup_frame_kernel anyway)
-    if (A.finfo_by_k1 && tid == 0) {
+  // K1.5 folded in: the last band of the frame to get here publishes the frame's constants for K2 / K3 (gray mean of
+  // the "divided by 255" pass; clips whose maximum turns out to be <= 1 are redone by fixup_frame_kernel anyway)
+  if (A.finfo_by_k1 && tid == 0) {
+    __threadfence();
+    if (atomicAdd(&A.frame_done[frame], 1u) == (unsigned)nb - 1u) {
       __threadfence();
-      if (atomicAdd(&A.frame_done[frame], 1u) == (unsigned)nb - 1u) {
-        __threadfence();
-        write_frame_info(P, A, frame, 0, nb);
-        __threadfence();
-        atomicExch(&A.frame_done[frame], kFrameReady);   // published: intermediate rows, clip flag and FrameInfo are visible
-      }
+      write_frame_info(P, A, frame, 0, nb);
+      __threadfence();
+      atomicExch(&A.frame_done[frame], kFrameReady);   // published: intermediate rows, clip flag and FrameInfo are visible
     }
   }
 }
@@ -1341,9 +1299,7 @@ __global__ void __launch_bounds__(128) frame_stats_kernel(const __grid_constant_
 // K2: contrast/saturation/hue in place on the frame's content box (which always fills the
 // [bh][bw] allocation: letterbox shows every resized row, a crop shows exactly cs x cs of them), 8-byte q15 pixels.
 constexpr int kColourPerThread = 8;
-#ifndef NEXAR_COL_MINB
-#define NEXAR_COL_MINB 6
-#endif
+constexpr int kColMinB = 6;   // CTAs per SM (8 measured: no change)
 // Wait until the resize kernel has published a frame (overlapped launch only).  Bounded: a stuck wait traps instead of
 // hanging the device.
 __device__ __forceinline__ void wait_frame_ready(const unsigned* flag) {
@@ -1362,7 +1318,7 @@ __device__ __forceinline__ void wait_frame_ready(const unsigned* flag) {
   }
 }
 
-__global__ void __launch_bounds__(256, NEXAR_COL_MINB) colour_kernel(const __grid_constant__ DevPlan P, const __grid_constant__ KArgs A) {
+__global__ void __launch_bounds__(256, kColMinB) colour_kernel(const __grid_constant__ DevPlan P, const __grid_constant__ KArgs A) {
   __shared__ unsigned go;
   int frame;
   if (A.overlap) {
@@ -1458,18 +1414,6 @@ __device__ __forceinline__ void point_effects(float& r, float& g, float& b, cons
 enum { GEO_GENERAL = 0, GEO_FILL = 1, GEO_INTERIOR = 2 };
 constexpr unsigned kTailFlags = NEXAR_GRAYSCALE | NEXAR_NOISE | NEXAR_BLUR | NEXAR_POSTERIZE | NEXAR_SOLARIZE | NEXAR_INVERT | NEXAR_CUTOUT;
 
-// ---------------------------------------------------------------------------------
-// Fused tail of resize_fast_kernel<..., FUSED = true>: K2 + K3 of one frame inside the cluster that resized it.
-//   phase B  every CTA runs contrast -> saturation -> hue in place on the rows of the intermediate its own band wrote
-//            (needs the frame's gray mean: the band sums are exchanged through global memory and the first cluster barrier);
-//   phase C  after the second cluster barrier every CTA produces a share of the OUTPUT rows (groups of four rows dealt round
-//            robin, so that pad and content rows are spread evenly): a warp owns 16 x 4 output pixels, two horizontally
-//            adjacent pixels per lane (one 32-bit bf16x2 / 64-bit float2 store per channel), classified FILL / INTERIOR /
-//            general exactly like geometry_kernel; the four neighbours are 8-byte loads of the q15 intermediate (L2 / L1
-//            hits: the cluster wrote them microseconds ago), unpacked with one PRMT per sample:
-//              sum_canvas(w * img) = pad * (m - wc) + k * sum_content(w * F) - k * wc,   F = 1 + q / 32768, k = 32768 / 32767
-//            with m the interpolated ones-mask and wc the total weight of the content neighbours; out = m * that (tv fill = 0).
-// ---------------------------------------------------------------------------------
 struct GeoPx {
   int o00, o01, o10, o11;                     // pixel offsets from the frame's canvas origin
   float w00, w01, w10, w11, m, wc;
@@ -1505,24 +1449,31 @@ __device__ __forceinline__ void store_pair<__nv_bfloat16>(__nv_bfloat16* p, floa
   asm volatile("st.global.b32 [%0], %1;" ::"l"(p), "r"(*(const unsigned*)&h) : "memory");
 }
 
-template <typename DstT, int NT, bool CLUSTER>
-__device__ __forceinline__ void fused_colour_geometry(const DevPlan& P, const KArgs& A, const NexarClipParams* cp,
-                                                      unsigned flags, int frame, int clip, int t, int band, int nb,
-                                                      const Box& B, int i0, int i1, int slot) {
+// ---------------------------------------------------------------------------------
+// Augmentation tail of fixup_frame_kernel: K1.5 + K2 + K3 of one frame inside the CTA of 256 threads that has just
+// resampled all of it (rows B.i_lo .. B.i_hi, gray sum in slot 1).
+//   phase B  contrast -> saturation -> hue in place on the frame's rows of the intermediate;
+//   phase C  the OUTPUT in tiles of 32 x 4 pixels pulled from a shared counter: a warp owns one tile at a time, two
+//            horizontally adjacent pixels per lane (one 32-bit bf16x2 / 64-bit float2 store per channel), classified
+//            FILL / INTERIOR / general exactly like geometry_kernel; the four neighbours are 8-byte loads of the q15
+//            intermediate (L2 / L1 hits: this CTA wrote them microseconds ago), unpacked with one PRMT per sample:
+//              sum_canvas(w * img) = pad * (m - wc) + k * sum_content(w * F) - k * wc,   F = 1 + q / 32768, k = 32768 / 32767
+//            with m the interpolated ones-mask and wc the total weight of the content neighbours; out = m * that (tv fill = 0).
+// ---------------------------------------------------------------------------------
+template <typename DstT>
+__device__ __forceinline__ void fixup_colour_geometry(const DevPlan& P, const KArgs& A, const NexarClipParams* cp,
+                                                      unsigned flags, int frame, int clip, int t, const Box& B) {
+  constexpr int NT = 256;
   __shared__ float fconst[4];  // pad colour after the colour chain, contrast_q * gray mean
   __shared__ unsigned char tile_cls[kMaxTileClasses];
   __shared__ int tile_next[1];
   const int tid = threadIdx.x;
-  // CLUSTER: the nb bands of the frame are the CTAs of one cluster; otherwise one CTA owns the whole frame (nb == 1)
-  auto sync_all = [&]() {
-    if (CLUSTER) cluster_sync_all();
-    else { __threadfence_block(); __syncthreads(); }
-  };
-  sync_all();                  // every band's gray sum is in global memory
+  __threadfence_block();       // the frame's gray sum is in global memory
+  __syncthreads();
   ColourParams c;
   c.contrast = cp->contrast; c.saturation = cp->saturation; c.saturation_q = cp->saturation_q; c.hue6 = 6.0f * cp->hue;
   if (tid == 0) {
-    c.cmean = __fmul_rn(cp->contrast_q, frame_mean(A, P, frame, slot, nb));
+    c.cmean = __fmul_rn(cp->contrast_q, frame_mean(A, P, frame, 1, 1));
     float r = 0.0f, g = 0.0f, b = 0.0f;
     colour_chain(r, g, b, c);
     fconst[0] = r; fconst[1] = g; fconst[2] = b; fconst[3] = c.cmean;
@@ -1530,40 +1481,38 @@ __device__ __forceinline__ void fused_colour_geometry(const DevPlan& P, const KA
   __syncthreads();
   const float padr = fconst[0], padg = fconst[1], padb = fconst[2];
   c.cmean = fconst[3];
-  // ---- phase B: colour chain in place on this band's rows -------------------------------------------------------
-  if (!(NEXAR_EXP & 1)) {
-    const int nrows = i1 - i0, bwid = B.bx1 - B.bx0;
-    uint2* const rows = A.inter + ((int64_t)frame * A.bh + (i0 + B.oy - B.by0)) * A.bw;
-    if (bwid == A.bw) {  // the content box fills the allocation (always, for a letterbox): one flat, coalesced sweep
-      const int n = nrows * A.bw;
-      constexpr int U = 4;
-      for (int e0 = tid; e0 < n; e0 += U * NT) {
-        uint2 v[U];
+  // ---- phase B: colour chain in place on the frame's rows -------------------------------------------------------
+  const int nrows = B.i_hi - B.i_lo, bwid = B.bx1 - B.bx0;
+  uint2* const rows = A.inter + ((int64_t)frame * A.bh + (B.i_lo + B.oy - B.by0)) * A.bw;
+  if (bwid == A.bw) {  // the content box fills the allocation (always, for a letterbox): one flat, coalesced sweep
+    const int n = nrows * A.bw;
+    constexpr int U = 4;
+    for (int e0 = tid; e0 < n; e0 += U * NT) {
+      uint2 v[U];
 #pragma unroll
-        for (int k = 0; k < U; ++k)
-          if (e0 + k * NT < n) v[k] = rows[e0 + k * NT];
+      for (int k = 0; k < U; ++k)
+        if (e0 + k * NT < n) v[k] = rows[e0 + k * NT];
 #pragma unroll
-        for (int k = 0; k < U; ++k)
-          if (e0 + k * NT < n) {
-            float r, g, b;
-            colour_chain_q21(v[k], r, g, b, c);
-            rows[e0 + k * NT] = pack_q15(r, g, b);
-          }
-      }
-    } else {
-      for (int row = tid >> 5; row < nrows; row += NT / 32)
-        for (int col = tid & 31; col < bwid; col += 32) {
-          uint2* q = rows + row * A.bw + col;
-          const uint2 v = *q;
+      for (int k = 0; k < U; ++k)
+        if (e0 + k * NT < n) {
           float r, g, b;
-          colour_chain_q21(v, r, g, b, c);
-          *q = pack_q15(r, g, b);
+          colour_chain_q21(v[k], r, g, b, c);
+          rows[e0 + k * NT] = pack_q15(r, g, b);
         }
     }
+  } else {
+    for (int row = tid >> 5; row < nrows; row += NT / 32)
+      for (int col = tid & 31; col < bwid; col += 32) {
+        uint2* q = rows + row * A.bw + col;
+        const uint2 v = *q;
+        float r, g, b;
+        colour_chain_q21(v, r, g, b, c);
+        *q = pack_q15(r, g, b);
+      }
   }
   // ---- tile classes of phase C (geometry only: done before the barrier so that it overlaps the wait) -------------------
   const int ngroups = (P.cs + 3) >> 2, tiles_x = (P.cs + 31) >> 5;
-  const int ntiles = (band < ngroups ? (ngroups - band + nb - 1) / nb : 0) * tiles_x;
+  const int ntiles = max(ngroups, 0) * tiles_x;
   auto classify = [&](int tx, int ty0) -> int {
     if (!(flags & NEXAR_AFFINE)) return GEO_GENERAL;
     const float fcs = (float)P.cs, half = 0.5f * fcs;
@@ -1584,14 +1533,15 @@ __device__ __forceinline__ void fused_colour_geometry(const DevPlan& P, const KA
   };
   for (int tile = tid; tile < min(ntiles, kMaxTileClasses); tile += NT) {
     const int gk = tile / tiles_x, tx = tile - gk * tiles_x;
-    tile_cls[tile] = (unsigned char)classify(tx, (band + gk * nb) * 4);
+    tile_cls[tile] = (unsigned char)classify(tx, gk * 4);
   }
   if (tid == 0) *tile_next = 0;
-  sync_all();                  // the whole frame is colour-adjusted
+  __threadfence_block();       // the whole frame is colour-adjusted
+  __syncthreads();
   // ---- phase C: affine gather + effects + normalise + store -------------------------------------------------------
-  // Warp tile = 32 x 4 output pixels: lane -> (x pair = lane & 15, row = lane >> 4), two passes two rows apart.  The CTA's
-  // tiles (its row groups x the tile columns) were classified once, into shared memory, before the barrier above; the
-  // warps then pull tiles from a shared counter (FILL tiles cost a few stores, general ones about 700 instructions).
+  // Warp tile = 32 x 4 output pixels: lane -> (x pair = lane & 15, row = lane >> 4), two passes two rows apart.  The
+  // frame's tiles (its row groups x the tile columns) were classified once, into shared memory, before the barrier above;
+  // the warps then pull tiles from a shared counter (FILL tiles cost a few stores, general ones about 700 instructions).
   const int cs = P.cs;
   const int lane = tid & 31;
   const float half = (float)cs * 0.5f, fcs = (float)cs;
@@ -1677,9 +1627,9 @@ __device__ __forceinline__ void fused_colour_geometry(const DevPlan& P, const KA
     int tile = 0;
     if (lane == 0) tile = atomicAdd(tile_next, 1);
     tile = __shfl_sync(0xffffffffu, tile, 0);
-    if (tile >= ((NEXAR_EXP & 2) ? 0 : ntiles)) break;
+    if (tile >= ntiles) break;
     const int gk = tile / tiles_x, tx = tile - gk * tiles_x;
-    const int ty0 = (band + gk * nb) * 4;
+    const int ty0 = gk * 4;
     const int cls = tile < kMaxTileClasses ? (int)tile_cls[tile] : classify(tx, ty0);
     const int x = tx * 32 + lx;
     const bool has2 = x + 1 < cs;
@@ -1740,7 +1690,7 @@ __device__ __forceinline__ void fused_colour_geometry(const DevPlan& P, const KA
 
 // Second pass of the fast path: the clips whose maximum was <= 1 are NOT divided by 255 (nexar_video_aug.py:814).  Rare, so
 // it is ONE launch of one CTA per frame that exits at once for every other clip: the general fp32 resample of the whole
-// frame (values in [0,1] are below the resolution of the fixed-point staging) and, for augmented clips, the fused tail.
+// frame (values in [0,1] are below the resolution of the fixed-point staging) and, for augmented clips, fixup_colour_geometry.
 template <typename SrcT, typename DstT>
 __global__ void __launch_bounds__(256) fixup_frame_kernel(const __grid_constant__ DevPlan P, const __grid_constant__ KArgs A) {
   extern __shared__ float vbuf[];  // [src_w*3]
@@ -1756,7 +1706,7 @@ __global__ void __launch_bounds__(256) fixup_frame_kernel(const __grid_constant_
   const unsigned flags = cp->flags;
   if (flags & NEXAR_AUG) {
     const Box B = clip_box(P, cp->crop_dy, cp->crop_dx, (flags & NEXAR_FLIP) != 0u);
-    fused_colour_geometry<DstT, 256, false>(P, A, cp, flags, frame, clip, frame - clip * A.T, 0, 1, B, B.i_lo, B.i_hi, 1);
+    fixup_colour_geometry<DstT>(P, A, cp, flags, frame, clip, frame - clip * A.T, B);
   }
 }
 
@@ -1773,22 +1723,11 @@ __global__ void __launch_bounds__(256) fixup_frame_kernel(const __grid_constant_
 //   sum_canvas(w * img) = pad * (m - wc) + k * sum_content(w * F) - k * wc,   F = 1 + q / 32768, k = 32768 / 32767
 // and out = m * that (torchvision's fill = 0 multiplies the zero-padded sample by the interpolated mask once more).
 // Offsets inside one clip of the intermediate and one frame of the destination are 32-bit (checked on the host).
-#ifndef NEXAR_GEO_FRAMES
-#define NEXAR_GEO_FRAMES 4
-#endif
-constexpr int kGeoFrames = NEXAR_GEO_FRAMES;  // frames of one clip per CTA
-#ifndef NEXAR_GEO_MINB
-#define NEXAR_GEO_MINB 4
-#endif
-#ifndef NEXAR_GEO_PASSES
-#define NEXAR_GEO_PASSES 2   // row passes per warp: the warp tile is 32 x (2 * passes) pixels
-#endif
-#ifndef NEXAR_GEO_OPAQUE
-#define NEXAR_GEO_OPAQUE 1   // per-frame base pointers made opaque to the compiler (cheaper addresses, loads stay per frame)
-#endif
-constexpr int kGeoPasses = NEXAR_GEO_PASSES;
+constexpr int kGeoFrames = 4;   // frames of one clip per CTA
+constexpr int kGeoMinB = 4;     // CTAs per SM
+constexpr int kGeoPasses = 2;   // row passes per warp: the warp tile is 32 x (2 * passes) pixels
 template <typename DstT, bool TAIL>
-__global__ void __launch_bounds__(256, NEXAR_GEO_MINB) geometry_kernel(const __grid_constant__ DevPlan P, const __grid_constant__ KArgs A) {
+__global__ void __launch_bounds__(256, kGeoMinB) geometry_kernel(const __grid_constant__ DevPlan P, const __grid_constant__ KArgs A) {
   asm volatile("griddepcontrol.launch_dependents;");   // the fix-up launch may drain through this grid's last wave
   const int nchunk = (A.T + kGeoFrames - 1) / kGeoFrames;
   const int clip = blockIdx.z / nchunk;
@@ -1908,10 +1847,8 @@ __global__ void __launch_bounds__(256, NEXAR_GEO_MINB) geometry_kernel(const __g
       const float4 padv = __ldg(fi4 + 5 * f);  // FrameInfo is five float4; the pad colour comes first
       const uint2* fr = (const uint2*)((const char*)fr0 + f * fbytes);
       DstT* ob = (DstT*)((char*)obase0 + f * stbytes);
-      if (NEXAR_GEO_OPAQUE) {
-        asm volatile("" : "+l"(fr));
-        asm volatile("" : "+l"(ob));
-      }
+      asm volatile("" : "+l"(fr));
+      asm volatile("" : "+l"(ob));
       float rr[2] = {padv.x, padv.x}, gg[2] = {padv.y, padv.y}, bb[2] = {padv.z, padv.z};
       if (cls != GEO_FILL) {
         uint2 v[2][4];
@@ -1999,69 +1936,23 @@ __global__ void __launch_bounds__(256, NEXAR_GEO_MINB) geometry_kernel(const __g
 //   * the blend runs on packed fp32 pairs (FFMA2: the two pixels of a lane, channel by channel) and the interior
 //     class folds the q15 scale and the normalisation into one multiply-add per channel.
 // Same formulas and the same per-pixel operation order as geometry_kernel, which stays the general fallback.
-#ifndef NEXAR_GEO2_FRAMES
-#define NEXAR_GEO2_FRAMES 8
-#endif
-#ifndef NEXAR_GEO2_MINB
-#define NEXAR_GEO2_MINB 6
-#endif
-#ifndef NEXAR_GEO2_AHEAD
-#define NEXAR_GEO2_AHEAD 0   // groups ahead whose frames the first tile column prefetches into L2 (0: off)
-#endif
-#ifndef NEXAR_GEO2_REVERSE
-#define NEXAR_GEO2_REVERSE 1   // measured: 0.3952 -> 0.3935 ms at cfg2
-#endif
-#ifndef NEXAR_GEO2_XU
-#define NEXAR_GEO2_XU 0      // channels (0..2: none, B, G + B) unpacked through the conversion pipe instead of the ALU pipe
-#endif
-#ifndef NEXAR_GEO2_WARPS
-#define NEXAR_GEO2_WARPS 4   // warps per CTA: the CTA tile is 32 x (4 * warps) pixels (3 / 4 / 5 / 8 measured: 4 is best by 1 %)
-#endif
+constexpr int kGeo2Frames = 8;   // frames of one clip per CTA
+constexpr int kGeo2MinB = 6;     // CTAs per SM (5 / 6 / 7 measured: 6 is best, 0.393 vs 0.399 / 0.399 ms)
+constexpr int kGeo2Warps = 4;    // warps per CTA: the CTA tile is 32 x (4 * warps) pixels (3 / 4 / 5 / 8 measured: 4 is best by 1 %)
 __device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) { return __ffma2_rn(a, b, c); }
 __device__ __forceinline__ float2 fmul2(float2 a, float2 b) { return __fmul2_rn(a, b); }
-#ifndef NEXAR_GEO2_EXP
-#define NEXAR_GEO2_EXP 0
-#endif
-#if NEXAR_GEO2_EXP & 2   /* timing experiment: no loads */
-__device__ __forceinline__ uint2 ldg_u2(const uint2* p) { return make_uint2((unsigned)(size_t)p, (unsigned)((size_t)p >> 3)); }
-#else
-__device__ __forceinline__ uint2 ldg_u2(const uint2* p) { return __ldg(p); }
-#endif
 __device__ __forceinline__ void l2_prefetch_line(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-#ifndef NEXAR_GEO2_L2PF
-#define NEXAR_GEO2_L2PF 1   // first frame of the group whose rows are prefetched into L2 at the start of a pass (0: off)
-#endif
 
 template <typename DstT, bool TAIL, int BH, int BW, int CS>
-__global__ void __launch_bounds__(32 * NEXAR_GEO2_WARPS, NEXAR_GEO2_MINB) geometry_spec_kernel(const __grid_constant__ DevPlan P, const __grid_constant__ KArgs A) {
+__global__ void __launch_bounds__(32 * kGeo2Warps, kGeo2MinB) geometry_spec_kernel(const __grid_constant__ DevPlan P, const __grid_constant__ KArgs A) {
   static_assert(BH >= 2 && BW >= 2, "the clamped 2 x 2 window needs a 2 x 2 box");
-  constexpr int NF = NEXAR_GEO2_FRAMES;
+  constexpr int NF = kGeo2Frames;
   constexpr int FPX = BH * BW;   // pixels of one intermediate frame
   constexpr int OPX = CS * CS;   // elements of one output plane
   asm volatile("griddepcontrol.launch_dependents;");   // the fix-up launch may drain through this grid's last wave
   const int ngroup = (A.T + NF - 1) / NF;
-#if NEXAR_GEO2_REVERSE
-  const int bz = (int)(gridDim.z - 1u - blockIdx.z);   // last frame groups first: the colour kernel wrote them last (L2)
-#else
-  const int bz = (int)blockIdx.z;
-#endif
-#if NEXAR_GEO2_AHEAD
-  // Group prefetch: the CTAs of the first tile column pull the frames of the group that will be processed about one wave
-  // from now (NEXAR_GEO2_AHEAD groups further on) from DRAM into L2 with the bulk-copy engine, one slice of a frame per
-  // CTA row and thread: by the time that group's tiles gather from it, every load is an L2 hit.
-  if (blockIdx.x == 0 && threadIdx.x < NF) {
-    const int gz = bz - NEXAR_GEO2_AHEAD * (NEXAR_GEO2_REVERSE ? 1 : -1);
-    if (gz >= 0 && gz < (int)gridDim.z) {
-      const int c2 = gz / ngroup, t2 = (gz - c2 * ngroup) * NF + (int)threadIdx.x;
-      if (t2 < A.T) {
-        const char* base = (const char*)(A.inter + (int64_t)(c2 * A.T + t2) * FPX);
-        const int per = ((FPX * 8 / (int)gridDim.y) + 15) & ~15, off = (int)blockIdx.y * per;
-        const int n = min(per, FPX * 8 - off);
-        if (n > 0) l2_prefetch_bulk(base + off, (unsigned)n);
-      }
-    }
-  }
-#endif
+  // last frame groups first: the colour kernel wrote them last (L2).  Measured: 0.3952 -> 0.3935 ms at cfg2
+  const int bz = (int)(gridDim.z - 1u - blockIdx.z);
   const int clip = bz / ngroup;
   const int t0 = (bz - clip * ngroup) * NF;
   const int nfr = min(NF, A.T - t0);
@@ -2075,7 +1966,7 @@ __global__ void __launch_bounds__(32 * NEXAR_GEO2_WARPS, NEXAR_GEO2_MINB) geomet
   // the 32 lanes of a load read 32 consecutive 8-byte pixels of one source row (two or three 128-byte lines) and the
   // 32 lanes of a store write 32 consecutive elements, which halves the L1 wavefronts of a two-pixels-per-lane row layout.
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int tx0 = blockIdx.x * 32, ty0 = (blockIdx.y * NEXAR_GEO2_WARPS + warp) * 4;
+  const int tx0 = blockIdx.x * 32, ty0 = (blockIdx.y * kGeo2Warps + warp) * 4;
   const int x = tx0 + lane;
   if (ty0 >= CS) return;
   const float4 q2 = __ldg(fi4 + 2);
@@ -2105,17 +1996,10 @@ __global__ void __launch_bounds__(32 * NEXAR_GEO2_WARPS, NEXAR_GEO2_MINB) geomet
   const int64_t osc = A.sc;
   const bool tail_fx = TAIL && (flags & kTailFlags) != 0u;
   const float nsr = A.nscale[0], nsg = A.nscale[1], nsb = A.nscale[2], nbr = A.nbias[0], nbg = A.nbias[1], nbb = A.nbias[2];
-  // Unpacking: a byte permute per sample (ALU pipe, which bounds this kernel) - except for NEXAR_GEO2_XU of the three
-  // channels, which go through I2F.U16 on the otherwise idle conversion pipe: the stored 0x8000 | q reads as 32768 * F there,
-  // and the factor goes into that channel's constants.
-  constexpr float kXg = (NEXAR_GEO2_XU >= 2 && !NEXAR_STAGE2_Q16) ? 1.0f / 32768.0f : 1.0f;
-  constexpr float kXb = (NEXAR_GEO2_XU >= 1 && !NEXAR_STAGE2_Q16) ? 1.0f / 32768.0f : 1.0f;
-  auto ur = [](uint2 v) { return q15_r(v); };
-  auto ug = [](uint2 v) { return kXg != 1.0f ? (float)(unsigned short)(v.x >> 16) : q15_g(v); };
-  auto ub = [](uint2 v) { return kXb != 1.0f ? (float)(unsigned short)(v.y & 0xFFFFu) : q15_b(v); };
-  constexpr float kInvR = kS2Inv, kInvG = kS2Inv * kXg, kInvB = kS2Inv * kXb;
+  // Unpacking: a byte permute per sample (ALU pipe, which bounds this kernel).  Measured: sending the B channel through
+  // I2F.U16 on the conversion pipe instead changes nothing, the G and B channels lose 2 %.
   // interior class: out = s * (k * ns) + (nb - k * ns), s = sum(w * F), F = 1 + q / 32768, k = 32768 / 32767
-  const float kir = kInvR * nsr, kig = kInvG * nsg, kib = kInvB * nsb;
+  const float kir = kS2Inv * nsr, kig = kS2Inv * nsg, kib = kS2Inv * nsb;
   const float cir = fmaf(kS2Off, nsr, nbr), cig = fmaf(kS2Off, nsg, nbg), cib = fmaf(kS2Off, nsb, nbb);
   const float xb = (float)x - half + 0.5f;
   const float xg0 = xb * g0, xg3 = xb * g3;
@@ -2186,31 +2070,24 @@ __global__ void __launch_bounds__(32 * NEXAR_GEO2_WARPS, NEXAR_GEO2_MINB) geomet
     DstT* const pog = por + osc;
     DstT* const pob = pog + osc;
     auto put = [&](DstT* p, int f, float va, float vb) {   // one channel of the lane's two pixels, frame f of the group
-#if NEXAR_GEO2_EXP & 1   /* timing experiment: no stores (unless NaN, to keep the arithmetic alive) */
-      if (va != va || vb != vb)
-#endif
-      {
       store_out_global<DstT>(p + f * OPX, va);
       if (has2) store_out_global<DstT>(p + (f * OPX + CS), vb);
-      }
     };
     // ---- the frames of the group (fully unrolled: every address below is [pointer + immediate]); the eight neighbour
     // loads of frame f + 1 are issued before frame f is blended ----
     uint2 va[2][4], vb[2][4];
     if (cls != GEO_FILL) {
-#if NEXAR_GEO2_L2PF
       // pull the three source rows this lane needs from the LATER frames of the group into L2 now (the intermediate of a
       // whole batch does not stay L2-resident behind the 1.4 GB source stream): their loads then find an L2 hit
 #pragma unroll
-      for (int f = NEXAR_GEO2_L2PF; f < NF; ++f)
+      for (int f = 1; f < NF; ++f)
         if (f < nfr) {
           l2_prefetch_line(pa + f * FPX);
           l2_prefetch_line(pa + f * FPX + BW);
           l2_prefetch_line(pb + f * FPX + BW);
         }
-#endif
-      va[0][0] = ldg_u2(pa); va[0][1] = ldg_u2(pa + 1); va[0][2] = ldg_u2(pa + BW); va[0][3] = ldg_u2(pa + BW + 1);
-      vb[0][0] = ldg_u2(pb); vb[0][1] = ldg_u2(pb + 1); vb[0][2] = ldg_u2(pb + BW); vb[0][3] = ldg_u2(pb + BW + 1);
+      va[0][0] = __ldg(pa); va[0][1] = __ldg(pa + 1); va[0][2] = __ldg(pa + BW); va[0][3] = __ldg(pa + BW + 1);
+      vb[0][0] = __ldg(pb); vb[0][1] = __ldg(pb + 1); vb[0][2] = __ldg(pb + BW); vb[0][3] = __ldg(pb + BW + 1);
     }
 #pragma unroll
     for (int f = 0; f < NF; ++f) {
@@ -2223,23 +2100,23 @@ __global__ void __launch_bounds__(32 * NEXAR_GEO2_WARPS, NEXAR_GEO2_MINB) geomet
           const uint2* qb = pb + (f + 1) * FPX;
           uint2* na = va[(f + 1) & 1];
           uint2* nb = vb[(f + 1) & 1];
-          na[0] = ldg_u2(qa); na[1] = ldg_u2(qa + 1); na[2] = ldg_u2(qa + BW); na[3] = ldg_u2(qa + BW + 1);
-          nb[0] = ldg_u2(qb); nb[1] = ldg_u2(qb + 1); nb[2] = ldg_u2(qb + BW); nb[3] = ldg_u2(qb + BW + 1);
+          na[0] = __ldg(qa); na[1] = __ldg(qa + 1); na[2] = __ldg(qa + BW); na[3] = __ldg(qa + BW + 1);
+          nb[0] = __ldg(qb); nb[1] = __ldg(qb + 1); nb[2] = __ldg(qb + BW); nb[3] = __ldg(qb + BW + 1);
         }
         const uint2* ca = va[f & 1];
         const uint2* cb = vb[f & 1];
-        float2 sr = fmul2(make_float2(ur(ca[0]), ur(cb[0])), w00);
-        float2 sg = fmul2(make_float2(ug(ca[0]), ug(cb[0])), w00);
-        float2 sb = fmul2(make_float2(ub(ca[0]), ub(cb[0])), w00);
-        sr = ffma2(make_float2(ur(ca[1]), ur(cb[1])), w01, sr);
-        sg = ffma2(make_float2(ug(ca[1]), ug(cb[1])), w01, sg);
-        sb = ffma2(make_float2(ub(ca[1]), ub(cb[1])), w01, sb);
-        sr = ffma2(make_float2(ur(ca[2]), ur(cb[2])), w10, sr);
-        sg = ffma2(make_float2(ug(ca[2]), ug(cb[2])), w10, sg);
-        sb = ffma2(make_float2(ub(ca[2]), ub(cb[2])), w10, sb);
-        sr = ffma2(make_float2(ur(ca[3]), ur(cb[3])), w11, sr);
-        sg = ffma2(make_float2(ug(ca[3]), ug(cb[3])), w11, sg);
-        sb = ffma2(make_float2(ub(ca[3]), ub(cb[3])), w11, sb);
+        float2 sr = fmul2(make_float2(q15_r(ca[0]), q15_r(cb[0])), w00);
+        float2 sg = fmul2(make_float2(q15_g(ca[0]), q15_g(cb[0])), w00);
+        float2 sb = fmul2(make_float2(q15_b(ca[0]), q15_b(cb[0])), w00);
+        sr = ffma2(make_float2(q15_r(ca[1]), q15_r(cb[1])), w01, sr);
+        sg = ffma2(make_float2(q15_g(ca[1]), q15_g(cb[1])), w01, sg);
+        sb = ffma2(make_float2(q15_b(ca[1]), q15_b(cb[1])), w01, sb);
+        sr = ffma2(make_float2(q15_r(ca[2]), q15_r(cb[2])), w10, sr);
+        sg = ffma2(make_float2(q15_g(ca[2]), q15_g(cb[2])), w10, sg);
+        sb = ffma2(make_float2(q15_b(ca[2]), q15_b(cb[2])), w10, sb);
+        sr = ffma2(make_float2(q15_r(ca[3]), q15_r(cb[3])), w11, sr);
+        sg = ffma2(make_float2(q15_g(ca[3]), q15_g(cb[3])), w11, sg);
+        sb = ffma2(make_float2(q15_b(ca[3]), q15_b(cb[3])), w11, sb);
         if (cls == GEO_INTERIOR) {  // m = wc = 1
           if (!tail_fx) {           // scale and normalisation in one multiply-add
             put(por, f, fmaf(sr.x, kir, cir), fmaf(sr.y, kir, cir));
@@ -2247,13 +2124,13 @@ __global__ void __launch_bounds__(32 * NEXAR_GEO2_WARPS, NEXAR_GEO2_MINB) geomet
             put(pob, f, fmaf(sb.x, kib, cib), fmaf(sb.y, kib, cib));
             continue;
           }
-          rr = make_float2(fmaf(sr.x, kInvR, kS2Off), fmaf(sr.y, kInvR, kS2Off));
-          gg = make_float2(fmaf(sg.x, kInvG, kS2Off), fmaf(sg.y, kInvG, kS2Off));
-          bb = make_float2(fmaf(sb.x, kInvB, kS2Off), fmaf(sb.y, kInvB, kS2Off));
+          rr = make_float2(fmaf(sr.x, kS2Inv, kS2Off), fmaf(sr.y, kS2Inv, kS2Off));
+          gg = make_float2(fmaf(sg.x, kS2Inv, kS2Off), fmaf(sg.y, kS2Inv, kS2Off));
+          bb = make_float2(fmaf(sb.x, kS2Inv, kS2Off), fmaf(sb.y, kS2Inv, kS2Off));
         } else {
-          rr = make_float2(mq[0] * fmaf(sr.x, kInvR, fmaf(padv.x, pmq[0], t0q[0])), mq[1] * fmaf(sr.y, kInvR, fmaf(padv.x, pmq[1], t0q[1])));
-          gg = make_float2(mq[0] * fmaf(sg.x, kInvG, fmaf(padv.y, pmq[0], t0q[0])), mq[1] * fmaf(sg.y, kInvG, fmaf(padv.y, pmq[1], t0q[1])));
-          bb = make_float2(mq[0] * fmaf(sb.x, kInvB, fmaf(padv.z, pmq[0], t0q[0])), mq[1] * fmaf(sb.y, kInvB, fmaf(padv.z, pmq[1], t0q[1])));
+          rr = make_float2(mq[0] * fmaf(sr.x, kS2Inv, fmaf(padv.x, pmq[0], t0q[0])), mq[1] * fmaf(sr.y, kS2Inv, fmaf(padv.x, pmq[1], t0q[1])));
+          gg = make_float2(mq[0] * fmaf(sg.x, kS2Inv, fmaf(padv.y, pmq[0], t0q[0])), mq[1] * fmaf(sg.y, kS2Inv, fmaf(padv.y, pmq[1], t0q[1])));
+          bb = make_float2(mq[0] * fmaf(sb.x, kS2Inv, fmaf(padv.z, pmq[0], t0q[0])), mq[1] * fmaf(sb.y, kS2Inv, fmaf(padv.z, pmq[1], t0q[1])));
         }
       }
       if (tail_fx) {
@@ -2462,15 +2339,9 @@ static int sm_count() {  // of the current device (cached per device)
   return cached[dev];
 }
 
-#ifdef NEXAR_WITH_FUSED_CLUSTER
-constexpr bool kWithFused = true;
-#else
-constexpr bool kWithFused = false;   // the `fused` branch below is never taken; it then names the unfused instantiation
-#endif
-// launch of the fast resize kernel; cluster > 0: the `cluster` bands of a frame form one thread-block cluster (fused path)
+// launch of the fast resize kernel
 template <typename Kern>
-static cudaError_t launch_fast(Kern kern, dim3 grid, int nt, size_t smem, cudaStream_t st, int cluster, const DevPlan& P,
-                               const KArgs& K) {
+static cudaError_t launch_fast(Kern kern, dim3 grid, int nt, size_t smem, cudaStream_t st, const DevPlan& P, const KArgs& K) {
   if (smem > 48 * 1024) {
     const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
@@ -2480,15 +2351,6 @@ static cudaError_t launch_fast(Kern kern, dim3 grid, int nt, size_t smem, cudaSt
   cfg.blockDim = dim3(nt);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  if (cluster > 0) {
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = (unsigned)cluster;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-  }
   return cudaLaunchKernelEx(&cfg, kern, P, K);
 }
 
@@ -2534,11 +2396,11 @@ static int launch_all(const NexarPlan* p, const NexarTransformArgs* a, KArgs& K,
     // tensor take the specialised kernel; everything else the general one
     const bool planar = K.sx == 1 && K.sy == cs && K.st == (int64_t)cs * cs && g_geo_variant != 1;
     const bool tail = (a->any_flags & kTailFlags) != 0;
-    const dim3 sgrid((cs + 31) / 32, (cs + 4 * NEXAR_GEO2_WARPS - 1) / (4 * NEXAR_GEO2_WARPS), n_clips * ((a->frames_per_clip + NEXAR_GEO2_FRAMES - 1) / NEXAR_GEO2_FRAMES));
+    const dim3 sgrid((cs + 31) / 32, (cs + 4 * kGeo2Warps - 1) / (4 * kGeo2Warps), n_clips * ((a->frames_per_clip + kGeo2Frames - 1) / kGeo2Frames));
 #define NEXAR_GEO_SPEC(BHV, BWV, CSV)                                                   \
   {                                                                                     \
-    if (tail) geometry_spec_kernel<DstT, true, BHV, BWV, CSV><<<sgrid, 32 * NEXAR_GEO2_WARPS, 0, st>>>(P, K); \
-    else geometry_spec_kernel<DstT, false, BHV, BWV, CSV><<<sgrid, 32 * NEXAR_GEO2_WARPS, 0, st>>>(P, K);  \
+    if (tail) geometry_spec_kernel<DstT, true, BHV, BWV, CSV><<<sgrid, 32 * kGeo2Warps, 0, st>>>(P, K); \
+    else geometry_spec_kernel<DstT, false, BHV, BWV, CSV><<<sgrid, 32 * kGeo2Warps, 0, st>>>(P, K);  \
   }
     if (planar && K.bh == 125 && K.bw == 224 && cs == 224) NEXAR_GEO_SPEC(125, 224, 224)
     else if (planar && K.bh == 180 && K.bw == 320 && cs == 320) NEXAR_GEO_SPEC(180, 320, 320)
@@ -2560,28 +2422,15 @@ static int launch_all(const NexarPlan* p, const NexarTransformArgs* a, KArgs& K,
     if (g_fast_bands > 0) {
       nbands = imin(g_fast_bands, kMaxBands);
     } else {
-      const int slots = sm_count() * (need_threads <= 256 ? NEXAR_MINB : 2);
+      const int slots = sm_count() * (need_threads <= 256 ? kFastMinB : 2);
       nbands = imin(8, ((9 * slots) / 2 + nf - 1) / nf);
     }
     nbands = imax(1, imin(nbands, imin(kMaxBands, vis_rows)));
-    // Variant 4: augmented batches take the fused kernel, the bands of a frame being one cluster (1, 2, 4 or 8 CTAs).
-    // Measured on B200 it is not faster than K1 + K2 + K3 (the SMs are issue-bound either way and K2 / K3 run at twice
-    // the occupancy), so it is not the default; it does have the lowest DRAM traffic (1.12x algorithmic).
-#ifdef NEXAR_WITH_FUSED_CLUSTER
-    const bool fused = aug_mode && g_resize_variant == 4;
-#else
-    const bool fused = false;   // the one-launch variant is compiled only with -DNEXAR_WITH_FUSED_CLUSTER (measured slower)
-#endif
-    if (fused) {
-      int c = 1;
-      while (2 * c <= nbands && 2 * c <= 8) c *= 2;
-      nbands = c;
-    }
     const int kx = P.kx_al;
     const size_t smem = 2 * (size_t)((P.src_w * 3 + kx * 3 + 15) & ~7) * sizeof(unsigned short);
     dim3 grid(nbands, nf);
     K.pass = 0;
-    K.finfo_by_k1 = aug_mode && !fused;
+    K.finfo_by_k1 = aug_mode;
     const int ng = (kx / 2 + 3) / 4;
     const int nt_fast = need_threads <= 256 ? 256 : need_threads <= 320 ? 320 : 384;
     const size_t smem_fast = smem + (size_t)ng * nt_fast * 16 + (size_t)(P.n_pairs + 1) * 16;
@@ -2589,19 +2438,17 @@ static int launch_all(const NexarPlan* p, const NexarTransformArgs* a, KArgs& K,
 #define NEXAR_FAST_RS(KXV, NTV, MB, RSV)                                                                          \
   {                                                                                                               \
     constexpr bool kAl = (KXV) == 10;  /* 8-byte window loads exist for the 10-tap kernels only */                \
-    if (fused)                                                                                                    \
-      CUDA_TRY(launch_fast(resize_fast_kernel<KXV, NTV, MB, RSV, DstT, kWithFused, false>, grid, NTV, smem_fast, st, nbands, P, K)); \
-    else if (kAl && P.x_align4)                                                                                   \
-      CUDA_TRY(launch_fast(resize_fast_kernel<KXV, NTV, MB, RSV, DstT, false, kAl>, grid, NTV, smem_fast, st, 0, P, K)); \
+    if (kAl && P.x_align4)                                                                                        \
+      CUDA_TRY(launch_fast(resize_fast_kernel<KXV, NTV, MB, RSV, DstT, kAl>, grid, NTV, smem_fast, st, P, K));    \
     else                                                                                                          \
-      CUDA_TRY(launch_fast(resize_fast_kernel<KXV, NTV, MB, RSV, DstT, false, false>, grid, NTV, smem_fast, st, 0, P, K)); \
+      CUDA_TRY(launch_fast(resize_fast_kernel<KXV, NTV, MB, RSV, DstT, false>, grid, NTV, smem_fast, st, P, K));  \
   }
 #define NEXAR_FAST(KXV, NTV, MB) NEXAR_FAST_RS(KXV, NTV, MB, 0)
 // tightly packed 720p / 1080p rows get the row stride as a compile-time constant (immediate load offsets)
 #define NEXAR_FAST_SPEC(KXV, NTV, MB, RSV) \
   if (K.src_row_stride == RSV) NEXAR_FAST_RS(KXV, NTV, MB, RSV) else NEXAR_FAST_RS(KXV, NTV, MB, 0)
     if (need_threads <= 256) {
-      if (kx == 10) NEXAR_FAST(10, 256, NEXAR_MINB) else if (kx == 14) NEXAR_FAST_SPEC(14, 256, NEXAR_MINB, 3840) else NEXAR_FAST(20, 256, 2)
+      if (kx == 10) NEXAR_FAST(10, 256, kFastMinB) else if (kx == 14) NEXAR_FAST_SPEC(14, 256, kFastMinB, 3840) else NEXAR_FAST(20, 256, 2)
     } else if (need_threads <= 320) {
       if (kx == 10) NEXAR_FAST_SPEC(10, 320, 2, 3840) else if (kx == 14) NEXAR_FAST(14, 320, 2) else NEXAR_FAST(20, 320, 2)
     } else {
@@ -2614,7 +2461,7 @@ static int launch_all(const NexarPlan* p, const NexarTransformArgs* a, KArgs& K,
     // fix-up of clips whose maximum was <= 1 (not divided by 255): their values live in [0,1], below the
     // resolution of the 15-bit staging, so the rare second pass uses the fp32 resample.
     // K1.5 / K2 / K3 for the clips whose maximum was > 1 (pass 4: the others are skipped, see fixup_frame_kernel)
-    if (aug_mode && !fused) {
+    if (aug_mode) {
       K.pass = 4;
       launch_tail();
     }
@@ -2636,7 +2483,7 @@ static int launch_all(const NexarPlan* p, const NexarTransformArgs* a, KArgs& K,
       at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
       at[0].val.programmaticStreamSerializationAllowed = 1;
       cfg.attrs = at;
-      cfg.numAttrs = (!fused && g_resize_variant != 2) ? 1 : 0;
+      cfg.numAttrs = g_resize_variant != 2 ? 1 : 0;
       K.overlap = cfg.numAttrs && !aug_mode;   // directly behind the resize kernel: wait for its completion on the device
       CUDA_TRY(cudaLaunchKernelEx(&cfg, fixup_frame_kernel<SrcT, DstT>, P, K));
       K.overlap = 0;
