@@ -176,6 +176,32 @@ typedef struct NexarYuvFormat {
 
 /* A plan for YUV 4:2:0 surfaces.  geom->src_h / src_w are the visible picture (both even). */
 int nexar_plan_create_yuv(const NexarGeometry* geom, const NexarYuvFormat* fmt, NexarPlan** out);
+
+/* A plan for YUV 4:2:0 surfaces of 16-bit little-endian samples (10-, 12- or 16-bit decoder output).
+ * fmt->layout NEXAR_YUV_NV12 is semi-planar (P010 / P012 / P016: interleaved U V words), NEXAR_YUV_I420 planar
+ * (libavcodec's yuv420p10le).  sample_shift aligns each sample to the top of a 16-bit word: 0 for MSB-aligned samples
+ * (P010 / P012 / P016), 6 for LSB-aligned 10-bit samples (yuv420p10le), 4 for LSB-aligned 12-bit samples; any other
+ * value is NEXAR_ERR_INVALID.
+ *
+ * Addressing is the 8-bit addressing above in bytes with 2-byte samples: pitch = src_row_stride is in bytes and must be
+ * even with 2*src_w <= pitch; the chroma starts at L*pitch (NV12: L/2 rows of pitch bytes, U0 V0 U1 V1 ... words;
+ * I420: U plane of L/2 rows of pitch/2 bytes, then the V plane at L*pitch*5/4).
+ *
+ * Conversion: every sample is read as the word w = (sample << sample_shift) & 0xFFFF, and with the coefficients of the
+ * table above, unchanged,
+ *   C = w_Y - (Yo << 8), D = w_U - 32768, E = w_V - 32768
+ *   R = clip((Ys C + Rv E + 32768) >> 16), G = clip((Ys C - Gu D - Gv E + 32768) >> 16), B = clip((Ys C + Bu D + 32768) >> 16)
+ * to RGB bytes, then the NEXAR_SRC_U8 path.  A word x << 8 converts exactly as the 8-bit code x does
+ * ((256 x + 32768) >> 16 == (x + 128) >> 8), so P010 words made from an NV12 surface give its result bit for bit; and
+ * (64 X + 32768) >> 16 == (X + 512) >> 10, so 10-bit content is rounded once from its full precision.  A 10-bit code is
+ * read as 4 x an 8-bit code, the limited-range convention of BT.709 / BT.2100 (for full range it differs from the
+ * code / 1023 scaling by 0.25 %).
+ *
+ * The conversion reads 16 luma pixels of two rows per thread with 16-byte loads when src and every frame_offsets[i]
+ * are multiples of 16 (the offsets are not checked), src_w % 16 == 0 and the pitch keeps the chroma rows 16-byte
+ * aligned (pitch % 16 == 0 for NV12, pitch % 32 == 0 for I420); any other even size, pitch or alignment takes a
+ * byte-wise kernel. */
+int nexar_plan_create_yuv16(const NexarGeometry* geom, const NexarYuvFormat* fmt, int32_t sample_shift, NexarPlan** out);
 /* The integer coefficients {Yo, Ys, Rv, Gu, Gv, Bu} the conversion uses for (matrix, range), for binding checks. */
 int nexar_yuv_coefficients(int32_t matrix, int32_t range, int32_t out[6]);
 size_t nexar_sizeof_yuv_format(void);

@@ -3,8 +3,8 @@
 Device-resident legs: the cfg2 batch of bench.py (32 clips x 16 frames, 720p -> 224, bf16) with the `val` and `custom`
 kwargs, fed once per source format.  Every input is >= 0.7 GB (more than the 126 MB L2), built from 4 distinct clips.
 The legs alternate round by round in one process; each round times >= 100 steps with CUDA events, and each leg's extra
-time over the RGB leg is taken within the same round.  End-to-end legs: the same batch through HostClipPipeline from
-pinned host memory (rgb, nv12, i420).  One JSON line per leg goes to stdout and to OUTDIR/yuv_lines.jsonl, with the
+time over the RGB leg is taken within the same round.  The 16-bit legs (p010, i010) carry 10-bit surfaces, uint16.
+End-to-end legs: the same batch through HostClipPipeline from pinned host memory (rgb, nv12, i420, p010, i010).  One JSON line per leg goes to stdout and to OUTDIR/yuv_lines.jsonl, with the
 GPU's name, power limit and maximum SM clock read in the same run.
 
 With NEXAR_LIB pointing at an older build (which has only NV12 BT.601 limited range), run the `rgb` and `nv12_601l`
@@ -39,9 +39,13 @@ LEGS = {
     "i420_709l": (720, 1280, dict(pixel_format="i420", color_matrix="bt709"), None, None),
     "rgb_1080p": (1080, 1920, None, None, None),
     "nv12_1080p_in_1088x2048": (1080, 1920, dict(pixel_format="nv12", color_matrix="bt709"), 1088, 2048),
+    "p010_601l": (720, 1280, dict(pixel_format="p010"), None, None),
+    "i010_709l": (720, 1280, dict(pixel_format="i010", color_matrix="bt709"), None, None),
+    "p010_1080p_in_1088x2048": (1080, 1920, dict(pixel_format="p010", color_matrix="bt709"), 1088, 2048),
 }
 BASE = {"rgb": "rgb", "nv12_601l": "rgb", "nv12_709f": "rgb", "i420_709l": "rgb", "rgb_1080p": "rgb_1080p",
-        "nv12_1080p_in_1088x2048": "rgb_1080p"}
+        "nv12_1080p_in_1088x2048": "rgb_1080p", "p010_601l": "rgb", "i010_709l": "rgb",
+        "p010_1080p_in_1088x2048": "rgb_1080p"}
 
 
 def gpu_provenance():
@@ -57,7 +61,7 @@ _RGB = {}
 
 def make_inputs(leg, dev):
     """Device tensor of B clips (4 distinct ones repeated) in the leg's source format, plus its picture size."""
-    from vision_collision_detection_b200.synth import make_clip_torch, rgb_to_yuv420
+    from vision_collision_detection_b200.synth import make_clip_torch, rgb_to_yuv420, rgb_to_yuv420_16
     h, w, kw, lr, pitch = LEGS[leg]
     distinct = []
     for i in range(4):
@@ -67,9 +71,10 @@ def make_inputs(leg, dev):
         if kw is None:
             distinct.append(torch.from_numpy(rgb))
         else:
-            distinct.append(torch.from_numpy(rgb_to_yuv420(rgb, kw["pixel_format"], kw.get("color_matrix", "bt601"),
-                                                           kw.get("color_range", "limited"), lr, pitch)))
-    x = torch.empty((B,) + tuple(distinct[0].shape), dtype=torch.uint8, device=dev)
+            enc = rgb_to_yuv420_16 if kw["pixel_format"] in ("p010", "i010") else rgb_to_yuv420
+            distinct.append(torch.from_numpy(enc(rgb, kw["pixel_format"], kw.get("color_matrix", "bt601"),
+                                                 kw.get("color_range", "limited"), lr, pitch)))
+    x = torch.empty((B,) + tuple(distinct[0].shape), dtype=distinct[0].dtype, device=dev)
     for i in range(B):
         x[i].copy_(distinct[i % 4])
     return x, h, w
@@ -141,7 +146,7 @@ def main():
             extra = [a - b for a, b in zip(ms[leg], ms[BASE[leg]])]
             x, h, w = inputs[leg]
             emit({"leg": "device", "source": leg, "mode": mode, "batch": [B, T, h, w], "crop": CS, "out": "bf16",
-                  "input_bytes": x.numel(), "steps_per_round": args.steps, "rounds": args.rounds,
+                  "input_bytes": x.numel() * x.element_size(), "steps_per_round": args.steps, "rounds": args.rounds,
                   "ms_step_median": round(med, 4), "ms_step_rounds": [round(v, 4) for v in ms[leg]],
                   "spread_ms": round(max(ms[leg]) - min(ms[leg]), 4), "clips_per_s": round(B / (med * 1e-3), 1),
                   "extra_ms_over": BASE[leg], "extra_ms_median": round(statistics.median(extra), 4),
@@ -152,8 +157,10 @@ def main():
         tf = create_video_transforms(**KW["custom"], crop_size=CS, out_dtype=torch.bfloat16)
         random.seed(1234)
         ps = [tf.sample_params(B, 720, 1280) for _ in range(4)]
-        for src, leg in (("rgb", "rgb"), ("nv12", "nv12_601l"), ("i420", "i420_709l")):
+        for src, leg in (("rgb", "rgb"), ("nv12", "nv12_601l"), ("i420", "i420_709l"), ("p010", "p010_601l"),
+                         ("i010", "i010_709l")):
             x = inputs[leg][0] if leg in inputs else make_inputs(leg, dev)[0]
+            nbytes = x.numel() * x.element_size()
             kw = LEGS[leg][2] or {}
             pipe = HostClipPipeline(tf, n_clips=B, frames=T, height=720, width=1280, device=dev, **kw)
             ins = [pipe.pinned_input(), pipe.pinned_input()]
@@ -173,9 +180,9 @@ def main():
             torch.cuda.synchronize()
             ms_step = (time.perf_counter() - t0) * 1e3 / args.e2e_steps
             emit({"leg": "e2e", "source": src, "mode": "custom", "batch": [B, T, 720, 1280], "crop": CS, "out": "bf16",
-                  "h2d_bytes_per_step": ins[0].numel(), "steps": args.e2e_steps, "ms_step": round(ms_step, 3),
+                  "h2d_bytes_per_step": nbytes, "steps": args.e2e_steps, "ms_step": round(ms_step, 3),
                   "clips_per_s": round(B / (ms_step * 1e-3), 1),
-                  "h2d_GBs": round(ins[0].numel() / (ms_step * 1e-3) / 1e9, 2)})
+                  "h2d_GBs": round(nbytes / (ms_step * 1e-3) / 1e9, 2)})
             del pipe, ins
     with open(os.path.join(args.outdir, "yuv_lines.jsonl"), "a") as f:
         f.write("\n".join(out_lines) + "\n")

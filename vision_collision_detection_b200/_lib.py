@@ -160,6 +160,25 @@ def yuv_lib():
     return L
 
 
+_yuv16_bound = False
+
+
+def yuv16_lib():
+    """``yuv_lib()`` with ``nexar_plan_create_yuv16`` bound (16-bit P010 / I010 surfaces), on first use only: a library
+    built before it existed serves every 8-bit format and refuses the 16-bit ones with this error."""
+    global _yuv16_bound
+    L = yuv_lib()
+    if not _yuv16_bound:
+        try:
+            fn = L.nexar_plan_create_yuv16
+        except AttributeError:
+            raise RuntimeError(f"{LIB_PATH} predates 16-bit YUV surfaces (no nexar_plan_create_yuv16); rebuild it to "
+                               "convert p010 / i010 frames") from None
+        fn.argtypes = [C.POINTER(Geometry), C.POINTER(YuvFormat), C.c_int32, C.POINTER(C.c_void_p)]
+        _yuv16_bound = True
+    return L
+
+
 def yuv_coefficients(matrix: int, range_: int):
     """-> (Yo, Ys, Rv, Gu, Gv, Bu), the integer conversion coefficients the library uses."""
     out = (C.c_int32 * 6)()

@@ -9,7 +9,7 @@
 //   K3 geometry : affine gather with the fill=0 mask quirk, effects, normalise, store (a kernel specialised for the
 //                 production letterboxes, a general one for everything else).
 //   K4 blur     : only when blur_sigma > 0 (reflect-padded gaussian, then the rest of the chain).
-//   YUV 4:2:0 -> RGB : decoder surfaces (NV12 / I420, BT.601 / BT.709, limited / full range) converted in front of K1; window gather for inference.
+//   YUV 4:2:0 -> RGB : decoder surfaces (NV12 / I420 with 8- or 16-bit samples, BT.601 / BT.709, limited / full range) converted in front of K1; window gather for inference.
 // The /255 decision of VideoTransform.forward is clip-global and data dependent
 // (nexar_video_aug.py:814): K1 runs assuming "max > 1", records the clip maximum, and
 // a second, normally empty, launch (fixup_frame_kernel) redoes the clips whose maximum was <= 1.
@@ -87,6 +87,8 @@ struct NexarPlan {
   int src_dtype;               // NEXAR_SRC_NV12 stands for every YUV 4:2:0 source; yuv_* below say which
   int yuv_layout = NEXAR_YUV_NV12;
   int yuv_luma_rows = 0;
+  bool yuv_16bit = false;      // 2-byte samples (nexar_plan_create_yuv16), aligned to the word's top by yuv_shift
+  int yuv_shift = 0;
   YuvCoef yuv_coef = kYuvCoef[NEXAR_YUV_BT601][NEXAR_YUV_LIMITED];
   DevPlan d;
   void* dev_tables;
@@ -379,6 +381,19 @@ extern "C" int nexar_plan_create_yuv(const NexarGeometry* g, const NexarYuvForma
   if (f->matrix != NEXAR_YUV_BT601 && f->matrix != NEXAR_YUV_BT709) return fail(NEXAR_ERR_INVALID, "plan_create_yuv: unknown matrix");
   if (f->range != NEXAR_YUV_LIMITED && f->range != NEXAR_YUV_FULL) return fail(NEXAR_ERR_INVALID, "plan_create_yuv: unknown range");
   return plan_create(g, NEXAR_SRC_NV12, f, out);
+}
+
+extern "C" int nexar_plan_create_yuv16(const NexarGeometry* g, const NexarYuvFormat* f, int32_t sample_shift, NexarPlan** out) {
+  if (!out) return fail(NEXAR_ERR_INVALID, "plan_create_yuv16: null argument");
+  if (sample_shift != 0 && sample_shift != 4 && sample_shift != 6)
+    return fail(NEXAR_ERR_INVALID, "plan_create_yuv16: sample_shift must be 0, 4 or 6");
+  NexarPlan* p = nullptr;
+  const int rc = nexar_plan_create_yuv(g, f, &p);
+  if (rc != NEXAR_OK) return rc;
+  p->yuv_16bit = true;
+  p->yuv_shift = sample_shift;
+  *out = p;
+  return NEXAR_OK;
 }
 
 static int plan_create(const NexarGeometry* g, int32_t src_dtype, const NexarYuvFormat* yuv, NexarPlan** out) {
@@ -2326,6 +2341,124 @@ __global__ void __launch_bounds__(256) yuv420_to_rgb_any_kernel(const unsigned c
 }
 
 // ---------------------------------------------------------------------------------
+// 16-bit samples (P010 / P012 / P016, yuv420p10le; nexar_plan_create_yuv16): the same surfaces with 2-byte little-endian
+// samples (pitch, uoff and voff in bytes as above).  Every sample is read as the word w = (sample << shift) & 0xFFFF and
+// converted with the same coefficients at 16 bits of precision,
+//   C = w_Y - (Yo << 8), D = w_U - 32768, E = w_V - 32768
+//   R = clip((Ys C + Rv E + 32768) >> 16)   G = clip((Ys C - Gu D - Gv E + 32768) >> 16)   B = clip((Ys C + Bu D + 32768) >> 16)
+// so a word x << 8 gives exactly the 8-bit result of the code x, and 10-bit content is rounded once to bytes.  Every term
+// fits int32 (298 * 65535 + 541 * 32768 < 2^31); clip(x >> 16) is evaluated as clamp(x, 0, 2^24 - 1) >> 16
+// (tests/yuv16_oracle.py states the same formula in numpy).
+// ---------------------------------------------------------------------------------
+__device__ __forceinline__ int clamp_u24(int x) { return min(max(x, 0), (1 << 24) - 1); }
+__device__ __forceinline__ ChromaTerms chroma_terms16(int u, int v, const YuvCoef& k) {
+  const int d = u - 32768, e = v - 32768;
+  const int base = 32768 - k.ys * (k.yo << 8);
+  return {k.rv * e + base, -k.gu * d - k.gv * e + base, k.bu * d + base};
+}
+// the two samples of a 32-bit word, each moved to the top of its 16-bit half
+__device__ __forceinline__ unsigned align_words(unsigned w, int shift) { return (w & ((0xFFFFu >> shift) * 0x10001u)) << shift; }
+// one sample at any byte address (little-endian), moved to the top of the word
+__device__ __forceinline__ int load_word(const unsigned char* p, int shift) { return ((p[0] | (p[1] << 8)) << shift) & 0xFFFF; }
+
+// 16 pixels of two rows per thread: four 16-byte luma loads, two 16-byte chroma loads (NV12: the U V words of the 8
+// chroma pairs; I420: 8 U words and 8 V words), six 16-byte stores
+template <int Layout>
+__global__ void __launch_bounds__(256) yuv420_16_to_rgb_vec_kernel(const unsigned char* __restrict__ src, const int64_t* __restrict__ frame_offsets,
+                                                                   int64_t pitch, int64_t uoff, int64_t voff, YuvCoef kc, int shift, int H, int W,
+                                                                   unsigned char* __restrict__ rgb, int64_t* __restrict__ out_offsets) {
+  const int frame = blockIdx.y;
+  const int cols = W >> 4;
+  const int unit = blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t fbytes = (int64_t)H * W * 3;
+  if (unit == 0) out_offsets[frame] = (int64_t)frame * fbytes;
+  if (unit >= cols * (H >> 1)) return;
+  const int r2 = unit / cols, c = unit - r2 * cols;
+  const unsigned char* f = src + frame_offsets[frame];
+  const unsigned char* ra = f + (int64_t)(2 * r2) * pitch + 32 * c;
+  const uint4 ya0 = __ldcs((const uint4*)ra), ya1 = __ldcs((const uint4*)(ra + 16));
+  const uint4 yb0 = __ldcs((const uint4*)(ra + pitch)), yb1 = __ldcs((const uint4*)(ra + pitch + 16));
+  unsigned uvw[8];   // U | V << 16 of chroma pairs 0 .. 7
+  if (Layout == NEXAR_YUV_NV12) {
+    const unsigned char* q = f + uoff + (int64_t)r2 * pitch + 32 * c;
+    const uint4 a = __ldcs((const uint4*)q), b = __ldcs((const uint4*)(q + 16));
+    uvw[0] = a.x, uvw[1] = a.y, uvw[2] = a.z, uvw[3] = a.w, uvw[4] = b.x, uvw[5] = b.y, uvw[6] = b.z, uvw[7] = b.w;
+  } else {
+    const int64_t cp = pitch >> 1;
+    const uint4 u = __ldcs((const uint4*)(f + uoff + (int64_t)r2 * cp + 16 * c));
+    const uint4 v = __ldcs((const uint4*)(f + voff + (int64_t)r2 * cp + 16 * c));
+    const unsigned uw[4] = {u.x, u.y, u.z, u.w}, vw[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) uvw[2 * i] = __byte_perm(uw[i], vw[i], 0x5410), uvw[2 * i + 1] = __byte_perm(uw[i], vw[i], 0x7632);
+  }
+  const unsigned yaw[8] = {ya0.x, ya0.y, ya0.z, ya0.w, ya1.x, ya1.y, ya1.z, ya1.w};
+  const unsigned ybw[8] = {yb0.x, yb0.y, yb0.z, yb0.w, yb1.x, yb1.y, yb1.z, yb1.w};
+  unsigned oa[12], ob[12];   // 48 output bytes per row
+#pragma unroll
+  for (int q = 0; q < 8; ++q) {  // two pixels (one chroma pair) per 32-bit word of luma
+    const unsigned cw = align_words(uvw[q], shift);
+    const ChromaTerms t = chroma_terms16(cw & 0xFFFFu, cw >> 16, kc);
+    const unsigned wa = align_words(yaw[q], shift), wb = align_words(ybw[q], shift);
+    unsigned char* pa = (unsigned char*)oa + 6 * q;
+    unsigned char* pb = (unsigned char*)ob + 6 * q;
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int la = kc.ys * (int)((wa >> (16 * k)) & 0xFFFFu), lb = kc.ys * (int)((wb >> (16 * k)) & 0xFFFFu);
+      pa[3 * k + 0] = (unsigned char)(clamp_u24(la + t.r) >> 16);
+      pa[3 * k + 1] = (unsigned char)(clamp_u24(la + t.g) >> 16);
+      pa[3 * k + 2] = (unsigned char)(clamp_u24(la + t.b) >> 16);
+      pb[3 * k + 0] = (unsigned char)(clamp_u24(lb + t.r) >> 16);
+      pb[3 * k + 1] = (unsigned char)(clamp_u24(lb + t.g) >> 16);
+      pb[3 * k + 2] = (unsigned char)(clamp_u24(lb + t.b) >> 16);
+    }
+  }
+  unsigned char* o = rgb + (int64_t)frame * fbytes + ((int64_t)(2 * r2) * W + 16 * c) * 3;
+  uint4* da = (uint4*)o;
+  uint4* db = (uint4*)(o + (int64_t)W * 3);
+#pragma unroll
+  for (int v = 0; v < 3; ++v) {
+    da[v] = make_uint4(oa[4 * v], oa[4 * v + 1], oa[4 * v + 2], oa[4 * v + 3]);
+    db[v] = make_uint4(ob[4 * v], ob[4 * v + 1], ob[4 * v + 2], ob[4 * v + 3]);
+  }
+}
+
+// any even size / even pitch / alignment: one 2 x 2 block per thread, every sample read byte by byte
+template <int Layout>
+__global__ void __launch_bounds__(256) yuv420_16_to_rgb_any_kernel(const unsigned char* __restrict__ src, const int64_t* __restrict__ frame_offsets,
+                                                                   int64_t pitch, int64_t uoff, int64_t voff, YuvCoef kc, int shift, int H, int W,
+                                                                   unsigned char* __restrict__ rgb, int64_t* __restrict__ out_offsets) {
+  const int frame = blockIdx.y;
+  const int cols = W >> 1;
+  const int unit = blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t fbytes = (int64_t)H * W * 3;
+  if (unit == 0) out_offsets[frame] = (int64_t)frame * fbytes;
+  if (unit >= cols * (H >> 1)) return;
+  const int r2 = unit / cols, c = unit - r2 * cols;
+  const unsigned char* f = src + frame_offsets[frame];
+  int u, v;
+  if (Layout == NEXAR_YUV_NV12) {
+    const unsigned char* uvp = f + uoff + (int64_t)r2 * pitch + 4 * c;
+    u = load_word(uvp, shift), v = load_word(uvp + 2, shift);
+  } else {
+    const int64_t at = (int64_t)r2 * (pitch >> 1) + 2 * c;
+    u = load_word(f + uoff + at, shift), v = load_word(f + voff + at, shift);
+  }
+  const ChromaTerms t = chroma_terms16(u, v, kc);
+#pragma unroll
+  for (int dy = 0; dy < 2; ++dy) {
+    const unsigned char* yp = f + (int64_t)(2 * r2 + dy) * pitch + 4 * c;
+    unsigned char* o = rgb + (int64_t)frame * fbytes + ((int64_t)(2 * r2 + dy) * W + 2 * c) * 3;
+#pragma unroll
+    for (int dx = 0; dx < 2; ++dx) {
+      const int l = kc.ys * load_word(yp + 2 * dx, shift);
+      o[3 * dx + 0] = (unsigned char)(clamp_u24(l + t.r) >> 16);
+      o[3 * dx + 1] = (unsigned char)(clamp_u24(l + t.g) >> 16);
+      o[3 * dx + 2] = (unsigned char)(clamp_u24(l + t.b) >> 16);
+    }
+  }
+}
+
+// ---------------------------------------------------------------------------------
 // launcher
 // ---------------------------------------------------------------------------------
 static int sm_count() {  // of the current device (cached per device)
@@ -2613,10 +2746,13 @@ extern "C" int nexar_clip_transform(const NexarPlan* p, const NexarTransformArgs
     if (a->normalize && !(a->std[c] != 0.0f)) return fail(NEXAR_ERR_INVALID, "clip_transform: std must be non-zero");
   const bool nv12 = p->src_dtype == NEXAR_SRC_NV12;
   const size_t esz = p->src_dtype == NEXAR_SRC_F32 ? 4 : 1;
-  if (a->src_row_stride < (int64_t)(nv12 ? p->g.src_w : p->g.src_w * 3 * esz))
+  const int64_t sample_bytes = nv12 && p->yuv_16bit ? 2 : 1;
+  if (a->src_row_stride < (int64_t)(nv12 ? p->g.src_w * sample_bytes : p->g.src_w * 3 * esz))
     return fail(NEXAR_ERR_INVALID, "clip_transform: src_row_stride smaller than a row");
   if (nv12 && p->yuv_layout == NEXAR_YUV_I420 && (a->src_row_stride & 1))
     return fail(NEXAR_ERR_INVALID, "clip_transform: I420 surfaces need an even src_row_stride");
+  if (nv12 && p->yuv_16bit && (a->src_row_stride & 1))
+    return fail(NEXAR_ERR_INVALID, "clip_transform: 16-bit surfaces need an even src_row_stride");
 
   Workspace w = carve(p, a->n_clips, a->frames_per_clip, a->workspace, a->any_flags);
   KArgs K;
@@ -2633,7 +2769,22 @@ extern "C" int nexar_clip_transform(const NexarPlan* p, const NexarTransformArgs
     // pitch % 16 == 0 with an even luma height also keeps the 8-byte I420 chroma loads aligned
     const bool vec = (W % 16) == 0 && (pitch % 16) == 0 && (((uintptr_t)a->src) & 15) == 0;
     const dim3 gv(((W / 16) * (H / 2) + 255) / 256, nf), ga(((W / 2) * (H / 2) + 255) / 256, nf);
-    if (p->yuv_layout == NEXAR_YUV_I420) {
+    if (p->yuv_16bit) {
+      // 32-byte luma / NV12 chroma and 16-byte I420 chroma loads per thread: the chroma rows stay 16-byte aligned
+      const int sh = p->yuv_shift;
+      const bool vec16 = (W % 16) == 0 && (pitch % (p->yuv_layout == NEXAR_YUV_I420 ? 32 : 16)) == 0 && (((uintptr_t)a->src) & 15) == 0;
+      if (p->yuv_layout == NEXAR_YUV_I420) {
+        if (vec16)
+          yuv420_16_to_rgb_vec_kernel<NEXAR_YUV_I420><<<gv, 256, 0, st>>>(s, a->frame_offsets, pitch, uoff, voff, p->yuv_coef, sh, H, W, w.rgb, w.rgb_offsets);
+        else
+          yuv420_16_to_rgb_any_kernel<NEXAR_YUV_I420><<<ga, 256, 0, st>>>(s, a->frame_offsets, pitch, uoff, voff, p->yuv_coef, sh, H, W, w.rgb, w.rgb_offsets);
+      } else {
+        if (vec16)
+          yuv420_16_to_rgb_vec_kernel<NEXAR_YUV_NV12><<<gv, 256, 0, st>>>(s, a->frame_offsets, pitch, uoff, voff, p->yuv_coef, sh, H, W, w.rgb, w.rgb_offsets);
+        else
+          yuv420_16_to_rgb_any_kernel<NEXAR_YUV_NV12><<<ga, 256, 0, st>>>(s, a->frame_offsets, pitch, uoff, voff, p->yuv_coef, sh, H, W, w.rgb, w.rgb_offsets);
+      }
+    } else if (p->yuv_layout == NEXAR_YUV_I420) {
       if (vec)
         yuv420_to_rgb_vec_kernel<NEXAR_YUV_I420><<<gv, 256, 0, st>>>(s, a->frame_offsets, pitch, uoff, voff, p->yuv_coef, H, W, w.rgb, w.rgb_offsets);
       else

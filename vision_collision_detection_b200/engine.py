@@ -38,14 +38,19 @@ def _alloc_out(layout: str, b: int, t: int, cs: int, dtype, device):
 class Plan:
     """RAII wrapper of NexarPlan."""
 
-    def __init__(self, geom: _lib.Geometry, src_dtype: int, yuv: Optional[Tuple[int, int, int, int]] = None):
-        """``yuv``: (layout, matrix, range, luma_rows) of YUV 4:2:0 surfaces (``nexar_plan_create_yuv``); None for the
-        sources of ``nexar_plan_create``, NV12 BT.601 limited range with an unpadded luma plane among them."""
+    def __init__(self, geom: _lib.Geometry, src_dtype: int, yuv: Optional[Tuple[int, ...]] = None):
+        """``yuv``: (layout, matrix, range, luma_rows) of YUV 4:2:0 surfaces (``nexar_plan_create_yuv``), or
+        (layout, matrix, range, luma_rows, sample_shift) of surfaces with 16-bit samples (``nexar_plan_create_yuv16``);
+        None for the sources of ``nexar_plan_create``, NV12 BT.601 limited range with an unpadded luma plane among them."""
         self.geom = geom
         self.src_dtype = _lib.SRC_NV12 if yuv is not None else src_dtype
+        self.sample_bytes = 2 if yuv is not None and len(yuv) == 5 else 1
         h = C.c_void_p()
         if yuv is None:
             _lib.check(_lib.lib().nexar_plan_create(C.byref(geom), src_dtype, C.byref(h)))
+        elif len(yuv) == 5:
+            f = _lib.YuvFormat(C.sizeof(_lib.YuvFormat), *yuv[:4])
+            _lib.check(_lib.yuv16_lib().nexar_plan_create_yuv16(C.byref(geom), C.byref(f), yuv[4], C.byref(h)))
         else:
             f = _lib.YuvFormat(C.sizeof(_lib.YuvFormat), *yuv)
             _lib.check(_lib.yuv_lib().nexar_plan_create_yuv(C.byref(geom), C.byref(f), C.byref(h)))
@@ -79,7 +84,7 @@ class ClipTransformEngine:
         self.last_launches = 0
 
     # -- plans ---------------------------------------------------------------------
-    def plan(self, geom: _lib.Geometry, src_dtype: int, yuv: Optional[Tuple[int, int, int, int]] = None) -> Plan:
+    def plan(self, geom: _lib.Geometry, src_dtype: int, yuv: Optional[Tuple[int, ...]] = None) -> Plan:
         key = geom.as_tuple() + (src_dtype, yuv)
         p = self._plans.get(key)
         if p is None:
@@ -95,7 +100,8 @@ class ClipTransformEngine:
 
     def letterbox_plan(self, h: int, w: int, cs: int, src_dtype=torch.uint8) -> Plan:
         """``src_dtype``: torch.uint8 / torch.float32 (packed RGB), the string "nv12" (decoder surfaces, BT.601 limited
-        range) or a YUV 4:2:0 format tuple (layout, matrix, range, luma_rows) of ``_lib.YUV_*`` values."""
+        range) or a YUV 4:2:0 format tuple (layout, matrix, range, luma_rows) of ``_lib.YUV_*`` values, with a fifth entry,
+        the sample shift, for 16-bit samples."""
         return self._plan_for(_lib.letterbox_geometry(h, w, cs), src_dtype)
 
     def resize_crop_plan(self, h: int, w: int, size: int, cs: int, src_dtype=torch.uint8) -> Plan:
@@ -148,7 +154,8 @@ class ClipTransformEngine:
             raise TypeError(f"unsupported output dtype {out.dtype}")
         g = plan.geom
         esz = 4 if plan.src_dtype == _lib.SRC_F32 else 1
-        row = g.src_w if plan.src_dtype == _lib.SRC_NV12 else g.src_w * 3 * esz   # NV12: the pitch of the Y / UV planes
+        # YUV: the pitch of the Y / UV planes, in bytes (2 per 16-bit sample)
+        row = g.src_w * plan.sample_bytes if plan.src_dtype == _lib.SRC_NV12 else g.src_w * 3 * esz
         a = _lib.TransformArgs()
         a.struct_size = C.sizeof(_lib.TransformArgs)
         a.n_clips, a.frames_per_clip = n_clips, frames_per_clip

@@ -12,7 +12,7 @@ from typing import Any, Dict, List, Optional
 import torch
 
 from .engine import ClipTransformEngine
-from .video_aug import GpuVideoTransform, check_pixel_format
+from .video_aug import GpuVideoTransform, check_pixel_format, source_dtype
 
 
 def bind_to_gpu_numa_node(device_index: int) -> Optional[List[int]]:
@@ -50,19 +50,21 @@ class HostClipPipeline:
                  pixel_format: str = "rgb", color_matrix: str = "bt601", color_range: str = "limited"):
         """``pixel_format="nv12"`` / ``"i420"``: the host clips are YUV 4:2:0 decoder surfaces, uint8 ``[B,T,H*3/2,W]``
         — half the bytes of RGB over PCIe (the link is what bounds this path), converted to RGB on the device with
-        ``color_matrix`` / ``color_range`` (see ``GpuVideoTransform.forward_batch``)."""
+        ``color_matrix`` / ``color_range`` (see ``GpuVideoTransform.forward_batch``).  ``"p010"`` / ``"i010"``: 16-bit
+        surfaces, uint16 ``[B,T,H*3/2,W]`` — as many bytes as RGB over PCIe."""
         self.tf = transform
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
         yuv = check_pixel_format(pixel_format, color_matrix, color_range)
         self.pixel_format = pixel_format
         self.yuv_kw = dict(pixel_format=pixel_format, color_matrix=color_matrix, color_range=color_range)
         self.shape = (n_clips, frames, height * 3 // 2, width) if yuv else (n_clips, frames, height, width, 3)
+        self.dtype = source_dtype(pixel_format)
         self.chunk = max(1, min(clips_per_chunk, n_clips))
         self.out_dtype = out_dtype or transform.out_dtype
         cs = transform.crop_size
         self.streams = [torch.cuda.Stream(self.device) for _ in range(n_streams)]
         self.engines = [ClipTransformEngine(self.device) for _ in range(n_streams)]
-        self.dev_in = [torch.empty((self.chunk,) + self.shape[1:], dtype=torch.uint8, device=self.device)
+        self.dev_in = [torch.empty((self.chunk,) + self.shape[1:], dtype=self.dtype, device=self.device)
                        for _ in range(n_streams)]
         self.dev_out = [torch.empty((self.chunk, 3, frames, cs, cs), dtype=self.out_dtype, device=self.device)
                         for _ in range(n_streams)]
@@ -73,14 +75,14 @@ class HostClipPipeline:
         self._slot = 0
 
     def pinned_input(self) -> torch.Tensor:
-        return torch.empty(self.shape, dtype=torch.uint8).pin_memory()
+        return torch.empty(self.shape, dtype=self.dtype).pin_memory()
 
     @torch.no_grad()
     def submit(self, host_clips: torch.Tensor, params: Optional[List[Dict[str, Any]]] = None) -> int:
-        """Enqueue one batch (pinned uint8 [B,T,H,W,3]); returns a ticket for ``wait``.  At most two batches may be
+        """Enqueue one batch (pinned uint8 [B,T,H,W,3], or the surfaces of ``pixel_format``); returns a ticket for ``wait``.  At most two batches may be
         in flight; the input buffer must stay untouched until its ticket has been waited for."""
-        if tuple(host_clips.shape) != self.shape or host_clips.dtype != torch.uint8:
-            raise ValueError(f"expected uint8 {self.shape}")
+        if tuple(host_clips.shape) != self.shape or host_clips.dtype != self.dtype:
+            raise ValueError(f"expected {self.dtype} {self.shape}")
         n = self.shape[0]
         if params is None:
             h = self.shape[2] * 2 // 3 if self.pixel_format != "rgb" else self.shape[2]
@@ -111,5 +113,5 @@ class HostClipPipeline:
 
     @torch.no_grad()
     def run(self, host_clips: torch.Tensor, params: Optional[List[Dict[str, Any]]] = None) -> torch.Tensor:
-        """host_clips: pinned uint8 [B,T,H,W,3] (or [B,T,H*3/2,W] for nv12 / i420).  Returns the pinned [B,3,T,cs,cs] result (valid on return)."""
+        """host_clips: pinned uint8 [B,T,H,W,3] (or [B,T,H*3/2,W] for nv12 / i420, uint16 for p010 / i010).  Returns the pinned [B,3,T,cs,cs] result (valid on return)."""
         return self.wait(self.submit(host_clips, params))

@@ -54,7 +54,8 @@ class SlidingWindowTransform:
     def frames(self, video_u8: torch.Tensor, pixel_format: str = "rgb", color_matrix: str = "bt601",
                color_range: str = "limited", frame_size=None) -> torch.Tensor:
         """[N,H,W,3] uint8 on the device -> [N,3,cs,cs]: every frame transformed once.  YUV surfaces [N,R,P] with
-        ``pixel_format="nv12"`` / ``"i420"`` and the other source-format keywords of forward_batch."""
+        ``pixel_format="nv12"`` / ``"i420"`` (uint16 with ``"p010"`` / ``"i010"``) and the other source-format keywords
+        of forward_batch."""
         if check_pixel_format(pixel_format, color_matrix, color_range):
             if video_u8.dim() != 3:
                 raise ValueError(f"expected [N,R,P] {pixel_format} surfaces, got {tuple(video_u8.shape)}")

@@ -124,3 +124,42 @@ def rgb_to_yuv420(clip: np.ndarray, layout: str = "nv12", matrix: str = "bt601",
         planes[..., lr // 2: lr // 2 + h // 2, : w // 2] = q(v)
         out[..., lr:, :] = planes.reshape(lead + (lr // 2, p))
     return out
+
+
+def rgb_to_yuv420_16(clip: np.ndarray, layout: str = "p010", matrix: str = "bt601", range_: str = "limited",
+                     luma_rows: int = None, pitch: int = None) -> np.ndarray:
+    """Synthetic 10-bit decoder surfaces: uint8 ``[...,H,W,3]`` -> uint16 ``[...,L*3/2,P]`` (``P`` the pitch in samples),
+    ``layout`` "p010" (semi-planar, the 10 bits in the high bits of each word) or "i010" (planar, the 10 bits in the low
+    bits: yuv420p10le).  The encode is the float64 one of ``rgb_to_yuv420`` at 10-bit precision, a 10-bit code being
+    4 x the 8-bit one (limited range: Y in [64, 940]); every padding sample is 0xFFFF."""
+    if layout not in ("p010", "i010") or range_ not in ("limited", "full"):
+        raise ValueError(f"unknown range or layout: {range_!r}, {layout!r}")
+    kr, kb = {"bt601": (0.299, 0.114), "bt709": (0.2126, 0.0722)}[matrix]
+    x = clip.astype(np.float64)
+    h, w = x.shape[-3], x.shape[-2]
+    lr = h if luma_rows is None else luma_rows
+    p = w if pitch is None else pitch
+    if h % 2 or w % 2 or lr % 2 or lr < h or p < w or p % 2:
+        raise ValueError(f"bad surface: picture {h}x{w}, luma rows {lr}, pitch {p}")
+    yv = kr * x[..., 0] + (1 - kr - kb) * x[..., 1] + kb * x[..., 2]
+    blk = x.reshape(x.shape[:-3] + (h // 2, 2, w // 2, 2, 3)).mean(axis=(-4, -2))
+    ym = kr * blk[..., 0] + (1 - kr - kb) * blk[..., 1] + kb * blk[..., 2]
+    pb = (blk[..., 2] - ym) / (2 * (1 - kb))
+    pr = (blk[..., 0] - ym) / (2 * (1 - kr))
+    if range_ == "limited":
+        y, u, v = 16 + yv * 219 / 255, 128 + pb * 224 / 255, 128 + pr * 224 / 255
+    else:
+        y, u, v = yv, 128 + pb, 128 + pr
+    shift = 6 if layout == "p010" else 0
+    q = lambda a: (np.clip(np.floor(4 * a + 0.5), 0, 1023).astype(np.uint16) << shift).astype(np.uint16)
+    lead = x.shape[:-3]
+    out = np.full(lead + (lr * 3 // 2, p), 0xFFFF, np.uint16)
+    out[..., :h, :w] = q(y)
+    if layout == "p010":
+        out[..., lr: lr + h // 2, :w] = np.stack([q(u), q(v)], axis=-1).reshape(lead + (h // 2, w))
+    else:
+        planes = np.full(lead + (lr, p // 2), 0xFFFF, np.uint16)   # U plane rows, then V plane rows, P/2 samples each
+        planes[..., : h // 2, : w // 2] = q(u)
+        planes[..., lr // 2: lr // 2 + h // 2, : w // 2] = q(v)
+        out[..., lr:, :] = planes.reshape(lead + (lr // 2, p))
+    return out

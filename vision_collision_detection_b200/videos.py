@@ -29,7 +29,7 @@ import torch
 from torch.utils.data import Dataset, default_collate
 
 from .sensors import find_sensor_path, load_and_sync_sensor, window_sensor
-from .video_aug import GpuVideoTransform, check_pixel_format
+from .video_aug import GpuVideoTransform, check_pixel_format, source_dtype
 
 
 # ---------------------------------------------------------------------------------
@@ -131,12 +131,21 @@ def _source_format(defer: bool, pixel_format: str, color_matrix: str, color_rang
 
 def _blank_frame(shape, fmt: Optional[Dict[str, str]]) -> np.ndarray:
     """A frame that converts to RGB zeros: zero bytes for RGB; for a YUV surface ``[H*3/2,W]`` Y = 16 (limited range)
-    or 0 (full range) and U = V = 128 (zero bytes there would be a strongly coloured picture)."""
+    or 0 (full range) and U = V = 128 (zero bytes there would be a strongly coloured picture), in the sample scale of
+    the format: 16 << 8 and 32768 for p010, 64 and 512 for i010."""
     if fmt is None:
         return np.zeros(shape, np.uint8)
-    f = np.full(shape, 128, np.uint8)
-    f[: shape[0] * 2 // 3] = 16 if fmt["color_range"] == "limited" else 0
+    scale = {"p010": 256, "i010": 4}.get(fmt["pixel_format"], 1)
+    f = np.full(shape, 128 * scale, np.uint16 if scale > 1 else np.uint8)
+    f[: shape[0] * 2 // 3] = 16 * scale if fmt["color_range"] == "limited" else 0
     return f
+
+
+def _check_surfaces(frames: torch.Tensor, fmt: Optional[Dict[str, str]]) -> None:
+    """A decoder that delivers the wrong element type for its YUV format is a set-up error, not a failed item."""
+    if fmt is not None and frames.dtype != source_dtype(fmt["pixel_format"]):
+        raise ValueError(f"{fmt['pixel_format']} decoder output must be {source_dtype(fmt['pixel_format'])} [n,H*3/2,W] "
+                         f"surfaces, got {frames.dtype}")
 
 
 def _picture_hw(frames, fmt: Optional[Dict[str, str]]):
@@ -154,7 +163,8 @@ class GpuDashcamDataset(Dataset):
 
     ``pixel_format="nv12"`` / ``"i420"`` (``defer=True`` only): the decoder's ``get_batch`` returns packed YUV 4:2:0
     surfaces ``[n,H*3/2,W]``; they are what crosses to the main process (half the bytes of RGB) and ``GpuAugLoader``
-    converts them on the device with ``color_matrix`` / ``color_range``."""
+    converts them on the device with ``color_matrix`` / ``color_range``.  ``"p010"`` / ``"i010"``: uint16 surfaces of
+    10-bit video (see ``GpuVideoTransform.forward_batch``), as many bytes as RGB."""
 
     def __init__(self, metadata_df, base_dirs=None, fps=10, duration=5, is_train=True, skip_missing=True,
                  transform: Optional[GpuVideoTransform] = None, sample_strategy="random", sensor_subdir="signals",
@@ -253,6 +263,7 @@ class GpuDashcamDataset(Dataset):
             return {"frames": torch.zeros(need, size[0], size[1], 3), "sensor": torch.zeros(need, 4), "target": target,
                     "id": vid}
         if self.defer:
+            _check_surfaces(frames, self.source_format)
             t = self.transform
             params = t.sample_params(1, *_picture_hw(frames, self.source_format))[0] if t is not None else None
             item = {"frames_u8": frames, "params": params, "sensor": sensor, "target": target, "id": vid, "need": need}
@@ -344,6 +355,7 @@ class GpuVideoDataset(Dataset):
             size = (224, 224) if self.transform else (720, 1280)   # ncwv:183-190
             return {"frames": torch.zeros(need, size[0], size[1], 3), "target": label, "id": vid}
         if self.defer:
+            _check_surfaces(frames, self.source_format)
             t = self.transform
             params = t.sample_params(1, *_picture_hw(frames, self.source_format))[0] if t is not None else None
             item = {"frames_u8": frames, "params": params, "target": label, "id": vid, "need": need}
