@@ -54,7 +54,12 @@ enum {
  * nexar_plan_create(g, NEXAR_SRC_NV12, ...) is nexar_plan_create_yuv(g, {NV12, BT601, LIMITED, 0}, ...); the other
  * 4:2:0 variants (I420, BT.709, full range, padded luma height) are described by NexarYuvFormat below. */
 enum { NEXAR_SRC_U8 = 0, NEXAR_SRC_F32 = 1, NEXAR_SRC_NV12 = 2 };
-enum { NEXAR_DST_F32 = 0, NEXAR_DST_BF16 = 1 };
+/* Destination element type.  BF16 and F16 elements are the fp32 value the NEXAR_DST_F32 output of the same call holds,
+ * rounded to nearest even (__float2bfloat16_rn / __float2half_rn).  F16 is therefore bit for bit what
+ * torch.Tensor.to(torch.float16) makes of the F32 output, as fp16 autocast does with it; values beyond fp16's range
+ * become +-inf, as that conversion gives.  Any other value is NEXAR_ERR_INVALID; a library built before F16 existed
+ * refuses 2 the same way ("bad dst_dtype"), so it never falls back to another type. */
+enum { NEXAR_DST_F32 = 0, NEXAR_DST_BF16 = 1, NEXAR_DST_F16 = 2 };
 
 /* NexarClipParams.flags */
 enum {

@@ -8,7 +8,7 @@ the fused GPU augmentation.  Reports t_aug / t_step from CUDA events (max over r
 library code (torchvision / cuDNN) and is NOT part of the product; this script only measures how much of
 a real step the transform now costs.
 
-  python tools/train_step_share.py [--batch 8] [--frames 16] [--steps 10]
+  python tools/train_step_share.py [--batch 8] [--frames 16] [--steps 10] [--out-dtype f32|f16]
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/train_step_share.py
 """
 import argparse
@@ -52,6 +52,8 @@ def main():
     ap.add_argument("--frames", type=int, default=16)
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--out-dtype", default="f32", choices=["f32", "f16"],
+                    help="transform output: f16 is what autocast makes of the f32 output, at half the bytes")
     ap.add_argument("--sync-every-step", action="store_true", help="synchronize after every step (unoverlapped transform latency)")
     args = ap.parse_args()
     rank, world, local = (int(os.environ.get(k, d)) for k, d in (("RANK", 0), ("WORLD_SIZE", 1), ("LOCAL_RANK", 0)))
@@ -73,12 +75,13 @@ def main():
     # One event triple per step and a single synchronize at the end: like a real training loop the host runs ahead of the
     # device, so ev[0] -> ev[1] is the time the DEVICE spends on the transform inside a step (the host-side parameter
     # packing of step i+1 overlaps the model's kernels of step i); --sync-every-step gives the unoverlapped latency instead.
+    out_dtype = {"f32": torch.float32, "f16": torch.float16}[args.out_dtype]
     n_total = args.warmup + args.steps
     evs = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(n_total)]
     for i in range(n_total):
         ev = evs[i]
         ev[0].record()
-        x = tf.forward_batch(clips)                                   # [B,3,T,224,224] fp32
+        x = tf.forward_batch(clips, out_dtype=out_dtype)              # [B,3,T,224,224]
         ev[1].record()
         with torch.autocast("cuda", dtype=torch.float16):
             loss = nn.functional.cross_entropy(model(x), labels)
@@ -101,7 +104,8 @@ def main():
                           "cfg5 (1 GPU): convnext_tiny+GRU (random init), fp16 autocast, AdamW",
                           "model": "stand-in with the input contract and layer types of nexar_arch.EnhancedFrameCNN('convnext_tiny', "
                                    "temporal_mode='gru') (nexar_arch.py:390-443), built from torchvision; NOT the reference class",
-                          "aug": "nexar_videos.py:2003-2010 kwargs, device-resident uint8 720p clips -> fp32 [B,3,T,224,224]",
+                          "aug": "nexar_videos.py:2003-2010 kwargs, device-resident uint8 720p clips -> "
+                                 f"{'fp32' if args.out_dtype == 'f32' else 'fp16'} [B,3,T,224,224]",
                           "n_gpus": world, "batch_per_gpu": args.batch, "frames": args.frames,
                           "ms_aug": a, "ms_step": s, "aug_share": a / s, "sync_every_step": bool(args.sync_every_step), "clips_per_s": world * args.batch / (s * 1e-3)}))
     if world > 1:

@@ -26,7 +26,7 @@ SRC_U8, SRC_F32, SRC_NV12 = 0, 1, 2
 YUV_NV12, YUV_I420 = 0, 1
 YUV_BT601, YUV_BT709 = 0, 1
 YUV_LIMITED, YUV_FULL = 0, 1
-DST_F32, DST_BF16 = 0, 1
+DST_F32, DST_BF16, DST_F16 = 0, 1, 2
 FLIP, AUG, AFFINE, GRAYSCALE, NOISE, BLUR, POSTERIZE, SOLARIZE, INVERT, CUTOUT = (1 << i for i in range(10))
 MAX_CUTOUT = 8
 MAX_BLUR_TAPS = 33

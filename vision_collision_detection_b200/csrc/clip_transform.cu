@@ -15,6 +15,7 @@
 // a second, normally empty, launch (fixup_frame_kernel) redoes the clips whose maximum was <= 1.
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 #include <cmath>
 #include <type_traits>
@@ -609,6 +610,10 @@ template <>
 __device__ __forceinline__ void store_out<__nv_bfloat16>(void* dst, int64_t idx, float v) {
   ((__nv_bfloat16*)dst)[idx] = __float2bfloat16_rn(v);
 }
+template <>
+__device__ __forceinline__ void store_out<__half>(void* dst, int64_t idx, float v) {
+  ((__half*)dst)[idx] = __float2half_rn(v);
+}
 
 // same, through an explicit st.global (for pointers whose provenance the compiler cannot see)
 template <typename T>
@@ -620,6 +625,11 @@ __device__ __forceinline__ void store_out_global<float>(float* p, float v) {
 template <>
 __device__ __forceinline__ void store_out_global<__nv_bfloat16>(__nv_bfloat16* p, float v) {
   const unsigned short h = __bfloat16_as_ushort(__float2bfloat16_rn(v));
+  asm volatile("st.global.u16 [%0], %1;" ::"l"(p), "h"(h) : "memory");
+}
+template <>
+__device__ __forceinline__ void store_out_global<__half>(__half* p, float v) {
+  const unsigned short h = __half_as_ushort(__float2half_rn(v));
   asm volatile("st.global.u16 [%0], %1;" ::"l"(p), "h"(h) : "memory");
 }
 
@@ -1463,13 +1473,18 @@ __device__ __forceinline__ void store_pair<__nv_bfloat16>(__nv_bfloat16* p, floa
   const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
   asm volatile("st.global.b32 [%0], %1;" ::"l"(p), "r"(*(const unsigned*)&h) : "memory");
 }
+template <>
+__device__ __forceinline__ void store_pair<__half>(__half* p, float a, float b) {
+  const __half2 h = __floats2half2_rn(a, b);
+  asm volatile("st.global.b32 [%0], %1;" ::"l"(p), "r"(*(const unsigned*)&h) : "memory");
+}
 
 // ---------------------------------------------------------------------------------
 // Augmentation tail of fixup_frame_kernel: K1.5 + K2 + K3 of one frame inside the CTA of 256 threads that has just
 // resampled all of it (rows B.i_lo .. B.i_hi, gray sum in slot 1).
 //   phase B  contrast -> saturation -> hue in place on the frame's rows of the intermediate;
 //   phase C  the OUTPUT in tiles of 32 x 4 pixels pulled from a shared counter: a warp owns one tile at a time, two
-//            horizontally adjacent pixels per lane (one 32-bit bf16x2 / 64-bit float2 store per channel), classified
+//            horizontally adjacent pixels per lane (one 32-bit bf16x2 / f16x2 / 64-bit float2 store per channel), classified
 //            FILL / INTERIOR / general exactly like geometry_kernel; the four neighbours are 8-byte loads of the q15
 //            intermediate (L2 / L1 hits: this CTA wrote them microseconds ago), unpacked with one PRMT per sample:
 //              sum_canvas(w * img) = pad * (m - wc) + k * sum_content(w * F) - k * wc,   F = 1 + q / 32768, k = 32768 / 32767
@@ -1730,7 +1745,7 @@ __global__ void __launch_bounds__(256) fixup_frame_kernel(const __grid_constant_
 // computed ONCE and reused for kGeoFrames consecutive frames of the clip; per frame only the pad colour changes.
 // CTA = 8 warps, a warp owns a tile of 32 x 4 output pixels (lane -> x pair = lane & 15, row = lane >> 4, two passes two
 // rows apart) x kGeoFrames frames: two horizontally adjacent pixels per lane, so every channel goes out as one 32-bit
-// bf16x2 / 64-bit float2 store.  The tile is classified once, by every lane identically, from the image of its centre
+// bf16x2 / f16x2 / 64-bit float2 store.  The tile is classified once, by every lane identically, from the image of its centre
 // and the half extents of the affine map: FILL — maps strictly inside the canvas and entirely into the pad band beside
 // the content: constant pad colour, no loads; INTERIOR — every bilinear neighbour is a content pixel (one address,
 // weights as they are, m = wc = 1); otherwise the four addresses are clamped into the content box and the weights of
@@ -2739,7 +2754,8 @@ extern "C" int nexar_clip_transform(const NexarPlan* p, const NexarTransformArgs
   if ((int64_t)a->n_clips * a->frames_per_clip > 65535)  // frames are a grid dimension (y / z): split larger batches
     return fail(NEXAR_ERR_UNSUPPORTED, "clip_transform: more than 65535 frames in one call");
   if (!a->src || !a->frame_offsets || !a->params || !a->dst) return fail(NEXAR_ERR_INVALID, "clip_transform: null buffer");
-  if (a->dst_dtype != NEXAR_DST_F32 && a->dst_dtype != NEXAR_DST_BF16) return fail(NEXAR_ERR_INVALID, "clip_transform: bad dst_dtype");
+  if (a->dst_dtype != NEXAR_DST_F32 && a->dst_dtype != NEXAR_DST_BF16 && a->dst_dtype != NEXAR_DST_F16)
+    return fail(NEXAR_ERR_INVALID, "clip_transform: bad dst_dtype");
   const size_t need = nexar_workspace_bytes_for(p, a->n_clips, a->frames_per_clip, a->any_flags);
   if (!a->workspace || a->workspace_bytes < need) return fail(NEXAR_ERR_WORKSPACE, "clip_transform: workspace too small");
   for (int c = 0; c < 3; ++c)
@@ -2835,8 +2851,10 @@ extern "C" int nexar_clip_transform(const NexarPlan* p, const NexarTransformArgs
   }
   if (p->src_dtype != NEXAR_SRC_F32) {
     if (a->dst_dtype == NEXAR_DST_F32) return launch_chunked<uint8_t, float>(p, a, K, aug_mode, blur_mode);
+    if (a->dst_dtype == NEXAR_DST_F16) return launch_chunked<uint8_t, __half>(p, a, K, aug_mode, blur_mode);
     return launch_chunked<uint8_t, __nv_bfloat16>(p, a, K, aug_mode, blur_mode);
   }
   if (a->dst_dtype == NEXAR_DST_F32) return launch_chunked<float, float>(p, a, K, aug_mode, blur_mode);
+  if (a->dst_dtype == NEXAR_DST_F16) return launch_chunked<float, __half>(p, a, K, aug_mode, blur_mode);
   return launch_chunked<float, __nv_bfloat16>(p, a, K, aug_mode, blur_mode);
 }

@@ -12,7 +12,7 @@ import torch
 
 from . import _lib
 
-_DST = {torch.float32: _lib.DST_F32, torch.bfloat16: _lib.DST_BF16}
+_DST = {torch.float32: _lib.DST_F32, torch.bfloat16: _lib.DST_BF16, torch.float16: _lib.DST_F16}
 _SRC = {torch.uint8: _lib.SRC_U8, torch.float32: _lib.SRC_F32, "nv12": _lib.SRC_NV12}
 
 # output layouts: name -> (shape builder, element strides for (clip, channel, frame, y, x))
