@@ -72,7 +72,12 @@ enum {
   NEXAR_POSTERIZE = 1u << 6,   /* :174 */
   NEXAR_SOLARIZE = 1u << 7,    /* :173 */
   NEXAR_INVERT = 1u << 8,      /* :172 */
-  NEXAR_CUTOUT = 1u << 9       /* :144 */
+  NEXAR_CUTOUT = 1u << 9,      /* :144 */
+  /* The source values are bytes 0..255: scale them by 1/255 whatever the clip's maximum.  Without it the clip is divided
+   * by 255 only when some value is > 1 (nexar_video_aug.py:809-821), so a clip of frames that hold only 0 and 1 (a
+   * near-black stretch) is left unscaled.  A caller that transforms one video in several calls sets it, so that each
+   * call scales as the whole video would be scaled.  Off in every record the library's own callers draw. */
+  NEXAR_RANGE_255 = 1u << 10
 };
 
 #define NEXAR_MAX_CUTOUT 8
@@ -231,6 +236,18 @@ int nexar_clip_transform(const NexarPlan* plan, const NexarTransformArgs* args);
  * dst[k][c][t] = frames[min(k * stride + t, n_frames - 1)][c] (the last frame repeats past the end, nexar_videos.py:429-433). */
 int nexar_gather_windows(const void* frames, int64_t n_frames, int64_t plane_bytes, int32_t window, int32_t stride,
                          int64_t n_windows, void* dst, void* stream);
+/* The same gather from a ring of per-frame results, for a video that is transformed chunk by chunk as it is decoded.
+ * `ring` holds ring_frames slots of 3 planes of plane_bytes each (layout BTCHW of nexar_clip_transform); video frame f
+ * lives in slot f % ring_frames.  dst receives n_windows windows of [3][window] planes with
+ *   dst[k][c][t] = ring[min(first_frame + k * stride + t, last_frame) % ring_frames][c]
+ * i.e. window k starts at video frame first_frame + k * stride and frames past last_frame repeat last_frame.
+ * nexar_gather_windows is the case ring_frames = n_frames, first_frame = 0, last_frame = n_frames - 1.  Requires
+ * 0 <= first_frame <= last_frame, and the frames read, first_frame .. min(first_frame + (n_windows - 1) * stride +
+ * window - 1, last_frame), must number at most ring_frames (more would need a slot twice); else NEXAR_ERR_INVALID.
+ * Planes are copied with 16-byte loads and streaming stores when plane_bytes, ring and dst are multiples of 16, byte by
+ * byte otherwise.  One launch on `stream`. */
+int nexar_gather_windows_ring(const void* ring, int32_t ring_frames, int64_t plane_bytes, int32_t window, int32_t stride,
+                              int64_t first_frame, int64_t last_frame, int64_t n_windows, void* dst, void* stream);
 
 /* Number of kernel launches the last nexar_clip_transform call on this thread enqueued. */
 int nexar_last_launch_count(void);

@@ -27,7 +27,7 @@ YUV_NV12, YUV_I420 = 0, 1
 YUV_BT601, YUV_BT709 = 0, 1
 YUV_LIMITED, YUV_FULL = 0, 1
 DST_F32, DST_BF16, DST_F16 = 0, 1, 2
-FLIP, AUG, AFFINE, GRAYSCALE, NOISE, BLUR, POSTERIZE, SOLARIZE, INVERT, CUTOUT = (1 << i for i in range(10))
+FLIP, AUG, AFFINE, GRAYSCALE, NOISE, BLUR, POSTERIZE, SOLARIZE, INVERT, CUTOUT, RANGE_255 = (1 << i for i in range(11))
 MAX_CUTOUT = 8
 MAX_BLUR_TAPS = 33
 
@@ -176,6 +176,26 @@ def yuv16_lib():
                                "convert p010 / i010 frames") from None
         fn.argtypes = [C.POINTER(Geometry), C.POINTER(YuvFormat), C.c_int32, C.POINTER(C.c_void_p)]
         _yuv16_bound = True
+    return L
+
+
+_ring_bound = False
+
+
+def ring_lib():
+    """``lib()`` with ``nexar_gather_windows_ring`` bound, on first use only: a library built before it existed serves
+    every other call and refuses window streams with this error."""
+    global _ring_bound
+    L = lib()
+    if not _ring_bound:
+        try:
+            fn = L.nexar_gather_windows_ring
+        except AttributeError:
+            raise RuntimeError(f"{LIB_PATH} predates window streams (no nexar_gather_windows_ring); rebuild it to "
+                               "stream sliding windows") from None
+        fn.argtypes = [C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int64,
+                       C.c_void_p, C.c_void_p]
+        _ring_bound = True
     return L
 
 

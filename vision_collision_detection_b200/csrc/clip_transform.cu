@@ -735,6 +735,10 @@ template <typename SrcT>
 __global__ void clip_max_kernel(DevPlan P, KArgs A) {
   const int frame = blockIdx.y;
   const int clip = frame / A.T;
+  if (A.params[clip].flags & NEXAR_RANGE_255) {  // byte-range values: divided by 255 whatever the maximum
+    if (threadIdx.x == 0) atomicOr(&A.clip_max[clip], 1u);
+    return;
+  }
   const char* base = (const char*)A.src + A.frame_offsets[frame];
   const int n = P.src_w * 3;
   float m = -INFINITY;
@@ -781,7 +785,7 @@ __device__ __forceinline__ void resize_general_body(const DevPlan& P, const KArg
     nbi[c] = A.normalize ? A.nbias[c] : 0.0f;
   }
   const int64_t dbase = (int64_t)clip * A.sb + (int64_t)t * A.st;
-  float vmax = -INFINITY;
+  float vmax = (flags & NEXAR_RANGE_255) ? INFINITY : -INFINITY;  // byte-range clips count as "max > 1" from the start
   unsigned long long gsum = 0ull;  // one thread may cover many pixels here
 
   for (int i = i0; i < i1; ++i) {
@@ -1206,7 +1210,7 @@ resize_fast_kernel(const __grid_constant__ DevPlan P, const __grid_constant__ KA
 
   if (!aug) fill_pads<DstT, NT>(P, A, B, dbase, band, nb, i0, i1, tid);
   if (A.pass == 0) {
-    const bool big = (orv & 0xFEFEFEFEu) != 0u;
+    const bool big = (orv & 0xFEFEFEFEu) != 0u || (flags & NEXAR_RANGE_255) != 0u;
     if (__any_sync(0xffffffffu, big) && (tid & 31) == 0) atomicOr(&A.clip_max[clip], 1u);
   }
   if (aug) {
@@ -2705,19 +2709,22 @@ static int launch_chunked(const NexarPlan* p, const NexarTransformArgs* a, const
 
 // ---------------------------------------------------------------------------------
 // Materialised sliding windows (BASELINE config 4): the val chain is per frame, so a video is transformed once into
-// [N][3][cs][cs] planes and window k = frames k*stride .. k*stride+window-1 (the last frame repeated past the end,
-// nexar_videos.py:429-433).  dst[k][c][t] = frames[min(k*stride + t, N-1)][c]: whole-plane copies, 16 bytes per thread.
+// [3][cs][cs] planes per frame and window k = frames first + k*stride .. first + k*stride+window-1 (the last frame repeated
+// past the end, nexar_videos.py:429-433).  The per-frame results live in a ring of ring_frames slots (video frame f in
+// slot f % ring_frames; a whole video is the ring of n_frames slots):
+// dst[k][c][t] = ring[min(first + k*stride + t, last) % ring_frames][c].  Whole-plane copies, 16 bytes per thread.
 // ---------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) gather_windows_kernel(const unsigned char* __restrict__ frames, long long n_frames, long long plane_bytes,
-                                                             int window, int stride, unsigned char* __restrict__ dst) {
+__global__ void __launch_bounds__(256) gather_windows_kernel(const unsigned char* __restrict__ ring, long long ring_frames,
+                                                             long long plane_bytes, int window, int stride, long long first_frame,
+                                                             long long last_frame, unsigned char* __restrict__ dst) {
   const long long plane = blockIdx.x;              // (k * 3 + c) * window + t
   const int t = (int)(plane % window);
   const long long kc = plane / window;
   const int c = (int)(kc % 3);
   const long long k = kc / 3;
-  long long f = k * stride + t;
-  if (f > n_frames - 1) f = n_frames - 1;
-  const unsigned char* s = frames + (f * 3 + c) * plane_bytes;
+  long long f = first_frame + k * stride + t;
+  if (f > last_frame) f = last_frame;
+  const unsigned char* s = ring + ((f % ring_frames) * 3 + c) * plane_bytes;
   unsigned char* d = dst + plane * plane_bytes;
   const long long lo = (long long)blockIdx.y * plane_bytes / gridDim.y, hi = (long long)(blockIdx.y + 1) * plane_bytes / gridDim.y;
   if ((plane_bytes & 15) == 0 && (lo & 15) == 0 && (hi & 15) == 0 && ((((uintptr_t)s) | ((uintptr_t)d)) & 15) == 0) {
@@ -2730,20 +2737,38 @@ __global__ void __launch_bounds__(256) gather_windows_kernel(const unsigned char
   }
 }
 
-extern "C" int nexar_gather_windows(const void* frames, int64_t n_frames, int64_t plane_bytes, int32_t window, int32_t stride,
-                                    int64_t n_windows, void* dst, void* stream) {
-  if (!frames || !dst || n_frames <= 0 || plane_bytes <= 0 || window <= 0 || stride <= 0 || n_windows <= 0)
-    return fail(NEXAR_ERR_INVALID, "gather_windows: bad argument");
+static int gather_windows(const char* who, const void* ring, int64_t ring_frames, int64_t plane_bytes, int32_t window,
+                          int32_t stride, int64_t first_frame, int64_t last_frame, int64_t n_windows, void* dst, void* stream) {
+  if (!ring || !dst || ring_frames <= 0 || plane_bytes <= 0 || window <= 0 || stride <= 0 || n_windows <= 0 ||
+      first_frame < 0 || last_frame < first_frame)
+    return fail(NEXAR_ERR_INVALID, std::string(who) + ": bad argument");
   const int64_t planes = n_windows * 3 * window;
-  if (planes > 2147483647LL) return fail(NEXAR_ERR_UNSUPPORTED, "gather_windows: more than 2^31 planes");
+  if (n_windows > 2147483647LL || planes > 2147483647LL) return fail(NEXAR_ERR_UNSUPPORTED, std::string(who) + ": more than 2^31 planes");
+  // the frames one call reads, first_frame .. min(first_frame + (n_windows-1)*stride + window-1, last_frame), must each
+  // have a slot of their own: a wider span would read a slot that has been overwritten with a later frame
+  const int64_t reach = (n_windows - 1) * stride + window - 1;
+  if ((reach < last_frame - first_frame ? reach : last_frame - first_frame) >= ring_frames)
+    return fail(NEXAR_ERR_INVALID, std::string(who) + ": the windows span more frames than the ring holds");
   // each plane is split over `split` CTAs so that short videos still fill the machine; splits fall on 16-byte boundaries
   int split = 1;
   while (split < 8 && planes * split < 4 * (int64_t)sm_count() && (plane_bytes / (2 * split)) % 16 == 0 && plane_bytes / (2 * split) >= 4096) split *= 2;
-  gather_windows_kernel<<<dim3((unsigned)planes, split), 256, 0, (cudaStream_t)stream>>>((const unsigned char*)frames, n_frames, plane_bytes,
-                                                                                       window, stride, (unsigned char*)dst);
+  gather_windows_kernel<<<dim3((unsigned)planes, split), 256, 0, (cudaStream_t)stream>>>((const unsigned char*)ring, ring_frames, plane_bytes,
+                                                                                       window, stride, first_frame, last_frame,
+                                                                                       (unsigned char*)dst);
   CUDA_TRY(cudaGetLastError());
   g_launches = 1;
   return NEXAR_OK;
+}
+
+extern "C" int nexar_gather_windows(const void* frames, int64_t n_frames, int64_t plane_bytes, int32_t window, int32_t stride,
+                                    int64_t n_windows, void* dst, void* stream) {
+  return gather_windows("gather_windows", frames, n_frames, plane_bytes, window, stride, 0, n_frames - 1, n_windows, dst, stream);
+}
+
+extern "C" int nexar_gather_windows_ring(const void* ring, int32_t ring_frames, int64_t plane_bytes, int32_t window, int32_t stride,
+                                         int64_t first_frame, int64_t last_frame, int64_t n_windows, void* dst, void* stream) {
+  return gather_windows("gather_windows_ring", ring, ring_frames, plane_bytes, window, stride, first_frame, last_frame,
+                        n_windows, dst, stream);
 }
 
 extern "C" int nexar_clip_transform(const NexarPlan* p, const NexarTransformArgs* a) {

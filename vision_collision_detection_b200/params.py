@@ -141,7 +141,7 @@ _WORDS = _lib.CLIP_PARAMS_DTYPE.itemsize // 4
 
 def pack_clip_params(records: Sequence[Dict[str, Any]], canvas: int,
                      aug_cfg: Optional[VideoAugmentation] = None) -> Tuple[np.ndarray, int]:
-    """records[i] = {'flip': bool, 'aug': dict|None, 'crop': (dy, dx)|None} ->
+    """records[i] = {'flip': bool, 'aug': dict|None, 'crop': (dy, dx)|None, optional 'range_255': bool} ->
     (structured array of NexarClipParams, OR of all flags).  Raises the errors
     torchvision would raise for out-of-range factors.  Scalars are gathered into
     per-field columns and written with a few vectorised assignments (this runs once
@@ -158,6 +158,8 @@ def pack_clip_params(records: Sequence[Dict[str, Any]], canvas: int,
     any_flags = 0
     for i, rec in enumerate(records):
         flags = _lib.FLIP if rec.get("flip") else 0
+        if rec.get("range_255"):      # bytes 0..255: divided by 255 whatever the clip's maximum (WindowStream's chunks)
+            flags |= _lib.RANGE_255
         crop = rec.get("crop")
         if crop is not None:
             iview[i, _F["crop_dy"]] = int(crop[0])

@@ -187,13 +187,16 @@ class GpuVideoTransform(nn.Module):
         """The never-called factory's default forward (nexar_video_aug.py:407-463): an antialiased short-side
         resize followed by a SECOND antialiased resize inside crop_tensor(use_letterbox=True).  Pass 1 writes
         the [0,1] float frames of size (rh, rw) on a square scratch canvas; pass 2 letterboxes those float
-        frames (strided rows) and applies flip / augmentation / normalisation."""
+        frames (strided rows) and applies flip / augmentation / normalisation.  A record's byte-range flag describes the
+        source frames, so it goes to pass 1 only: pass 2 reads values that are already in [0,1]."""
         h, w = frames.shape[2], frames.shape[3]
         rh, rw = self._resized_hw(h, w)
         cm = max(rh, rw)
         plan1 = eng.plan(_lib.Geometry(h, w, cm, rh, rw, 0, 0), _SRC[frames.dtype])
         mid, mid_strides = _alloc_out("BTHWC", n_clips, t_out, cm, torch.float32, frames.device)
-        neutral, _ = pack_clip_params([{"flip": False, "aug": None}] * n_clips, cm, None)
+        range_255 = packed["flags"] & _lib.RANGE_255
+        neutral, _ = pack_clip_params([{"flip": False, "aug": None, "range_255": bool(r)} for r in range_255], cm, None)
+        packed["flags"] &= ~range_255
         eng.run(plan1, frames, offsets, n_clips, t_out, eng.upload_params(neutral), 0, mid, mid_strides,
                 False, self.video_mean, self.video_std)
         plan2 = eng.plan(_lib.letterbox_geometry(rh, rw, self.crop_size), _lib.SRC_F32)
