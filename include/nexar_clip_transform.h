@@ -248,6 +248,18 @@ int nexar_gather_windows(const void* frames, int64_t n_frames, int64_t plane_byt
  * byte otherwise.  One launch on `stream`. */
 int nexar_gather_windows_ring(const void* ring, int32_t ring_frames, int64_t plane_bytes, int32_t window, int32_t stride,
                               int64_t first_frame, int64_t last_frame, int64_t n_windows, void* dst, void* stream);
+/* The same gather through a slot table, for many streams whose per-frame results share one pool.  `pool` holds
+ * pool_frames slots of 3 planes of plane_bytes each (layout BTCHW of nexar_clip_transform); `slots` is a device int32
+ * table of n_windows * window entries.  Exactly one of dst and dst_slots is non-NULL:
+ *   dst:       dst[k][c][t] = pool[slots[k * window + t]][c]        (n_windows windows of [3][window] planes)
+ *   dst_slots: pool[dst_slots[i]][c] = pool[slots[i]][c]            (window must be 1; i < n_windows; a device int32 table)
+ * Every slot read from either table is clamped into [0, pool_frames), so no table can address outside the pool; a
+ * destination slot that is also read by the same call gives an undefined value in that slot only.  NEXAR_ERR_INVALID for
+ * a null pool or slots, both or neither of dst / dst_slots, pool_frames, plane_bytes, window or n_windows <= 0, dst_slots
+ * with window != 1, and more than 2^31 - 1 planes.  Planes are copied as by nexar_gather_windows_ring.  One launch on
+ * `stream`. */
+int nexar_gather_windows_table(const void* pool, int32_t pool_frames, int64_t plane_bytes, int32_t window, const int32_t* slots,
+                               int64_t n_windows, void* dst, const int32_t* dst_slots, void* stream);
 
 /* Number of kernel launches the last nexar_clip_transform call on this thread enqueued. */
 int nexar_last_launch_count(void);

@@ -199,6 +199,26 @@ def ring_lib():
     return L
 
 
+_table_bound = False
+
+
+def table_lib():
+    """``lib()`` with ``nexar_gather_windows_table`` bound, on first use only: a library built before it existed serves
+    every other call and refuses multi-stream windows with this error."""
+    global _table_bound
+    L = lib()
+    if not _table_bound:
+        try:
+            fn = L.nexar_gather_windows_table
+        except AttributeError:
+            raise RuntimeError(f"{LIB_PATH} predates multi-stream windows (no nexar_gather_windows_table); rebuild it to "
+                               "serve many streams") from None
+        fn.argtypes = [C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                       C.c_void_p]
+        _table_bound = True
+    return L
+
+
 def yuv_coefficients(matrix: int, range_: int):
     """-> (Yo, Ys, Rv, Gu, Gv, Bu), the integer conversion coefficients the library uses."""
     out = (C.c_int32 * 6)()

@@ -2713,19 +2713,37 @@ static int launch_chunked(const NexarPlan* p, const NexarTransformArgs* a, const
 // past the end, nexar_videos.py:429-433).  The per-frame results live in a ring of ring_frames slots (video frame f in
 // slot f % ring_frames; a whole video is the ring of n_frames slots):
 // dst[k][c][t] = ring[min(first + k*stride + t, last) % ring_frames][c].  Whole-plane copies, 16 bytes per thread.
+// kTable: the slot of every window frame comes from a device table instead (many streams sharing one pool of per-frame
+// results): dst[k][c][t] = ring[slots[k*window + t]][c], or, with dst_slots (window 1), ring[dst_slots[k]][c].  Slots are
+// clamped into [0, ring_frames): a bad table can never address outside the pool.
 // ---------------------------------------------------------------------------------
+template <bool kTable>
 __global__ void __launch_bounds__(256) gather_windows_kernel(const unsigned char* __restrict__ ring, long long ring_frames,
                                                              long long plane_bytes, int window, int stride, long long first_frame,
-                                                             long long last_frame, unsigned char* __restrict__ dst) {
+                                                             long long last_frame, unsigned char* __restrict__ dst,
+                                                             const int* __restrict__ slots, const int* __restrict__ dst_slots) {
   const long long plane = blockIdx.x;              // (k * 3 + c) * window + t
   const int t = (int)(plane % window);
   const long long kc = plane / window;
   const int c = (int)(kc % 3);
   const long long k = kc / 3;
-  long long f = first_frame + k * stride + t;
-  if (f > last_frame) f = last_frame;
-  const unsigned char* s = ring + ((f % ring_frames) * 3 + c) * plane_bytes;
-  unsigned char* d = dst + plane * plane_bytes;
+  const unsigned char* s;
+  unsigned char* d;
+  if constexpr (kTable) {
+    const long long f = min(max((long long)__ldg(slots + k * window + t), 0LL), ring_frames - 1);
+    s = ring + (f * 3 + c) * plane_bytes;
+    if (dst_slots) {
+      const long long g = min(max((long long)__ldg(dst_slots + k), 0LL), ring_frames - 1);
+      d = dst + (g * 3 + c) * plane_bytes;
+    } else {
+      d = dst + plane * plane_bytes;
+    }
+  } else {
+    long long f = first_frame + k * stride + t;
+    if (f > last_frame) f = last_frame;
+    s = ring + ((f % ring_frames) * 3 + c) * plane_bytes;
+    d = dst + plane * plane_bytes;
+  }
   const long long lo = (long long)blockIdx.y * plane_bytes / gridDim.y, hi = (long long)(blockIdx.y + 1) * plane_bytes / gridDim.y;
   if ((plane_bytes & 15) == 0 && (lo & 15) == 0 && (hi & 15) == 0 && ((((uintptr_t)s) | ((uintptr_t)d)) & 15) == 0) {
     const uint4* s4 = (const uint4*)(s + lo);
@@ -2735,6 +2753,21 @@ __global__ void __launch_bounds__(256) gather_windows_kernel(const unsigned char
   } else {
     for (long long i = lo + threadIdx.x; i < hi; i += blockDim.x) d[i] = s[i];
   }
+}
+
+// each plane is split over `split` CTAs so that short videos still fill the machine; splits fall on 16-byte boundaries
+template <bool kTable>
+static int launch_gather_windows(int64_t planes, const void* ring, int64_t ring_frames, int64_t plane_bytes, int32_t window,
+                                 int32_t stride, int64_t first_frame, int64_t last_frame, void* dst, const int32_t* slots,
+                                 const int32_t* dst_slots, void* stream) {
+  int split = 1;
+  while (split < 8 && planes * split < 4 * (int64_t)sm_count() && (plane_bytes / (2 * split)) % 16 == 0 && plane_bytes / (2 * split) >= 4096) split *= 2;
+  gather_windows_kernel<kTable><<<dim3((unsigned)planes, split), 256, 0, (cudaStream_t)stream>>>(
+      (const unsigned char*)ring, ring_frames, plane_bytes, window, stride, first_frame, last_frame, (unsigned char*)dst, slots,
+      dst_slots);
+  CUDA_TRY(cudaGetLastError());
+  g_launches = 1;
+  return NEXAR_OK;
 }
 
 static int gather_windows(const char* who, const void* ring, int64_t ring_frames, int64_t plane_bytes, int32_t window,
@@ -2749,15 +2782,8 @@ static int gather_windows(const char* who, const void* ring, int64_t ring_frames
   const int64_t reach = (n_windows - 1) * stride + window - 1;
   if ((reach < last_frame - first_frame ? reach : last_frame - first_frame) >= ring_frames)
     return fail(NEXAR_ERR_INVALID, std::string(who) + ": the windows span more frames than the ring holds");
-  // each plane is split over `split` CTAs so that short videos still fill the machine; splits fall on 16-byte boundaries
-  int split = 1;
-  while (split < 8 && planes * split < 4 * (int64_t)sm_count() && (plane_bytes / (2 * split)) % 16 == 0 && plane_bytes / (2 * split) >= 4096) split *= 2;
-  gather_windows_kernel<<<dim3((unsigned)planes, split), 256, 0, (cudaStream_t)stream>>>((const unsigned char*)ring, ring_frames, plane_bytes,
-                                                                                       window, stride, first_frame, last_frame,
-                                                                                       (unsigned char*)dst);
-  CUDA_TRY(cudaGetLastError());
-  g_launches = 1;
-  return NEXAR_OK;
+  return launch_gather_windows<false>(planes, ring, ring_frames, plane_bytes, window, stride, first_frame, last_frame, dst,
+                                      nullptr, nullptr, stream);
 }
 
 extern "C" int nexar_gather_windows(const void* frames, int64_t n_frames, int64_t plane_bytes, int32_t window, int32_t stride,
@@ -2769,6 +2795,17 @@ extern "C" int nexar_gather_windows_ring(const void* ring, int32_t ring_frames, 
                                          int64_t first_frame, int64_t last_frame, int64_t n_windows, void* dst, void* stream) {
   return gather_windows("gather_windows_ring", ring, ring_frames, plane_bytes, window, stride, first_frame, last_frame,
                         n_windows, dst, stream);
+}
+
+extern "C" int nexar_gather_windows_table(const void* pool, int32_t pool_frames, int64_t plane_bytes, int32_t window,
+                                          const int32_t* slots, int64_t n_windows, void* dst, const int32_t* dst_slots,
+                                          void* stream) {
+  if (!pool || !slots || (dst == nullptr) == (dst_slots == nullptr) || pool_frames <= 0 || plane_bytes <= 0 || window <= 0 ||
+      n_windows <= 0 || (dst_slots && window != 1))
+    return fail(NEXAR_ERR_INVALID, "gather_windows_table: bad argument");
+  if (n_windows > 2147483647LL / (3LL * window)) return fail(NEXAR_ERR_INVALID, "gather_windows_table: more than 2^31 planes");
+  return launch_gather_windows<true>(n_windows * 3 * window, pool, pool_frames, plane_bytes, window, 1, 0, 0,
+                                     dst_slots ? const_cast<void*>(pool) : dst, slots, dst_slots, stream);
 }
 
 extern "C" int nexar_clip_transform(const NexarPlan* p, const NexarTransformArgs* a) {

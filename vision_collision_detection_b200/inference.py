@@ -14,17 +14,21 @@ Every entry point also takes a video of YUV 4:2:0 decoder surfaces ``[N,R,P]`` w
 ``GpuVideoTransform.forward_batch``.
 ``WindowStream`` / ``WindowPredictor.predict_stream`` take the same video chunk by chunk, as a decoder delivers it, and
 keep only the last ``window - 1`` transformed frames plus one chunk on the device: any length, bounded memory.
+``MultiWindowStream`` / ``WindowPredictor.predict_step`` do that for many videos at once (one per camera), with a few
+library calls per step whatever the number of videos.
 """
 from __future__ import annotations
 
 import itertools
-from typing import Any, Callable, Dict, Iterable, Iterator, List, Optional, Tuple
+from typing import Any, Callable, Dict, Iterable, Iterator, List, NamedTuple, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
 
 from . import _lib
-from .video_aug import GpuVideoTransform, check_pixel_format, create_video_transforms, source_dtype
+from .engine import get_engine
+from .params import pack_clip_params
+from .video_aug import GpuVideoTransform, check_pixel_format, create_video_transforms, frame_source, source_dtype
 from .videos import select_start_frame, window_indices
 
 
@@ -118,6 +122,44 @@ def ring_schedule(seen: int, n: int, window: int, stride: int, max_chunk: int) -
     return groups
 
 
+def check_chunk(frames: torch.Tensor, who: str, pixel_format: str = "rgb", color_matrix: str = "bt601",
+                color_range: str = "limited", frame_size=None) -> Tuple[bool, Dict[str, Any], Tuple]:
+    """Validates a chunk of ``n >= 1`` decoded frames and its source-format keywords -> (YUV?, the keywords as a dict,
+    the source key ``(frame shape, dtype, format)`` that every later chunk of the same video must match)."""
+    yuv = check_pixel_format(pixel_format, color_matrix, color_range)
+    if frames.dtype.is_floating_point:
+        raise TypeError(f"{who} takes decoded uint8 frames or YUV surfaces, got {frames.dtype}")
+    if yuv and frames.dim() != 3:
+        raise ValueError(f"expected a chunk of [n,R,P] {pixel_format} surfaces, got {tuple(frames.shape)}")
+    if not yuv and (frames.dim() != 4 or frames.shape[-1] != 3):
+        raise ValueError(f"expected a chunk of [n,H,W,3] frames, got {tuple(frames.shape)}")
+    if frames.shape[0] < 1:
+        raise ValueError("empty chunk")
+    fmt = dict(pixel_format=pixel_format, color_matrix=color_matrix, color_range=color_range,
+               frame_size=None if frame_size is None else (int(frame_size[0]), int(frame_size[1])))
+    return yuv, fmt, (tuple(frames.shape[1:]), frames.dtype, tuple(fmt.values()))
+
+
+def _mismatch(have, source) -> str:
+    return f"the stream's frames are {have}; a chunk of {source} cannot join it"
+
+
+def _draw_record(tf: GpuVideoTransform, frames: torch.Tensor, fmt: Dict[str, Any], yuv: bool) -> Dict[str, Any]:
+    """The parameter record of a video whose first chunk is ``frames``: ``tf.sample_params(1, h, w)`` for the visible
+    ``h x w``, as ``SlidingWindowTransform.frames()`` draws it for the whole video, with the byte-range flag (every chunk
+    is scaled by 1/255, ``NEXAR_RANGE_255``)."""
+    if frames.dtype != source_dtype(fmt["pixel_format"]):
+        raise ValueError(f"{fmt['pixel_format']} frames are {source_dtype(fmt['pixel_format'])}, got {frames.dtype}")
+    if yuv:
+        size = fmt["frame_size"]
+        h, w = (frames.shape[1] * 2 // 3, frames.shape[2]) if size is None else size
+    else:
+        h, w = frames.shape[1], frames.shape[2]
+    rec = dict(tf.sample_params(1, h, w)[0])
+    rec["range_255"] = True
+    return rec
+
+
 class WindowStream:
     """Sliding windows over a video that arrives in chunks of consecutive frames, in bounded device memory.
 
@@ -156,17 +198,7 @@ class WindowStream:
         self._staging: Optional[torch.Tensor] = None
 
     def _start(self, frames: torch.Tensor, yuv: bool):
-        if frames.dtype != source_dtype(self._format["pixel_format"]):
-            raise ValueError(f"{self._format['pixel_format']} frames are {source_dtype(self._format['pixel_format'])}, "
-                             f"got {frames.dtype}")
-        if yuv:
-            size = self._format["frame_size"]
-            h, w = (frames.shape[1] * 2 // 3, frames.shape[2]) if size is None else size
-        else:
-            h, w = frames.shape[1], frames.shape[2]
-        rec = dict(self.tf.sample_params(1, h, w)[0])
-        rec["range_255"] = True
-        self._params = [rec]
+        self._params = [_draw_record(self.tf, frames, self._format, yuv)]
         dev = frames.device if frames.is_cuda else torch.device("cuda", torch.cuda.current_device())
         _lib.ring_lib()           # a library without the ring gather fails here, before any work
         cs = self.tf.crop_size
@@ -189,24 +221,13 @@ class WindowStream:
         """A chunk of ``n >= 1`` consecutive frames -> (start frames, ``[k,3,window,cs,cs]``) of the windows it completes."""
         if self._finished:
             raise ValueError("push() after finish(): start a new WindowStream for the next video")
-        yuv = check_pixel_format(pixel_format, color_matrix, color_range)
-        if frames.dtype.is_floating_point:
-            raise TypeError(f"WindowStream takes decoded uint8 frames or YUV surfaces, got {frames.dtype}")
-        if yuv and frames.dim() != 3:
-            raise ValueError(f"expected a chunk of [n,R,P] {pixel_format} surfaces, got {tuple(frames.shape)}")
-        if not yuv and (frames.dim() != 4 or frames.shape[-1] != 3):
-            raise ValueError(f"expected a chunk of [n,H,W,3] frames, got {tuple(frames.shape)}")
-        if frames.shape[0] < 1:
-            raise ValueError("empty chunk")
-        fmt = dict(pixel_format=pixel_format, color_matrix=color_matrix, color_range=color_range,
-                   frame_size=None if frame_size is None else (int(frame_size[0]), int(frame_size[1])))
-        source = (tuple(frames.shape[1:]), frames.dtype, tuple(fmt.values()))
+        yuv, fmt, source = check_chunk(frames, "WindowStream", pixel_format, color_matrix, color_range, frame_size)
         if self._source is None:
             self._format = fmt
             self._start(frames, yuv)
             self._source = source
         elif source != self._source:
-            raise ValueError(f"the stream's frames are {self._source}; a chunk of {source} cannot join it")
+            raise ValueError(_mismatch(self._source, source))
         dev = self._ring.device
         if frames.is_cuda and frames.device != dev:
             raise ValueError(f"the stream lives on {dev}, the chunk on {frames.device}")
@@ -242,6 +263,325 @@ class WindowStream:
         out = self._windows_out(1)
         self._gather(out, 0, self.frames_seen - 1)
         return [0], out
+
+
+class StepRound(NamedTuple):
+    """One round of a ``MultiWindowStream`` step (``multi_stream_schedule``).
+
+    - ``pieces``: ``(q, lo, hi, slot)``: frames ``lo .. hi-1`` of queue entry ``q`` are transformed into step slots
+      ``slot ..``; ordered by source group (in order of first appearance), then push order, so each group's frames
+      fill a contiguous run of step slots.
+    - ``groups``: ``(group, p0, p1)``: pieces ``p0 .. p1-1`` belong to ``group``.
+    - ``windows``: ``(v, start)`` of every window the round completes, by video then start.
+    - ``gather``: int32 ``[len(windows) * window]``: the pool slot of each window frame (the table of
+      ``nexar_gather_windows_table``).
+    - ``copy_src`` / ``copy_dst``: int32 step slots and tail slots: each video's last ``min(window - 1, new frames)``
+      frames are copied into its tail, after the gather.
+    - ``done``: videos that end in this round (closed, every frame seen): their tail slots are free after it."""
+    pieces: List[Tuple[int, int, int, int]]
+    groups: List[Tuple[Any, int, int]]
+    windows: List[Tuple[int, int]]
+    gather: np.ndarray
+    copy_src: np.ndarray
+    copy_dst: np.ndarray
+    done: List[int]
+
+
+def multi_stream_schedule(videos: Sequence[Tuple[int, int, bool]], queue: Sequence[Tuple[int, int, Any]], window: int,
+                          stride: int, step_frames: int) -> List[StepRound]:
+    """The work of one ``MultiWindowStream`` step, on the host.  ``videos[v] = (seen, tail, closed)``: frames already
+    transformed, the first of the video's ``window - 1`` tail slots, and whether the video has been closed.
+    ``queue[q] = (v, n, group)``: the chunks pushed since the last step, in push order (``group``: the source group).
+
+    Pool slots ``0 .. step_frames-1`` are the step region.  Video frame ``f`` of an earlier round or step lives in tail
+    slot ``tail + f % (window - 1)``; only its last ``window - 1`` frames are kept, and a window that completes in a round
+    starts at or after ``seen - window + 1``, so each of its frames is either there or new in the round.  The frames are
+    taken in push order, at most ``step_frames`` per round.  A closed video ends in the round that takes its last frame
+    (round 0 when it has none queued); one that saw fewer than ``window`` frames then gets its padded window (its last
+    frame repeated, nexar_videos.py:429-433)."""
+    tail_len = window - 1
+    nv = len(videos)
+    seen = np.array([v[0] for v in videos], np.int64)
+    tail = np.array([v[1] for v in videos], np.int64)
+    left = np.zeros(nv, np.int64)                  # frames still queued per video
+    for v, n, _ in queue:
+        left[v] += n
+    ended = np.zeros(nv, bool)
+    rounds: List[StepRound] = []
+    qi, qoff = 0, 0
+    while True:
+        taken, budget = [], step_frames
+        while qi < len(queue) and budget > 0:
+            v, n, g = queue[qi]
+            take = min(n - qoff, budget)
+            taken.append((qi, qoff, qoff + take))
+            budget -= take
+            qoff += take
+            if qoff == n:
+                qi, qoff = qi + 1, 0
+        order: Dict[Any, int] = {}
+        for q, _, _ in taken:
+            order.setdefault(queue[q][2], len(order))
+        taken.sort(key=lambda p: order[queue[p[0]][2]])          # stable: push order within a group
+        pieces, groups, new_slots = [], [], {}
+        slot = 0
+        for i, (q, lo, hi) in enumerate(taken):
+            g = queue[q][2]
+            if not groups or groups[-1][0] != g:
+                groups.append([g, i, i])
+            groups[-1][2] = i + 1
+            pieces.append((q, lo, hi, slot))
+            new_slots.setdefault(queue[q][0], []).extend(range(slot, slot + hi - lo))
+            slot += hi - lo
+        n_new = np.zeros(nv, np.int64)
+        for v, sl in new_slots.items():
+            n_new[v] = len(sl)
+            left[v] -= len(sl)
+        done = [v for v in range(nv) if videos[v][2] and not ended[v] and left[v] == 0]
+        ended[done] = True
+        # windows, by video then start
+        win_v, win_s = [], []
+        for v in sorted(set(new_slots) | set(done)):
+            k0 = windows_complete(int(seen[v]), window, stride)
+            k1 = windows_complete(int(seen[v] + n_new[v]), window, stride)
+            win_v += [v] * (k1 - k0)
+            win_s += [k * stride for k in range(k0, k1)]
+            if v in done and seen[v] + n_new[v] < window:
+                win_v.append(v)
+                win_s.append(0)
+        gather = np.zeros(0, np.int32)
+        if win_v:
+            wv, ws = np.array(win_v, np.int64), np.array(win_s, np.int64)
+            vids = sorted(new_slots)
+            flat = np.array([s for v in vids for s in new_slots[v]] or [0], np.int64)
+            off = np.zeros(nv, np.int64)
+            pos = 0
+            for v in vids:
+                off[v] = pos
+                pos += len(new_slots[v])
+            f = np.minimum(ws[:, None] + np.arange(window)[None, :], (seen[wv] + n_new[wv] - 1)[:, None])
+            s0 = seen[wv][:, None]
+            is_new = f >= s0
+            from_step = flat[np.clip(off[wv][:, None] + f - s0, 0, flat.size - 1)]
+            from_tail = tail[wv][:, None] + f % max(tail_len, 1)
+            gather = np.where(is_new, from_step, from_tail).astype(np.int32).reshape(-1)
+        copy_src, copy_dst = [], []
+        if tail_len > 0:
+            for v, sl in new_slots.items():
+                if ended[v]:
+                    continue                                     # nothing reads the tail of a video that has ended
+                keep = min(tail_len, len(sl))
+                first = int(seen[v]) + len(sl) - keep
+                copy_src += sl[len(sl) - keep:]
+                copy_dst += [int(tail[v]) + (first + i) % tail_len for i in range(keep)]
+        seen += n_new
+        rounds.append(StepRound(pieces, [tuple(g) for g in groups], list(zip(win_v, win_s)), gather,
+                                np.array(copy_src, np.int32), np.array(copy_dst, np.int32), done))
+        if qi == len(queue):
+            return rounds
+
+
+class _Video:
+    """A video of a ``MultiWindowStream``: its key, record / tail slot, frame counts and source."""
+    __slots__ = ("key", "slot", "seen", "closed", "source", "fsrc")
+
+    def __init__(self, key, slot: int, source: Tuple, fsrc):
+        self.key, self.slot, self.source, self.fsrc = key, slot, source, fsrc
+        self.seen, self.closed = 0, False
+
+
+class MultiWindowStream:
+    """Sliding windows over many videos at once, each arriving in chunks of consecutive frames (one per camera, say),
+    in bounded device memory: every ``step()`` transforms the frames pushed since the last one with one transform call per
+    source group (frames of equal shape, dtype and source format), then builds every window they complete with one
+    gather and updates each video's last frames with one copy, whatever the number of videos.
+
+    ``push(key, chunk, **source_format)`` queues a chunk of video ``key`` (any hashable; the first push opens the video,
+    and draws its parameter record as ``WindowStream`` does); ``close(key)`` ends it.  ``step()`` returns ``(keys, starts,
+    windows)``: ``windows`` is a contiguous ``[K,3,window,cs,cs]`` tensor of every window completed, grouped by video in the
+    order the videos were opened and by start within a video, with each window's key and start frame.  For every video,
+    the windows it gets across all steps equal ``WindowStream(window, stride, transform, out_dtype)`` fed the same chunks,
+    bit for bit, under that class's conditions (a pixel above 1 in the video, no gaussian noise), for any interleaving of
+    pushes, steps and closes.  A video shorter than ``window`` gets its padded window at the step after its ``close``; a
+    push after ``close`` opens a new video under the same key.
+
+    Chunks are what ``WindowStream.push`` takes, on the device (read in place) or the host (copied with a non-blocking
+    copy; do not overwrite a pinned chunk before the step's work has run).  Videos may differ in resolution and format.
+    Device memory is one pool of ``max_frames_per_step`` step slots plus ``window - 1`` slots per open video, and a
+    host-staging buffer of at most ``max_frames_per_step`` frames per source group; a step with more queued frames than
+    ``max_frames_per_step`` runs in rounds, in push order.  It never depends on how long a video runs, and it is released
+    when every video has been closed and stepped.  All videos live on one device (the first chunk's, or the current one
+    for a host chunk); everything is enqueued on its current CUDA stream."""
+
+    def __init__(self, window: int = 16, stride: int = 8, transform: Optional[GpuVideoTransform] = None,
+                 out_dtype: torch.dtype = torch.bfloat16, max_frames_per_step: int = 1024):
+        if window < 1 or stride < 1 or max_frames_per_step < 1:
+            raise ValueError(f"window, stride and max_frames_per_step must be >= 1, got {window}, {stride}, "
+                             f"{max_frames_per_step}")
+        self.window, self.stride, self.max_frames_per_step = int(window), int(stride), int(max_frames_per_step)
+        self.tf = transform or create_video_transforms(mode="val", out_dtype=out_dtype)
+        self.out_dtype = out_dtype
+        self.device: Optional[torch.device] = None
+        self._videos: Dict[int, _Video] = {}      # every video not yet ended, in the order they were opened
+        self._open: Dict[Any, _Video] = {}        # key -> the video that takes its pushes
+        self._queue: List[Tuple[_Video, torch.Tensor]] = []
+        self._next_id = 0
+        self._free: List[int] = []                # record / tail slots of ended videos
+        self._n_slots = 0
+        self._records: Optional[np.ndarray] = None      # packed NexarClipParams, one per record slot
+        self._pool: Optional[torch.Tensor] = None       # [max_frames_per_step + n_slots * (window - 1), 3, cs, cs]
+        self._staging: Dict[Tuple, torch.Tensor] = {}
+
+    def _tail(self, slot: int) -> int:
+        return self.max_frames_per_step + slot * (self.window - 1)
+
+    def _take_slot(self, dev: torch.device) -> int:
+        if not self._free:                  # grow the pool and the records by doubling; the tails move with the copy
+            n = max(4, 2 * self._n_slots)
+            cs = self.tf.crop_size
+            pool = torch.empty((self._tail(n), 3, cs, cs), dtype=self.out_dtype, device=dev)
+            records = np.zeros(n, _lib.CLIP_PARAMS_DTYPE)
+            if self._pool is not None:
+                pool[:self._pool.shape[0]].copy_(self._pool)
+                records[:self._n_slots] = self._records
+            self._pool, self._records = pool, records
+            self._free = list(range(n - 1, self._n_slots - 1, -1))
+            self._n_slots = n
+        return self._free.pop()
+
+    @torch.no_grad()
+    def push(self, key, frames: torch.Tensor, pixel_format: str = "rgb", color_matrix: str = "bt601",
+             color_range: str = "limited", frame_size=None) -> None:
+        """Queues a chunk of ``n >= 1`` consecutive frames of video ``key`` for the next ``step()``."""
+        yuv, fmt, source = check_chunk(frames, "MultiWindowStream", pixel_format, color_matrix, color_range, frame_size)
+        video = self._open.get(key)
+        if video is not None and source != video.source:
+            raise ValueError(_mismatch(video.source, source))
+        fsrc = frame_source(source[0], frames.dtype, **fmt) if video is None else None   # refuses what forward_batch would
+        dev = self.device if self.device is not None else (
+            frames.device if frames.is_cuda else torch.device("cuda", torch.cuda.current_device()))
+        if frames.is_cuda and frames.device != dev:
+            raise ValueError(f"the streams live on {dev}, the chunk on {frames.device}")
+        if video is None:
+            rec = _draw_record(self.tf, frames, fmt, yuv)
+            packed, _ = pack_clip_params([rec], self.tf.crop_size, self.tf.video_aug)
+            _lib.table_lib()          # a library without the table gather fails here, before any work
+            self.device = dev
+            video = _Video(key, self._take_slot(dev), source, fsrc)
+            self._records[video.slot] = packed[0]
+            self._videos[self._next_id] = self._open[key] = video
+            self._next_id += 1
+        self._queue.append((video, frames.contiguous() if frames.is_cuda else frames))
+
+    def close(self, key) -> None:
+        """Ends video ``key``: its last windows (the padded one of a video shorter than ``window``) come out of the next
+        ``step()``, and its slots are freed there."""
+        video = self._open.pop(key, None)
+        if video is None:
+            raise ValueError(f"no open video under key {key!r}")
+        video.closed = True
+
+    def _windows_out(self, k: int) -> torch.Tensor:
+        cs = self.tf.crop_size
+        dev = self.device if self.device is not None else torch.device("cuda", torch.cuda.current_device())
+        return torch.empty((k, 3, self.window, cs, cs), dtype=self.out_dtype, device=dev)
+
+    def _staging_for(self, group, shape: Tuple[int, ...], dtype: torch.dtype, n: int) -> torch.Tensor:
+        buf = self._staging.get(group)
+        if buf is None or buf.shape[0] < n:
+            rows = min(self.max_frames_per_step, max(n, 2 * buf.shape[0] if buf is not None else n))
+            buf = self._staging[group] = torch.empty((rows,) + shape, dtype=dtype, device=self.device)
+        return buf
+
+    def _gather(self, table: torch.Tensor, n: int, dst: Optional[torch.Tensor], dst_slots: Optional[torch.Tensor]):
+        pool = self._pool
+        _lib.check(_lib.table_lib().nexar_gather_windows_table(
+            pool.data_ptr(), pool.shape[0], pool[0, 0].numel() * pool.element_size(), 1 if dst is None else self.window,
+            table.data_ptr(), n, None if dst is None else dst.data_ptr(), None if dst_slots is None else dst_slots.data_ptr(),
+            torch.cuda.current_stream(pool.device).cuda_stream))
+
+    def _round(self, eng, rnd: StepRound, videos: List[_Video]) -> Optional[torch.Tensor]:
+        """Enqueues one round: a transform call per source group into the step slots, the window gather, the tail copy."""
+        calls, offsets = [], []
+        for _, p0, p1 in rnd.groups:
+            pieces = rnd.pieces[p0:p1]
+            first = self._queue[pieces[0][0]]
+            fs, n = first[0].fsrc, sum(hi - lo for _, lo, hi, _ in pieces)
+            n_host = sum(hi - lo for q, lo, hi, _ in pieces if not self._queue[q][1].is_cuda)
+            staging = self._staging_for(first[0].source, first[0].source[0], first[1].dtype, n_host) if n_host else None
+            srcs, addr, rec, at = [], [], [], 0
+            for q, lo, hi, _ in pieces:
+                video, chunk = self._queue[q]
+                part = chunk[lo:hi]
+                if not chunk.is_cuda:        # host frames: one non-blocking copy per chunk into the group's staging
+                    part = staging[at:at + hi - lo]
+                    part.copy_(chunk[lo:hi], non_blocking=True)
+                    at += hi - lo
+                srcs.append(part)
+                addr.append(part.data_ptr() + fs.frame_bytes * np.arange(hi - lo, dtype=np.int64))
+                rec.append(np.full(hi - lo, video.slot, np.int64))
+            base = min(srcs, key=lambda t: t.data_ptr())       # offsets from the lowest frame address: all >= 0
+            offsets.append(np.concatenate(addr) - base.data_ptr())
+            params = self._records[np.concatenate(rec)]          # one vectorised index into the packed records
+            calls.append((base, fs, pieces[0][3], n, params))
+        # frame offsets and both slot tables: one upload through the engine's pinned staging
+        parts = offsets + [rnd.gather, rnd.copy_src, rnd.copy_dst]
+        raw = eng.upload_params(np.concatenate([np.ascontiguousarray(x).view(np.uint8) for x in parts])) \
+            if any(x.size for x in parts) else None
+        views, at = [], 0
+        for x in parts:
+            views.append(raw[at:at + x.nbytes].view(torch.int64 if x.dtype == np.int64 else torch.int32) if x.size else None)
+            at += x.nbytes
+        for (base, fs, slot, n, params), offs in zip(calls, views):
+            any_flags = int(np.bitwise_or.reduce(params["flags"]))
+            self.tf._transform_packed(eng, base, offs, n, 1, params, any_flags, fs, self._pool[slot:slot + n].unsqueeze(1),
+                                      "BTCHW", self.out_dtype)
+        gather, copy_src, copy_dst = views[len(calls):]
+        out = None
+        if rnd.windows:
+            out = self._windows_out(len(rnd.windows))
+            self._gather(gather, len(rnd.windows), out, None)
+        if copy_src is not None:             # after the gather, which may read the tail slots this overwrites
+            self._gather(copy_src, rnd.copy_src.size, None, copy_dst)
+        return out
+
+    @torch.no_grad()
+    def step(self) -> Tuple[List[Any], List[int], torch.Tensor]:
+        """Transforms every queued frame -> (keys, starts, ``[K,3,window,cs,cs]``) of the windows completed, grouped by
+        video in the order the videos were opened, by start within a video.  A step with nothing queued and no video
+        closed launches nothing."""
+        if not self._queue and not any(v.closed for v in self._videos.values()):
+            return [], [], self._windows_out(0)
+        ids = list(self._videos)
+        videos = [self._videos[i] for i in ids]
+        pos = {id(v): i for i, v in enumerate(videos)}
+        rounds = multi_stream_schedule([(v.seen, self._tail(v.slot), v.closed) for v in videos],
+                                       [(pos[id(v)], c.shape[0], v.source) for v, c in self._queue],
+                                       self.window, self.stride, self.max_frames_per_step)
+        eng = get_engine(self.device)
+        outs, order = [], []
+        with torch.cuda.device(self.device):
+            for rnd in rounds:
+                out = self._round(eng, rnd, videos)
+                if out is not None:
+                    outs.append(out)
+                    order += rnd.windows
+                for q, lo, hi, _ in rnd.pieces:
+                    self._queue[q][0].seen += hi - lo
+                for v in rnd.done:
+                    self._free.append(videos[v].slot)
+                    del self._videos[ids[v]]
+        self._queue = []
+        if not self._videos:                 # every video has ended: give the pool and the staging buffers back
+            self._pool, self._records, self._free, self._n_slots, self._staging = None, None, [], 0, {}
+        if not outs:
+            return [], [], self._windows_out(0)
+        windows = outs[0]
+        if len(outs) > 1:                    # rounds: put each video's windows together again
+            perm = sorted(range(len(order)), key=lambda i: order[i])
+            windows = torch.cat(outs)[torch.tensor(perm, dtype=torch.int64)]
+            order = [order[i] for i in perm]
+        return [videos[v].key for v, _ in order], [s for _, s in order], windows
 
 
 CLASS_MAP = {0: "Normal", 1: "Near Collision", 2: "Collision"}      # nexar_inference.py:239
@@ -316,6 +656,20 @@ class WindowPredictor:
                     parts, part_starts = [], []
         if part_starts:
             yield from self._classify(parts[0] if len(parts) == 1 else torch.cat(parts), part_starts, video_path, fps)
+
+    @torch.no_grad()
+    def predict_step(self, keys: Sequence[Any], starts: Sequence[int], windows: torch.Tensor,
+                     fps: float = 30.0) -> List[Dict[str, Any]]:
+        """Classifies the windows of one ``MultiWindowStream.step()`` (made with this predictor's window) in batches of
+        ``batch_size``: one dictionary per window, in the step's order, as ``predict`` returns them with the window's
+        stream key as ``video_path``."""
+        results: List[Dict[str, Any]] = []
+        for lo in range(0, len(keys), self.batch_size):
+            batch = self._classify(windows[lo:lo + self.batch_size], list(starts[lo:lo + self.batch_size]), "", fps)
+            for r, key in zip(batch, keys[lo:lo + self.batch_size]):
+                r["video_path"] = key
+            results.extend(batch)
+        return results
 
     def _classify(self, batch: torch.Tensor, starts: List[int], video_path: str, fps: float) -> List[Dict[str, Any]]:
         """One model call on a contiguous ``[b,3,T,cs,cs]`` batch -> one result dictionary per window."""

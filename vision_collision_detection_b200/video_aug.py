@@ -24,7 +24,7 @@ fp32 or bf16, optional frame gather) — the call the loaders and bench use.
 from __future__ import annotations
 
 import random
-from typing import Any, Dict, List, Optional, Sequence, Tuple
+from typing import Any, Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -58,6 +58,42 @@ def check_pixel_format(pixel_format: str, color_matrix: str = "bt601", color_ran
 def source_dtype(pixel_format: str) -> torch.dtype:
     """The element type of a frame tensor of ``pixel_format``: uint16 for the 16-bit surfaces, uint8 otherwise."""
     return torch.uint16 if pixel_format in _SAMPLE_SHIFT else torch.uint8
+
+
+class FrameSource(NamedTuple):
+    """How the kernels read one source frame: the visible ``h x w``, the bytes of a frame, the plan's source key (a torch
+    dtype for RGB, ``"nv12"`` or a YUV format tuple of ``Plan``) and the row pitch in bytes of YUV surfaces (None: packed
+    RGB rows)."""
+    h: int
+    w: int
+    frame_bytes: int
+    plan_src: Any
+    row_stride: Optional[int]
+    pixel_format: str
+
+
+def frame_source(frame_shape: Tuple[int, ...], dtype: torch.dtype, pixel_format: str = "rgb", color_matrix: str = "bt601",
+                 color_range: str = "limited", frame_size: Optional[Tuple[int, int]] = None) -> FrameSource:
+    """The ``FrameSource`` of frames ``[H,W,3]`` (RGB) or surfaces ``[R,P]`` (YUV) with the source-format keywords of
+    ``forward_batch``, which has checked them."""
+    if pixel_format == "rgb":
+        if frame_size is not None:
+            raise ValueError("frame_size describes the visible picture of YUV surfaces; RGB frames have no padding")
+        h, w = frame_shape[0], frame_shape[1]
+        return FrameSource(h, w, h * w * 3 * dtype.itemsize, dtype, None, pixel_format)
+    rows, pitch = frame_shape
+    if rows % 3 or pitch % 2:
+        raise ValueError(f"{pixel_format} surfaces are [H*3/2,W] with even H and W, got {tuple(frame_shape)}")
+    luma_rows = rows * 2 // 3
+    h, w = (luma_rows, pitch) if frame_size is None else (int(frame_size[0]), int(frame_size[1]))
+    if h <= 0 or w <= 0 or h % 2 or w % 2 or h > luma_rows or w > pitch:
+        raise ValueError(f"frame_size {(h, w)} must be even and fit the {luma_rows} luma rows x {pitch} pitch surface")
+    fmt = (_YUV_LAYOUT[pixel_format], _YUV_MATRIX[color_matrix], _YUV_RANGE[color_range], luma_rows)
+    if pixel_format in _SAMPLE_SHIFT:
+        src = fmt + (_SAMPLE_SHIFT[pixel_format],)
+    else:   # the format of the original NEXAR_SRC_NV12 plans keeps going through nexar_plan_create
+        src = "nv12" if fmt == (_lib.YUV_NV12, _lib.YUV_BT601, _lib.YUV_LIMITED, h) else fmt
+    return FrameSource(h, w, rows * pitch * dtype.itemsize, src, pitch * dtype.itemsize, pixel_format)
 
 
 class _Stage:
@@ -183,13 +219,12 @@ class GpuVideoTransform(nn.Module):
             raise RuntimeError("two-pass variant: handled by _forward_two_pass")
         return eng.resize_crop_plan(h, w, self.resize_short_side, cs, src_dtype)
 
-    def _forward_two_pass(self, eng, frames, offsets, n_clips, t_out, packed, any_flags, out, strides):
+    def _forward_two_pass(self, eng, frames, h, w, offsets, n_clips, t_out, packed, any_flags, out, strides):
         """The never-called factory's default forward (nexar_video_aug.py:407-463): an antialiased short-side
         resize followed by a SECOND antialiased resize inside crop_tensor(use_letterbox=True).  Pass 1 writes
         the [0,1] float frames of size (rh, rw) on a square scratch canvas; pass 2 letterboxes those float
         frames (strided rows) and applies flip / augmentation / normalisation.  A record's byte-range flag describes the
         source frames, so it goes to pass 1 only: pass 2 reads values that are already in [0,1]."""
-        h, w = frames.shape[2], frames.shape[3]
         rh, rw = self._resized_hw(h, w)
         cm = max(rh, rw)
         plan1 = eng.plan(_lib.Geometry(h, w, cm, rh, rw, 0, 0), _SRC[frames.dtype])
@@ -246,21 +281,9 @@ class GpuVideoTransform(nn.Module):
             raise ValueError("uint16 frames are 16-bit YUV surfaces: pass pixel_format='p010' or 'i010'")
         if frame_size is not None and not yuv:
             raise ValueError("frame_size describes the visible picture of YUV surfaces; RGB frames have no padding")
-        if yuv:
-            b, t, rows, pitch = frames.shape
-            luma_rows = rows * 2 // 3
-            h, w = (luma_rows, pitch) if frame_size is None else (int(frame_size[0]), int(frame_size[1]))
-            if h <= 0 or w <= 0 or h % 2 or w % 2 or h > luma_rows or w > pitch:
-                raise ValueError(f"frame_size {(h, w)} must be even and fit the {luma_rows} luma rows x {pitch} pitch surface")
-            frame_bytes = rows * pitch * frames.element_size()
-            fmt = (_YUV_LAYOUT[pixel_format], _YUV_MATRIX[color_matrix], _YUV_RANGE[color_range], luma_rows)
-            if pixel_format in _SAMPLE_SHIFT:
-                src = fmt + (_SAMPLE_SHIFT[pixel_format],)
-            else:   # the format of the original NEXAR_SRC_NV12 plans keeps going through nexar_plan_create
-                src = "nv12" if fmt == (_lib.YUV_NV12, _lib.YUV_BT601, _lib.YUV_LIMITED, h) else fmt
-        else:
-            b, t, h, w, _ = frames.shape
-            frame_bytes = h * w * 3 * frames.element_size()
+        b, t = frames.shape[:2]
+        source = frame_source(tuple(frames.shape[2:]), frames.dtype, pixel_format, color_matrix, color_range, frame_size)
+        h, w, frame_bytes = source.h, source.w, source.frame_bytes
         if not frames.is_cuda:
             raise ValueError("forward_batch needs device-resident frames (use forward() for host tensors)")
         if not yuv and frames.dtype not in _SRC:
@@ -290,23 +313,32 @@ class GpuVideoTransform(nn.Module):
             raise ValueError("one parameter record per clip is required")
         self.last_params = params
         packed, any_flags = pack_clip_params(params, self.crop_size, self.video_aug)
+        return self._transform_packed(eng, frames, offsets, n_clips, t_out, packed, any_flags, source, out, layout,
+                                      out_dtype or self.out_dtype)
+
+    def _transform_packed(self, eng, frames: torch.Tensor, offsets: torch.Tensor, n_clips: int, t_out: int,
+                          packed: np.ndarray, any_flags: int, source: FrameSource, out: Optional[torch.Tensor],
+                          layout: str, out_dtype: torch.dtype) -> torch.Tensor:
+        """The library call behind ``forward_batch``: ``n_clips`` clips of ``t_out`` frames read at the byte
+        ``offsets`` (int64, on the device) from ``frames.data_ptr()``, with the packed parameter records ``packed`` (one
+        per clip, ``pack_clip_params``).  ``frames`` only gives the base address, device and element type, so the
+        frames may lie anywhere above it (``MultiWindowStream`` gathers frames of many tensors in one call)."""
         two_pass = self.resize_short_side is not None and self.use_letterbox
-        if yuv and two_pass:
-            raise ValueError(f"{pixel_format} frames are not supported by the two-pass (short-side resize + letterbox) variant")
-        plan = None if two_pass else self._plan(eng, h, w, src if yuv else frames.dtype)
-        dt = out_dtype or self.out_dtype
+        if source.pixel_format != "rgb" and two_pass:
+            raise ValueError(f"{source.pixel_format} frames are not supported by the two-pass (short-side resize + letterbox) variant")
+        plan = None if two_pass else self._plan(eng, source.h, source.w, source.plan_src)
         if out is None:
-            out, strides = _alloc_out(layout, n_clips, t_out, self.crop_size, dt, frames.device)
+            out, strides = _alloc_out(layout, n_clips, t_out, self.crop_size, out_dtype, frames.device)
         else:
             probe, strides = _alloc_out(layout, n_clips, t_out, self.crop_size, out.dtype, "meta")
             if tuple(out.shape) != tuple(probe.shape) or not out.is_contiguous():
                 raise ValueError(f"out must be a contiguous {tuple(probe.shape)} tensor for layout {layout}")
         if two_pass:
-            return self._forward_two_pass(eng, frames, offsets, n_clips, t_out, packed, any_flags, out, strides)
+            return self._forward_two_pass(eng, frames, source.h, source.w, offsets, n_clips, t_out, packed, any_flags, out,
+                                          strides)
         pdev = eng.upload_params(packed)
         eng.run(plan, frames, offsets, n_clips, t_out, pdev, any_flags, out, strides,
-                self.normalize, self.video_mean, self.video_std,
-                src_row_stride=pitch * frames.element_size() if yuv else None)
+                self.normalize, self.video_mean, self.video_std, src_row_stride=source.row_stride)
         return out
 
     @torch.no_grad()
