@@ -392,3 +392,19 @@ def test_stream_errors_on_the_device():
     short.push(video[:3])
     starts, win = short.finish()
     assert starts == [0] and _same_bits(win, _offline(tf, video[:3]))
+
+
+@gpu
+def test_stream_refused_first_chunk_leaves_it_unopened():
+    """A first chunk the stream refuses (13 rows are no 4:2:0 surface) opens nothing: a correct video pushed next gets the
+    offline windows."""
+    from vision_collision_detection_b200 import create_video_transforms
+    from vision_collision_detection_b200.inference import WindowStream
+    video = _video(40)
+    tf = create_video_transforms(mode="val", crop_size=56)
+    ws = WindowStream(16, 8, tf)
+    with pytest.raises(ValueError):
+        ws.push(torch.zeros((3, 13, 8), dtype=torch.uint8, device="cuda"), pixel_format="nv12")
+    starts, got = _run_stream(ws, video, [7, 33])
+    assert starts == sliding_window_starts(40, 16, 8)
+    assert _same_bits(got, _offline(tf, video))

@@ -12,7 +12,8 @@ from typing import Any, Dict, List, Optional
 import torch
 
 from .engine import ClipTransformEngine
-from .video_aug import GpuVideoTransform, check_pixel_format, source_dtype
+from .source_format import SourceFormat
+from .video_aug import GpuVideoTransform
 
 
 def bind_to_gpu_numa_node(device_index: int) -> Optional[List[int]]:
@@ -54,11 +55,11 @@ class HostClipPipeline:
         surfaces, uint16 ``[B,T,H*3/2,W]`` — as many bytes as RGB over PCIe."""
         self.tf = transform
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-        yuv = check_pixel_format(pixel_format, color_matrix, color_range)
-        self.pixel_format = pixel_format
-        self.yuv_kw = dict(pixel_format=pixel_format, color_matrix=color_matrix, color_range=color_range)
-        self.shape = (n_clips, frames, height * 3 // 2, width) if yuv else (n_clips, frames, height, width, 3)
-        self.dtype = source_dtype(pixel_format)
+        fmt = SourceFormat.of(pixel_format, color_matrix, color_range)
+        self.yuv_kw = fmt._asdict()
+        self.height, self.width = height, width
+        self.shape = (n_clips, frames) + fmt.frame_shape(height, width)
+        self.dtype = fmt.dtype
         self.chunk = max(1, min(clips_per_chunk, n_clips))
         self.out_dtype = out_dtype or transform.out_dtype
         cs = transform.crop_size
@@ -85,8 +86,7 @@ class HostClipPipeline:
             raise ValueError(f"expected {self.dtype} {self.shape}")
         n = self.shape[0]
         if params is None:
-            h = self.shape[2] * 2 // 3 if self.pixel_format != "rgb" else self.shape[2]
-            params = self.tf.sample_params(n, h, self.shape[3])
+            params = self.tf.sample_params(n, self.height, self.width)
         slot = self._slot
         self._slot ^= 1
         host_out = self.host_outs[slot]

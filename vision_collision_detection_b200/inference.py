@@ -28,7 +28,8 @@ import torch
 from . import _lib
 from .engine import get_engine
 from .params import pack_clip_params
-from .video_aug import GpuVideoTransform, check_pixel_format, create_video_transforms, frame_source, source_dtype
+from .source_format import FrameSource, SourceFormat
+from .video_aug import GpuVideoTransform, create_video_transforms
 from .videos import select_start_frame, window_indices
 
 
@@ -63,14 +64,9 @@ class SlidingWindowTransform:
         """[N,H,W,3] uint8 on the device -> [N,3,cs,cs]: every frame transformed once.  YUV surfaces [N,R,P] with
         ``pixel_format="nv12"`` / ``"i420"`` (uint16 with ``"p010"`` / ``"i010"``) and the other source-format keywords
         of forward_batch."""
-        if check_pixel_format(pixel_format, color_matrix, color_range):
-            if video_u8.dim() != 3:
-                raise ValueError(f"expected [N,R,P] {pixel_format} surfaces, got {tuple(video_u8.shape)}")
-        elif video_u8.dim() != 4 or video_u8.shape[-1] != 3:
-            raise ValueError(f"expected [N,H,W,3], got {tuple(video_u8.shape)}")
-        n = video_u8.shape[0]
         out = self.tf.forward_batch(video_u8.unsqueeze(0), layout="BTCHW", out_dtype=self.out_dtype, pixel_format=pixel_format,
                                     color_matrix=color_matrix, color_range=color_range, frame_size=frame_size)  # [1,N,3,cs,cs]
+        n = out.shape[1]
         if n < self.window:       # pad by repeating the last frame
             out = torch.cat([out, out[:, -1:].expand(1, self.window - n, *out.shape[2:])], dim=1)
         return out[0]
@@ -122,42 +118,25 @@ def ring_schedule(seen: int, n: int, window: int, stride: int, max_chunk: int) -
     return groups
 
 
-def check_chunk(frames: torch.Tensor, who: str, pixel_format: str = "rgb", color_matrix: str = "bt601",
-                color_range: str = "limited", frame_size=None) -> Tuple[bool, Dict[str, Any], Tuple]:
-    """Validates a chunk of ``n >= 1`` decoded frames and its source-format keywords -> (YUV?, the keywords as a dict,
-    the source key ``(frame shape, dtype, format)`` that every later chunk of the same video must match)."""
-    yuv = check_pixel_format(pixel_format, color_matrix, color_range)
-    if frames.dtype.is_floating_point:
-        raise TypeError(f"{who} takes decoded uint8 frames or YUV surfaces, got {frames.dtype}")
-    if yuv and frames.dim() != 3:
-        raise ValueError(f"expected a chunk of [n,R,P] {pixel_format} surfaces, got {tuple(frames.shape)}")
-    if not yuv and (frames.dim() != 4 or frames.shape[-1] != 3):
-        raise ValueError(f"expected a chunk of [n,H,W,3] frames, got {tuple(frames.shape)}")
+def check_chunk(frames: torch.Tensor, pixel_format: str = "rgb", color_matrix: str = "bt601", color_range: str = "limited",
+                frame_size=None) -> FrameSource:
+    """Validates a chunk ``[n,*frame]`` of ``n >= 1`` decoded frames and its source-format keywords -> the source that
+    every later chunk of the same video must equal."""
+    source = SourceFormat.of(pixel_format, color_matrix, color_range).describe(frames.shape[1:], frames.dtype, frame_size,
+                                                                              decoded=True)
     if frames.shape[0] < 1:
         raise ValueError("empty chunk")
-    fmt = dict(pixel_format=pixel_format, color_matrix=color_matrix, color_range=color_range,
-               frame_size=None if frame_size is None else (int(frame_size[0]), int(frame_size[1])))
-    return yuv, fmt, (tuple(frames.shape[1:]), frames.dtype, tuple(fmt.values()))
+    return source
 
 
 def _mismatch(have, source) -> str:
     return f"the stream's frames are {have}; a chunk of {source} cannot join it"
 
 
-def _draw_record(tf: GpuVideoTransform, frames: torch.Tensor, fmt: Dict[str, Any], yuv: bool) -> Dict[str, Any]:
-    """The parameter record of a video whose first chunk is ``frames``: ``tf.sample_params(1, h, w)`` for the visible
-    ``h x w``, as ``SlidingWindowTransform.frames()`` draws it for the whole video, with the byte-range flag (every chunk
-    is scaled by 1/255, ``NEXAR_RANGE_255``)."""
-    if frames.dtype != source_dtype(fmt["pixel_format"]):
-        raise ValueError(f"{fmt['pixel_format']} frames are {source_dtype(fmt['pixel_format'])}, got {frames.dtype}")
-    if yuv:
-        size = fmt["frame_size"]
-        h, w = (frames.shape[1] * 2 // 3, frames.shape[2]) if size is None else size
-    else:
-        h, w = frames.shape[1], frames.shape[2]
-    rec = dict(tf.sample_params(1, h, w)[0])
-    rec["range_255"] = True
-    return rec
+def _draw_record(tf: GpuVideoTransform, source: FrameSource) -> Dict[str, Any]:
+    """The parameter record of a video of frames ``source``, drawn for its visible ``h x w`` as ``frames()`` draws it
+    for a whole video, with the byte-range flag (every chunk is scaled by 1/255, ``NEXAR_RANGE_255``)."""
+    return dict(tf.sample_params(1, source.h, source.w)[0], range_255=True)
 
 
 class WindowStream:
@@ -191,14 +170,14 @@ class WindowStream:
         self.out_dtype = out_dtype
         self.frames_seen = 0
         self._finished = False
-        self._source = None       # (frame shape, dtype, source format) of the first chunk: every chunk must match it
-        self._format: Dict[str, Any] = {}
+        self._source: Optional[FrameSource] = None      # the first chunk's: every chunk must equal it
+        self._format: Dict[str, Any] = {}                # its forward_batch keywords
         self._params = None
         self._ring: Optional[torch.Tensor] = None
         self._staging: Optional[torch.Tensor] = None
 
-    def _start(self, frames: torch.Tensor, yuv: bool):
-        self._params = [_draw_record(self.tf, frames, self._format, yuv)]
+    def _start(self, frames: torch.Tensor, source: FrameSource):
+        self._params = [_draw_record(self.tf, source)]
         dev = frames.device if frames.is_cuda else torch.device("cuda", torch.cuda.current_device())
         _lib.ring_lib()           # a library without the ring gather fails here, before any work
         cs = self.tf.crop_size
@@ -221,10 +200,10 @@ class WindowStream:
         """A chunk of ``n >= 1`` consecutive frames -> (start frames, ``[k,3,window,cs,cs]``) of the windows it completes."""
         if self._finished:
             raise ValueError("push() after finish(): start a new WindowStream for the next video")
-        yuv, fmt, source = check_chunk(frames, "WindowStream", pixel_format, color_matrix, color_range, frame_size)
+        source = check_chunk(frames, pixel_format, color_matrix, color_range, frame_size)
         if self._source is None:
-            self._format = fmt
-            self._start(frames, yuv)
+            self._start(frames, source)
+            self._format = dict(source.format._asdict(), frame_size=source.frame_size)
             self._source = source
         elif source != self._source:
             raise ValueError(_mismatch(self._source, source))
@@ -383,10 +362,10 @@ def multi_stream_schedule(videos: Sequence[Tuple[int, int, bool]], queue: Sequen
 
 class _Video:
     """A video of a ``MultiWindowStream``: its key, record / tail slot, frame counts and source."""
-    __slots__ = ("key", "slot", "seen", "closed", "source", "fsrc")
+    __slots__ = ("key", "slot", "seen", "closed", "source")
 
-    def __init__(self, key, slot: int, source: Tuple, fsrc):
-        self.key, self.slot, self.source, self.fsrc = key, slot, source, fsrc
+    def __init__(self, key, slot: int, source: FrameSource):
+        self.key, self.slot, self.source = key, slot, source
         self.seen, self.closed = 0, False
 
 
@@ -430,7 +409,7 @@ class MultiWindowStream:
         self._n_slots = 0
         self._records: Optional[np.ndarray] = None      # packed NexarClipParams, one per record slot
         self._pool: Optional[torch.Tensor] = None       # [max_frames_per_step + n_slots * (window - 1), 3, cs, cs]
-        self._staging: Dict[Tuple, torch.Tensor] = {}
+        self._staging: Dict[FrameSource, torch.Tensor] = {}
 
     def _tail(self, slot: int) -> int:
         return self.max_frames_per_step + slot * (self.window - 1)
@@ -453,21 +432,20 @@ class MultiWindowStream:
     def push(self, key, frames: torch.Tensor, pixel_format: str = "rgb", color_matrix: str = "bt601",
              color_range: str = "limited", frame_size=None) -> None:
         """Queues a chunk of ``n >= 1`` consecutive frames of video ``key`` for the next ``step()``."""
-        yuv, fmt, source = check_chunk(frames, "MultiWindowStream", pixel_format, color_matrix, color_range, frame_size)
+        source = check_chunk(frames, pixel_format, color_matrix, color_range, frame_size)
         video = self._open.get(key)
         if video is not None and source != video.source:
             raise ValueError(_mismatch(video.source, source))
-        fsrc = frame_source(source[0], frames.dtype, **fmt) if video is None else None   # refuses what forward_batch would
         dev = self.device if self.device is not None else (
             frames.device if frames.is_cuda else torch.device("cuda", torch.cuda.current_device()))
         if frames.is_cuda and frames.device != dev:
             raise ValueError(f"the streams live on {dev}, the chunk on {frames.device}")
         if video is None:
-            rec = _draw_record(self.tf, frames, fmt, yuv)
+            rec = _draw_record(self.tf, source)
             packed, _ = pack_clip_params([rec], self.tf.crop_size, self.tf.video_aug)
             _lib.table_lib()          # a library without the table gather fails here, before any work
             self.device = dev
-            video = _Video(key, self._take_slot(dev), source, fsrc)
+            video = _Video(key, self._take_slot(dev), source)
             self._records[video.slot] = packed[0]
             self._videos[self._next_id] = self._open[key] = video
             self._next_id += 1
@@ -486,11 +464,11 @@ class MultiWindowStream:
         dev = self.device if self.device is not None else torch.device("cuda", torch.cuda.current_device())
         return torch.empty((k, 3, self.window, cs, cs), dtype=self.out_dtype, device=dev)
 
-    def _staging_for(self, group, shape: Tuple[int, ...], dtype: torch.dtype, n: int) -> torch.Tensor:
-        buf = self._staging.get(group)
+    def _staging_for(self, source: FrameSource, n: int) -> torch.Tensor:
+        buf = self._staging.get(source)
         if buf is None or buf.shape[0] < n:
             rows = min(self.max_frames_per_step, max(n, 2 * buf.shape[0] if buf is not None else n))
-            buf = self._staging[group] = torch.empty((rows,) + shape, dtype=dtype, device=self.device)
+            buf = self._staging[source] = torch.empty((rows,) + source.shape, dtype=source.dtype, device=self.device)
         return buf
 
     def _gather(self, table: torch.Tensor, n: int, dst: Optional[torch.Tensor], dst_slots: Optional[torch.Tensor]):
@@ -506,9 +484,9 @@ class MultiWindowStream:
         for _, p0, p1 in rnd.groups:
             pieces = rnd.pieces[p0:p1]
             first = self._queue[pieces[0][0]]
-            fs, n = first[0].fsrc, sum(hi - lo for _, lo, hi, _ in pieces)
+            fs, n = first[0].source, sum(hi - lo for _, lo, hi, _ in pieces)
             n_host = sum(hi - lo for q, lo, hi, _ in pieces if not self._queue[q][1].is_cuda)
-            staging = self._staging_for(first[0].source, first[0].source[0], first[1].dtype, n_host) if n_host else None
+            staging = self._staging_for(fs, n_host) if n_host else None
             srcs, addr, rec, at = [], [], [], 0
             for q, lo, hi, _ in pieces:
                 video, chunk = self._queue[q]

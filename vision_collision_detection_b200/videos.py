@@ -29,7 +29,8 @@ import torch
 from torch.utils.data import Dataset, default_collate
 
 from .sensors import find_sensor_path, load_and_sync_sensor, window_sensor
-from .video_aug import GpuVideoTransform, check_pixel_format, source_dtype
+from .source_format import SourceFormat
+from .video_aug import GpuVideoTransform
 
 
 # ---------------------------------------------------------------------------------
@@ -119,38 +120,28 @@ def _to_uint8_array(frames) -> np.ndarray:
     return np.asarray(frames)
 
 
-def _source_format(defer: bool, pixel_format: str, color_matrix: str, color_range: str) -> Optional[Dict[str, str]]:
-    """The forward_batch keywords of a dataset whose decoder delivers YUV 4:2:0 surfaces (None for RGB frames)."""
-    if not check_pixel_format(pixel_format, color_matrix, color_range):
-        return None
-    if not defer:
+def _source_format(defer: bool, pixel_format: str, color_matrix: str, color_range: str) -> SourceFormat:
+    """The source format of a dataset's decoded frames: YUV 4:2:0 surfaces are converted on the device by GpuAugLoader."""
+    fmt = SourceFormat.of(pixel_format, color_matrix, color_range)
+    if fmt.yuv and not defer:
         raise ValueError(f"pixel_format={pixel_format!r} needs defer=True: the surfaces are converted on the device by "
                          "GpuAugLoader")
-    return {"pixel_format": pixel_format, "color_matrix": color_matrix, "color_range": color_range}
+    return fmt
 
 
 def _blank_frame(shape, fmt: Optional[Dict[str, str]]) -> np.ndarray:
-    """A frame that converts to RGB zeros: zero bytes for RGB; for a YUV surface ``[H*3/2,W]`` Y = 16 (limited range)
-    or 0 (full range) and U = V = 128 (zero bytes there would be a strongly coloured picture), in the sample scale of
-    the format: 16 << 8 and 32768 for p010, 64 and 512 for i010."""
-    if fmt is None:
-        return np.zeros(shape, np.uint8)
-    scale = {"p010": 256, "i010": 4}.get(fmt["pixel_format"], 1)
-    f = np.full(shape, 128 * scale, np.uint16 if scale > 1 else np.uint8)
-    f[: shape[0] * 2 // 3] = 16 * scale if fmt["color_range"] == "limited" else 0
-    return f
+    return SourceFormat.of(**(fmt or {})).blank_frame(shape)        # fmt: forward_batch keywords, None for RGB
 
 
-def _check_surfaces(frames: torch.Tensor, fmt: Optional[Dict[str, str]]) -> None:
-    """A decoder that delivers the wrong element type for its YUV format is a set-up error, not a failed item."""
-    if fmt is not None and frames.dtype != source_dtype(fmt["pixel_format"]):
-        raise ValueError(f"{fmt['pixel_format']} decoder output must be {source_dtype(fmt['pixel_format'])} [n,H*3/2,W] "
-                         f"surfaces, got {frames.dtype}")
-
-
-def _picture_hw(frames, fmt: Optional[Dict[str, str]]):
-    """(H, W) of a decoded window: [T,H,W,3] frames or [T,H*3/2,W] surfaces."""
-    return (frames.shape[1] * 2 // 3, frames.shape[2]) if fmt is not None else (frames.shape[1], frames.shape[2])
+def _deferred_item(frames: torch.Tensor, fmt: SourceFormat, transform: Optional[GpuVideoTransform], **item):
+    """A ``defer=True`` item: the window, its record drawn for the visible ``h x w`` and the keywords of YUV surfaces.  A
+    decoder that delivers frames the transform cannot take is a set-up error, not a failed item."""
+    source = fmt.describe(frames.shape[1:], frames.dtype)
+    params = transform.sample_params(1, source.h, source.w)[0] if transform is not None else None
+    item = dict(frames_u8=frames, params=params, **item)
+    if fmt.yuv:
+        item["format"] = fmt._asdict()
+    return item
 
 
 class GpuDashcamDataset(Dataset):
@@ -250,8 +241,8 @@ class GpuDashcamDataset(Dataset):
             indices, start, end = self._window(reader, row, idx)
             frames = _to_uint8_array(reader.get_batch(indices))
             if len(frames) < need:          # nexar_videos.py:429-433
-                default = (1080, 1280) if self.source_format else (720, 1280, 3)
-                last = frames[-1] if len(frames) else _blank_frame(frames.shape[1:] or default, self.source_format)
+                fmt = self.source_format
+                last = frames[-1] if len(frames) else fmt.blank_frame(frames.shape[1:] or fmt.frame_shape(720, 1280))
                 frames = np.concatenate([frames, np.repeat(last[None], need - len(frames), axis=0)], axis=0)
             frames = torch.from_numpy(np.ascontiguousarray(frames[:need]))
             sensor = self._sensor(reader, idx, start, end)
@@ -263,13 +254,8 @@ class GpuDashcamDataset(Dataset):
             return {"frames": torch.zeros(need, size[0], size[1], 3), "sensor": torch.zeros(need, 4), "target": target,
                     "id": vid}
         if self.defer:
-            _check_surfaces(frames, self.source_format)
-            t = self.transform
-            params = t.sample_params(1, *_picture_hw(frames, self.source_format))[0] if t is not None else None
-            item = {"frames_u8": frames, "params": params, "sensor": sensor, "target": target, "id": vid, "need": need}
-            if self.source_format:
-                item["format"] = self.source_format
-            return item
+            return _deferred_item(frames, self.source_format, self.transform, sensor=sensor, target=target, id=vid,
+                                  need=need)
         video = frames.permute(3, 0, 1, 2)                      # nexar_videos.py:441
         video = self.transform(video) if self.transform else video.float() / 255.0
         return {"frames": video.permute(1, 2, 3, 0), "sensor": sensor, "target": target, "id": vid}   # :451
@@ -346,7 +332,7 @@ class GpuVideoDataset(Dataset):
                 if len(frames) > 0:
                     frames = np.concatenate([frames, np.repeat(frames[-1][None], need - len(frames), axis=0)], axis=0)
                 else:
-                    blank = _blank_frame((1080, 1280) if self.source_format else (720, 1280, 3), self.source_format)
+                    blank = self.source_format.blank_frame(self.source_format.frame_shape(720, 1280))
                     frames = np.repeat(blank[None], need, axis=0)
             frames = torch.from_numpy(np.ascontiguousarray(frames[:need]))
         except Exception:
@@ -355,13 +341,7 @@ class GpuVideoDataset(Dataset):
             size = (224, 224) if self.transform else (720, 1280)   # ncwv:183-190
             return {"frames": torch.zeros(need, size[0], size[1], 3), "target": label, "id": vid}
         if self.defer:
-            _check_surfaces(frames, self.source_format)
-            t = self.transform
-            params = t.sample_params(1, *_picture_hw(frames, self.source_format))[0] if t is not None else None
-            item = {"frames_u8": frames, "params": params, "target": label, "id": vid, "need": need}
-            if self.source_format:
-                item["format"] = self.source_format
-            return item
+            return _deferred_item(frames, self.source_format, self.transform, target=label, id=vid, need=need)
         video = frames.permute(3, 0, 1, 2)                      # ncwv:172
         video = self.transform(video) if self.transform else video.float() / 255.0
         return {"frames": video.permute(1, 2, 3, 0), "target": label, "id": vid}   # ncwv:181
