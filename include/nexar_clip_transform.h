@@ -118,7 +118,13 @@ typedef struct NexarTransformArgs {
   int32_t n_clips, frames_per_clip;
   const void* src;              /* device: base of the decoded frames */
   const int64_t* frame_offsets; /* device [n_clips*frames_per_clip]: BYTE offset of each output frame's
-                                   source frame from src (temporal sampling = gather; repeats allowed) */
+                                   source frame from src (temporal sampling = gather; repeats allowed).
+                                   Every offset must be a multiple of 16 whenever src and src_row_stride are:
+                                   U8 frames are then read by the fast resize kernel, and YUV surfaces of a
+                                   width that is a multiple of 16 by the vector conversion kernels, with
+                                   16-byte loads at src + frame_offsets[i].  Not checked (the offsets live on
+                                   the device); a misaligned offset is a misaligned-address fault.  F32
+                                   frames need 4-byte offsets. */
   int64_t src_row_stride;       /* bytes between source rows */
   const NexarClipParams* params;/* device [n_clips] */
   uint32_t any_flags;           /* host hint: bitwise OR of params[i].flags; stages no clip needs are not launched */
@@ -263,6 +269,11 @@ int nexar_gather_windows_table(const void* pool, int32_t pool_frames, int64_t pl
 
 /* Number of kernel launches the last nexar_clip_transform call on this thread enqueued. */
 int nexar_last_launch_count(void);
+/* Which resize kernel the last nexar_clip_transform call on this thread launched: out = {1, KX, NT, RS, AL4} for the
+ * fixed-point fast kernel (taps per output pixel, threads per block, compile-time row stride or 0, 8-byte window loads)
+ * and {0, 0, 0, 0, 0} for the general kernel or a call that launched none.  Instances that differ only in RS or AL4
+ * compute the same bits; this says which one ran.  NEXAR_ERR_INVALID for a null out. */
+int nexar_last_resize_kernel(int32_t out[5]);
 
 /* Optional timing of the dominant (resize) kernel: after nexar_profile_begin(n) the next n calls record a
  * CUDA event pair around that kernel on the call's stream; nexar_profile_end synchronises those events,

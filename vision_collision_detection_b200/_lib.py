@@ -219,6 +219,27 @@ def table_lib():
     return L
 
 
+_probe_bound = False
+
+
+def last_resize_kernel():
+    """-> (fast, KX, NT, RS, AL4) of the resize kernel the last transform call on this thread launched (all 0 for the
+    general kernel).  Bound on first use only: a library built before it existed serves every other call."""
+    global _probe_bound
+    L = lib()
+    if not _probe_bound:
+        try:
+            fn = L.nexar_last_resize_kernel
+        except AttributeError:
+            raise RuntimeError(f"{LIB_PATH} predates the resize instance probe (no nexar_last_resize_kernel); "
+                               "rebuild it") from None
+        fn.argtypes = [C.c_void_p]
+        _probe_bound = True
+    out = (C.c_int32 * 5)()
+    check(L.nexar_last_resize_kernel(out))
+    return tuple(int(v) for v in out)
+
+
 def yuv_coefficients(matrix: int, range_: int):
     """-> (Yo, Ys, Rv, Gu, Gv, Bu), the integer conversion coefficients the library uses."""
     out = (C.c_int32 * 6)()

@@ -17,6 +17,7 @@
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
+#include <algorithm>
 #include <cmath>
 #include <type_traits>
 #include <cstdio>
@@ -31,6 +32,7 @@
 // ---------------------------------------------------------------------------------
 static thread_local std::string g_err;
 static thread_local int g_launches = 0;
+static thread_local int32_t g_resize_instance[5] = {0, 0, 0, 0, 0};  // nexar_last_resize_kernel: {fast, KX, NT, RS, AL4}
 // experiment knobs and the optional kernel timing are per calling thread (the library keeps no process-global mutable state)
 // 0 auto, 1 force the general fp32 kernels, 2 no programmatic overlap (K1 -> K2 and K3 -> fix-up serialised by the stream);
 // nexar_set_resize_kernel refuses anything else.  tests/test_launch_paths.py pins
@@ -111,6 +113,31 @@ struct NexarPlan {
 // begin1 << 3 (the slot's accumulators restart at this pair) | out_row << 4 | post tap << 16, and "w post" the first tap of the NEXT row of that slot when it falls in the same pair (it is
 // accumulated after the finished row has been flushed).  Returns false when the geometry does not fit.
 static const int kMaxPairs = 1024;
+// Fixed-point taps of one row that sum to exactly 2^15 (constant images stay constant): every tap is the floor of
+// w * 2^15, and the taps with the largest remainders (the first of equal ones) get one more until the row sums to 2^15,
+// so no tap is a unit or more from its exact value.  (Rounding each tap and putting the whole residual on the largest
+// one, up to 4 units, let 0/255 content aligned with the rounding reach 1.05e-3 after normalisation at 540x960 -> 224,
+// above the 1e-3 gate; this way every letterbox stays below 7.1e-4, see tests/fast_resize_model.py.)
+static bool quantise_taps(const float* w, int n, int shift, std::vector<long>& q) {
+  std::vector<double> rem(n);
+  std::vector<int> order(n);
+  q.assign(n, 0);
+  long sum = 0;
+  for (int k = 0; k < n; ++k) {
+    const double x = std::ldexp((double)w[k], shift);
+    q[k] = (long)std::floor(x);
+    rem[k] = x - (double)q[k];
+    sum += q[k];
+    order[k] = k;
+  }
+  const long deficit = (1L << shift) - sum;
+  if (deficit < 0 || deficit > n) return false;
+  std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return rem[a] > rem[b]; });
+  for (long k = 0; k < deficit; ++k) ++q[order[k]];
+  for (int k = 0; k < n; ++k)
+    if (q[k] < 0 || q[k] > 65535) return false;
+  return true;
+}
 static bool build_fast_tables(NexarPlan* p, int ky, int kx, int& shift, int& kx_al) {
   const NexarGeometry& g = p->g;
   if (p->src_dtype != NEXAR_SRC_U8 && p->src_dtype != NEXAR_SRC_NV12) return false;
@@ -144,17 +171,8 @@ static bool build_fast_tables(NexarPlan* p, int ky, int kx, int& shift, int& kx_
     if (yc <= 0) return false;
     if (i + 2 < g.resize_h && p->ystart[i + 2] < ys + yc) return false;  // three rows alive at once
     if (i + 1 < g.resize_h && p->ystart[i + 1] + p->ycount[i + 1] <= ys + yc) return false;  // must finish in order
-    const float* w = &p->ywt[(size_t)i * ky];
-    std::vector<long> q(yc);
-    long sum = 0;
-    int arg = 0;
-    for (int k = 0; k < yc; ++k) {
-      q[k] = std::lrint(std::ldexp((double)w[k], shift));
-      sum += q[k];
-      if (q[k] > q[arg]) arg = k;
-    }
-    q[arg] += (1L << shift) - sum;  // rows sum to exactly 2^shift: constant images stay constant
-    if (q[arg] < 0 || q[arg] > 65535) return false;
+    std::vector<long> q;
+    if (!quantise_taps(&p->ywt[(size_t)i * ky], yc, shift, q)) return false;
     const int slot = i % 2;
     const int prev_last = i >= 2 ? p->ystart[i - 2] + p->ycount[i - 2] - 1 : -1;  // last tap of the slot's previous row
     bool begun = false;
@@ -196,16 +214,8 @@ static bool build_fast_tables(NexarPlan* p, int ky, int kx, int& shift, int& kx_
   // two taps per word: byte0/1 = low bytes of the even/odd tap, byte2/3 = their high bytes.
   p->xw16.assign((size_t)g.resize_w * (kx_al / 2), 0u);
   for (int j = 0; j < g.resize_w; ++j) {
-    std::vector<long> q(kx_al);
-    long sum = 0;
-    int arg = 0;
-    for (int k = 0; k < kx_al; ++k) {
-      q[k] = std::lrint(std::ldexp((double)p->xwt_al[(size_t)j * kx_al + k], 15));
-      sum += q[k];
-      if (q[k] > q[arg]) arg = k;
-    }
-    q[arg] += (1L << 15) - sum;
-    if (q[arg] < 0 || q[arg] > 65535) return false;
+    std::vector<long> q;
+    if (!quantise_taps(&p->xwt_al[(size_t)j * kx_al], kx_al, 15, q)) return false;
     for (int m = 0; m < kx_al / 2; ++m) {
       const unsigned e = (unsigned)q[2 * m], o = (unsigned)q[2 * m + 1];
       p->xw16[(size_t)j * (kx_al / 2) + m] = (e & 255u) | ((o & 255u) << 8) | ((e >> 8) << 16) | ((o >> 8) << 24);
@@ -253,6 +263,15 @@ extern "C" size_t nexar_sizeof_clip_params(void) { return sizeof(NexarClipParams
 extern "C" size_t nexar_sizeof_transform_args(void) { return sizeof(NexarTransformArgs); }
 extern "C" const char* nexar_last_error(void) { return g_err.c_str(); }
 extern "C" int nexar_last_launch_count(void) { return g_launches; }
+extern "C" int nexar_last_resize_kernel(int32_t out[5]) {
+  if (!out) return fail(NEXAR_ERR_INVALID, "last_resize_kernel: null argument");
+  memcpy(out, g_resize_instance, sizeof(g_resize_instance));
+  return NEXAR_OK;
+}
+static void record_resize_instance(int fast, int kx, int nt, int rs, int al4) {
+  const int32_t v[5] = {fast, kx, nt, rs, al4};
+  memcpy(g_resize_instance, v, sizeof(v));
+}
 extern "C" int nexar_set_resize_kernel(int32_t v) {
   if (v == 4) return fail(NEXAR_ERR_UNSUPPORTED, "set_resize_kernel: variant 4 (the fused cluster kernel) was removed");
   if (v != 0 && v != 1 && v != 2)
@@ -2590,6 +2609,7 @@ static int launch_all(const NexarPlan* p, const NexarTransformArgs* a, KArgs& K,
 #define NEXAR_FAST_RS(KXV, NTV, MB, RSV)                                                                          \
   {                                                                                                               \
     constexpr bool kAl = (KXV) == 10;  /* 8-byte window loads exist for the 10-tap kernels only */                \
+    record_resize_instance(1, KXV, NTV, RSV, kAl && P.x_align4);                                                  \
     if (kAl && P.x_align4)                                                                                        \
       CUDA_TRY(launch_fast(resize_fast_kernel<KXV, NTV, MB, RSV, DstT, kAl>, grid, NTV, smem_fast, st, P, K));    \
     else                                                                                                          \
@@ -2643,6 +2663,7 @@ static int launch_all(const NexarPlan* p, const NexarTransformArgs* a, KArgs& K,
     tail_done = true;
     g_launches += 2;
   } else {
+    record_resize_instance(0, 0, 0, 0, 0);
     nbands = imax(1, imin(kMaxBands, vis_rows / 24));
     const size_t smem = (size_t)P.src_w * 3 * sizeof(float);
     if (smem > 48 * 1024)
@@ -2810,6 +2831,7 @@ extern "C" int nexar_gather_windows_table(const void* pool, int32_t pool_frames,
 
 extern "C" int nexar_clip_transform(const NexarPlan* p, const NexarTransformArgs* a) {
   g_launches = 0;
+  record_resize_instance(0, 0, 0, 0, 0);
   if (!p || !a) return fail(NEXAR_ERR_INVALID, "clip_transform: null argument");
   if (a->struct_size != sizeof(NexarTransformArgs)) return fail(NEXAR_ERR_INVALID, "clip_transform: NexarTransformArgs size mismatch (ABI)");
   if (a->n_clips <= 0 || a->frames_per_clip <= 0) return fail(NEXAR_ERR_INVALID, "clip_transform: empty batch");

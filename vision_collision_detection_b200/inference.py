@@ -360,6 +360,31 @@ def multi_stream_schedule(videos: Sequence[Tuple[int, int, bool]], queue: Sequen
             return rounds
 
 
+def group_frames(parts: Sequence[torch.Tensor], frame_bytes: int, device: torch.device,
+                 staging_for: Callable[[int], torch.Tensor]) -> Tuple[torch.Tensor, np.ndarray]:
+    """The frames of one transform call from several chunks -> (base tensor, int64 byte offset of every frame from its
+    ``data_ptr()``), the frames in the order of ``parts``.  A part on ``device`` whose address is a multiple of 16 is
+    read in place; every other part (host frames, or a device view at any other address) is copied, with one
+    non-blocking copy, into the buffer ``staging_for(n)`` returns for the ``n`` frames staged.  The library reads the
+    frames with 16-byte loads at base + offset whenever the base and the row stride are multiples of 16, and a frame
+    at any other address would be a misaligned-address fault; the parts taken in place and the staging buffer both
+    start on 16 bytes, so with frames of a multiple of 16 bytes every offset is one."""
+    in_place = [p.device == device and p.data_ptr() % 16 == 0 for p in parts]
+    n_staged = sum(p.shape[0] for p, keep in zip(parts, in_place) if not keep)
+    staging = staging_for(n_staged) if n_staged else None
+    srcs, addr, at = [], [], 0
+    for part, keep in zip(parts, in_place):
+        if not keep:
+            dst = staging[at:at + part.shape[0]]
+            dst.copy_(part, non_blocking=True)
+            at += part.shape[0]
+            part = dst
+        srcs.append(part)
+        addr.append(part.data_ptr() + frame_bytes * np.arange(part.shape[0], dtype=np.int64))
+    base = min(srcs, key=lambda t: t.data_ptr())       # offsets from the lowest frame address: all >= 0
+    return base, np.concatenate(addr) - base.data_ptr()
+
+
 class _Video:
     """A video of a ``MultiWindowStream``: its key, record / tail slot, frame counts and source."""
     __slots__ = ("key", "slot", "seen", "closed", "source")
@@ -384,8 +409,9 @@ class MultiWindowStream:
     pushes, steps and closes.  A video shorter than ``window`` gets its padded window at the step after its ``close``; a
     push after ``close`` opens a new video under the same key.
 
-    Chunks are what ``WindowStream.push`` takes, on the device (read in place) or the host (copied with a non-blocking
-    copy; do not overwrite a pinned chunk before the step's work has run).  Videos may differ in resolution and format.
+    Chunks are what ``WindowStream.push`` takes, on the device (read in place when it starts on a 16-byte boundary, as
+    every tensor torch allocates does; copied otherwise) or the host (copied with a non-blocking copy; do not overwrite
+    a pinned chunk before the step's work has run).  Videos may differ in resolution and format.
     Device memory is one pool of ``max_frames_per_step`` step slots plus ``window - 1`` slots per open video, and a
     host-staging buffer of at most ``max_frames_per_step`` frames per source group; a step with more queued frames than
     ``max_frames_per_step`` runs in rounds, in push order.  It never depends on how long a video runs, and it is released
@@ -483,23 +509,11 @@ class MultiWindowStream:
         calls, offsets = [], []
         for _, p0, p1 in rnd.groups:
             pieces = rnd.pieces[p0:p1]
-            first = self._queue[pieces[0][0]]
-            fs, n = first[0].source, sum(hi - lo for _, lo, hi, _ in pieces)
-            n_host = sum(hi - lo for q, lo, hi, _ in pieces if not self._queue[q][1].is_cuda)
-            staging = self._staging_for(fs, n_host) if n_host else None
-            srcs, addr, rec, at = [], [], [], 0
-            for q, lo, hi, _ in pieces:
-                video, chunk = self._queue[q]
-                part = chunk[lo:hi]
-                if not chunk.is_cuda:        # host frames: one non-blocking copy per chunk into the group's staging
-                    part = staging[at:at + hi - lo]
-                    part.copy_(chunk[lo:hi], non_blocking=True)
-                    at += hi - lo
-                srcs.append(part)
-                addr.append(part.data_ptr() + fs.frame_bytes * np.arange(hi - lo, dtype=np.int64))
-                rec.append(np.full(hi - lo, video.slot, np.int64))
-            base = min(srcs, key=lambda t: t.data_ptr())       # offsets from the lowest frame address: all >= 0
-            offsets.append(np.concatenate(addr) - base.data_ptr())
+            fs, n = self._queue[pieces[0][0]][0].source, sum(hi - lo for _, lo, hi, _ in pieces)
+            base, offs = group_frames([self._queue[q][1][lo:hi] for q, lo, hi, _ in pieces], fs.frame_bytes, self.device,
+                                      lambda k: self._staging_for(fs, k))
+            offsets.append(offs)
+            rec = [np.full(hi - lo, self._queue[q][0].slot, np.int64) for q, lo, hi, _ in pieces]
             params = self._records[np.concatenate(rec)]          # one vectorised index into the packed records
             calls.append((base, fs, pieces[0][3], n, params))
         # frame offsets and both slot tables: one upload through the engine's pinned staging
